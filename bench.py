@@ -252,6 +252,8 @@ def own_arm(a):
     free_b, _tot = torch.cuda.mem_get_info()
     need = 8 * nso * nt * nsim
     if need > 0.9 * free_b:
+        if a.dump_outputs:  # the dump must come from the same inputs on every run
+            raise SystemExit("bench.py: --dump-outputs needs room for all %d agents, but %.1f GB of device memory are free" % (nsim, free_b / 1e9))
         nsim = int(0.9 * free_b / (8 * nso * nt))
     g = torch.Generator(device=dev)
     g.manual_seed(SEED_INIT + rank)
@@ -289,6 +291,8 @@ def own_arm(a):
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     sim_ms = max_over_ranks(e0.elapsed_time(e1) / a.steps)
+    if a.dump_outputs and rank == 0:
+        dump_sim_outputs(a.dump_outputs, sol, d_sims, d_mom, nsim, nt, nso)
     sim_launches = lib.launch_count() - l0
     kern_ms = float(np.mean([x.elapsed_time(y) for x, y in kev]))
     alive = float(d_mom.view(nt, nso, 3)[:, 0, 2].sum().item())  # agent-periods written (all ranks after the all-reduce)
@@ -466,6 +470,10 @@ def measure_batch(a, rank, world, dev, with_cpu):
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1) / a.steps
+    if a.dump_outputs and rank == 0:  # a fixed sample of 1024 of the sweep's vectors keeps the dump small
+        vecs = np.sort(np.random.default_rng(4096).choice(nvec, min(nvec, 1024), replace=False))
+        _save(a.dump_outputs, "batch_vectors", vecs)
+        _save(a.dump_outputs, "batch_moments", table.view(nvec, nt, nso, 3)[torch.from_numpy(vecs).to(dev)].permute(0, 3, 2, 1).cpu().numpy())
     if world > 1:
         t = torch.tensor([ms], dtype=torch.float64, device=dev); dist.all_reduce(t, op=dist.ReduceOp.MAX); ms = float(t.item())
     # split of one step on this rank (events around the two calls, outside the timed region)
@@ -489,6 +497,45 @@ def measure_batch(a, rank, world, dev, with_cpu):
     return out
 
 
+def dump_sim_outputs(out, sol, d_sims, d_mom, nsim, nt, nso):
+    """What the timed path returned in its last step: the S1 solution (cells stacked in (it, ist) order, with their row
+    counts), the moments [3, nsimout, nt] and the records [k, nt, nsimout] of a fixed sample of k = 1024 agents (the full
+    path array is tens of GB)."""
+    import torch
+    M, D = sol.M, sol.D
+    cells = [(M[ist][it], D[ist][it]) for it in range(nt) for ist in range(len(M)) if M[ist][it] is not None and M[ist][it].size]
+    _save(out, "solve_M", np.concatenate([c[0] for c in cells]))
+    _save(out, "solve_D", np.concatenate([c[1] for c in cells]))
+    _save(out, "solve_cell_rows", np.array([[c[0].shape[0], c[1].shape[0]] for c in cells], dtype=np.float64))
+    _save(out, "sim_moments", d_mom.view(nt, nso, 3).permute(2, 1, 0).cpu().numpy())
+    k = min(nsim, 1024)
+    agents = np.sort(np.random.default_rng(SEED_SHOCKS).choice(nsim, k, replace=False))
+    _save(out, "sim_agents", agents.astype(np.float64))
+    _save(out, "sim_records", d_sims.view(nsim, nt, nso)[torch.from_numpy(agents).to(d_sims.device)].cpu().numpy())
+
+
+DUMP_CAP = 64 * 2 ** 20
+_dumped = [0]
+
+
+def _save(out, name, arr):
+    """DIR/<name>.npy with every entry finite, and DIR/<name>_nonfinite.npy coding the entries that were not (0 finite,
+    1 NaN, 2 +inf, 3 -inf; they are 0 in <name>.npy).  -inf is a value the solver and simulator do return (consumption
+    and value at zero consumption, and the moments summing them); NaN marks simulation columns a model leaves unset.
+    Split this way, two dumps compare entry by entry with a tolerance and still agree on every non-finite value."""
+    os.makedirs(out, exist_ok=True)
+    a = np.asarray(arr, dtype=np.float64)
+    code = np.zeros(a.shape, dtype=np.float32)
+    code[np.isnan(a)] = 1
+    code[a == np.inf] = 2
+    code[a == -np.inf] = 3
+    _dumped[0] += a.nbytes + code.nbytes
+    if _dumped[0] > DUMP_CAP:
+        raise SystemExit("bench.py: --dump-outputs would exceed %d MB at %s" % (DUMP_CAP >> 20, name))
+    np.save(os.path.join(out, name + ".npy"), np.where(code == 0, a, 0.0))
+    np.save(os.path.join(out, name + "_nonfinite.npy"), code)
+
+
 def _batch_worker(job):
     from egdst_b200 import examples
     from tests.oracles import oracle_for
@@ -505,8 +552,13 @@ def _batch_worker(job):
 
 def batch_cpu_baseline(params, nsim, a):
     """The reference C on every host core (BASELINE.md section 4): `cores` independent single-threaded reference
-    processes, each solving and simulating its share of a bounded sample of the sweep's vectors."""
+    processes, each solving and simulating its share of a bounded sample of the sweep's vectors.  None where the
+    reference is not built (oracle/ref.py)."""
     import multiprocessing as mp
+    from egdst_b200 import examples
+    from tests.oracles import ref_available
+    if not ref_available(examples.deaton2()):
+        return None
     cores = os.cpu_count() or 1
     nv = max(cores, min(a.batch_cpu_nvec, params.shape[0]))
     jobs = [(params[i, 0], params[i, 1], nsim, i) for i in range(nv)]
@@ -539,9 +591,12 @@ def batch_arm(a):
 
 
 def cpu_baseline(m, sol, a):
-    """Reference C (oracle/_ref) on one core: simulate a bounded sample of agents on the exported tables, and one S1 solve."""
+    """Reference C (oracle/_ref) on one core: simulate a bounded sample of agents on the exported tables, and one S1 solve.
+    Where the reference is not built, the simulation is timed with its C restatement (oracle/port) and the solve is
+    not timed (the solver has no restatement)."""
     from tests.oracles import oracle_for
     orc = oracle_for(m)
+    kind = orc.kind if orc.kind == "reference" else "port"
     M, D = sol.M, sol.D
     ns = a.cpu_nsim
     rng = np.random.default_rng(SEED_INIT)
@@ -549,11 +604,11 @@ def cpu_baseline(m, sol, a):
     rs = rng.random(4 * ns * m.nt)
     orc.simulate(M, D, init, rs, 0)
     sim_s = orc.seconds
-    cpu = {"value": ns * m.nt / sim_s, "unit": "agent-periods/s", "cores": 1, "kind": orc.kind,
+    cpu = {"value": ns * m.nt / sim_s, "unit": "agent-periods/s", "cores": 1, "kind": kind,
            "sample": "%d agents x %d periods on the S1 tables, gateway time %.2f s (reference simulator is single-threaded)" % (ns, m.nt, sim_s),
            "host_cores": os.cpu_count()}
     solve_cpu = None
-    if not a.no_cpu_solve:
+    if not a.no_cpu_solve and kind == "reference":
         orc.solve()
         s = orc.seconds
         solve_cpu = {"value": nominal_units(m) / s, "unit": "grid-point-periods/s", "cores": 1, "kind": orc.kind,
@@ -663,6 +718,7 @@ def main():
     ap.add_argument("--no-batch", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-cpu-solve", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed paths computed in their last step to DIR/<name>.npy (non-finite entries coded in DIR/<name>_nonfinite.npy; at most 64 MB; e.g. dumps/)")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3) if a.impl == "own" else a.warmup
     if a.impl == "reference":

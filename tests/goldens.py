@@ -5,6 +5,7 @@ import os
 import numpy as np
 
 from egdst_b200 import examples
+from tests.stored import SampledSims
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLDEN = os.path.join(HERE, "golden")
@@ -41,9 +42,19 @@ def load(name):
             "skipcols": skip}
 
 
+def paired(sa, sb):
+    """(sa, sb, period): the two simulations on the records ``sb`` holds, as [n, k, nsimout] arrays, and the period of
+    each record.  A stored ``SampledSims`` holds k = 1 record per row."""
+    if isinstance(sb, SampledSims):
+        return sb.pick(sa)[:, None, :], sb.records[:, None, :], sb.periods[:, None]
+    return sa, sb, np.broadcast_to(np.arange(sb.shape[1]), sb.shape[:2])
+
+
 def sims_errors(sa, sb, skipcols=()):
     """Compare two [nsim, nt, nsimout] simulation arrays: NaN pattern, discrete columns (id=4, ist=5)
-    exactly, everything else |d|/max(1,|f|).  ``skipcols`` are left out of the comparison."""
+    exactly, everything else |d|/max(1,|f|).  ``skipcols`` are left out of the comparison.  ``sb`` may be the stored
+    records of a simulation (tests/stored.py): the same records of ``sa`` are compared then."""
+    sa, sb, _ = paired(sa, sb)
     if len(skipcols):
         sa, sb = sa.copy(), sb.copy()
         sa[:, :, list(skipcols)] = 0.0

@@ -1,6 +1,7 @@
-"""Pick the checker for a model: oracle/_ref (the unmodified reference C, prebuilt .so or built from
-/root/reference) when available, else the C restatement in oracle/ (kind 'port')."""
+"""Pick the checker for a model: oracle/_ref (the unmodified reference C, prebuilt or built from its sources,
+oracle/ref.py) when available, else the stored outputs of tests/golden/stored.npz (kind 'stored', tests/stored.py)."""
 from oracle import ref
+from tests.stored import Stored
 
 
 class _Ref:
@@ -20,30 +21,13 @@ class _Ref:
         return self.r.last_seconds
 
 
-class _Port:
-    kind = "port"
-
-    def __init__(self, model):
-        from oracle import port
-        self.p = port.Port(model)
-
-    def solve(self):
-        return self.p.solve()  # raises: the solver's checker is the compiled reference only
-
-    def simulate(self, M, D, init, rs, rndtype=0):
-        return self.p.simulate(M, D, init, rs, rndtype)
-
-    @property
-    def seconds(self):
-        return self.p.last_seconds
-
-
 def ref_available(model) -> bool:
     return ref.build(model) is not None
 
 
-def oracle_for(model, prefer="reference"):
+def oracle_for(model, prefer="reference", whole=False):
+    """``whole``: a stored solution keeps every row of every cell (for tests that inspect the rows)."""
     model.prepare()
     if prefer == "reference" and ref_available(model):
         return _Ref(model)
-    return _Port(model)
+    return Stored(model, whole)

@@ -8,6 +8,8 @@ Thresholds, evf(a0) (row 0 of V) and the decision sequence are compared directly
 """
 import numpy as np
 
+from tests.stored import NOT_SAMPLED, SampledCell
+
 
 def _interp(M, F, x):
     # rows 1.. (row 0 is the a0 row: V there is evf(a0), not a value)
@@ -29,24 +31,34 @@ def _gap(a, b):
 
 
 def cell_errors(Ma, Da, Mb, Db, nprobe=50001, excl=1e-9):
-    lo = max(Ma[1, 0], Mb[1, 0])
-    hi = min(Ma[-1, 0], Mb[-1, 0])
-    out = {"range_lo": abs(Ma[1, 0] - Mb[1, 0]), "range_hi": abs(Ma[-1, 0] - Mb[-1, 0])}
-    x = np.linspace(lo, hi, nprobe)
-    mask = np.ones_like(x, dtype=bool)
+    """``Mb`` may be a stored SampledCell (tests/stored.py): its sampled rows are the probes then."""
+    sampled = isinstance(Mb, SampledCell)
+    if sampled:
+        out = {"range_lo": 0.0, "range_hi": 0.0}
+        x = Mb.x
+        mask = (x >= Ma[1, 0]) & (x <= Ma[-1, 0])
+    else:
+        lo = max(Ma[1, 0], Mb[1, 0])
+        hi = min(Ma[-1, 0], Mb[-1, 0])
+        out = {"range_lo": abs(Ma[1, 0] - Mb[1, 0]), "range_hi": abs(Ma[-1, 0] - Mb[-1, 0])}
+        x = np.linspace(lo, hi, nprobe)
+        mask = np.ones_like(x, dtype=bool)
     for th in np.concatenate([Da[:, 1], Db[:, 1]]):
         mask &= np.abs(x - th) > excl
     # also stay away from each solution's own double points (secondary-envelope kinks insert them too)
-    for M in (Ma, Mb):
+    for M in ((Ma,) if sampled else (Ma, Mb)):
         dm = np.diff(M[1:, 0])
         for xd in M[1:-1, 0][dm < 1e-9]:
             mask &= np.abs(x - xd) > excl
     x = x[mask]
-    ca, cb = _interp(Ma, Ma[1:, 1], x), _interp(Mb, Mb[1:, 1], x)
-    va, vb = _interp(Ma, Ma[1:, 3], x), _interp(Mb, Mb[1:, 3], x)
+    ca, va = _interp(Ma, Ma[1:, 1], x), _interp(Ma, Ma[1:, 3], x)
+    if sampled:
+        cb, vb = Mb.c[mask], Mb.v[mask]
+    else:
+        cb, vb = _interp(Mb, Mb[1:, 1], x), _interp(Mb, Mb[1:, 3], x)
     out["C"] = _gap(ca, cb)
     out["V"] = _gap(va, vb)
-    ea, eb = Ma[0, 3], Mb[0, 3]
+    ea, eb = Ma[0, 3], (Mb.evf if sampled else Mb[0, 3])
     out["evf"] = 0.0 if (ea == eb or (np.isinf(ea) and np.isinf(eb) and ea == eb)) else float(abs(ea - eb) / max(1.0, abs(eb)))
     out["nth"] = (Da.shape[0], Db.shape[0])
     if Da.shape[0] == Db.shape[0]:
@@ -55,7 +67,7 @@ def cell_errors(Ma, Da, Mb, Db, nprobe=50001, excl=1e-9):
     else:
         out["TH"] = float("inf")
         out["Dseq"] = False
-    out["rows"] = (Ma.shape[0], Mb.shape[0])
+    out["rows"] = (Ma.shape[0], Mb.nrows if sampled else Mb.shape[0])
     return out
 
 
@@ -65,6 +77,9 @@ def solution_errors(Ma, Da, Mb, Db, **kw):
     for ist in range(len(Mb)):
         for it in range(len(Mb[ist])):
             a, b = Ma[ist][it], Mb[ist][it]
+            if b is NOT_SAMPLED:
+                assert a is not None and a.size, "candidate lacks cell (ist=%d,it=%d)" % (ist, it)
+                continue
             if b is None or b.size == 0:
                 assert a is None or a.size == 0, "candidate has a solution where the oracle has none"
                 continue

@@ -7,6 +7,7 @@ import pytest
 from egdst_b200 import distributed as D
 from egdst_b200 import examples
 from oracle import ref
+from tests.goldens import paired
 from tests.oracles import oracle_for
 from tests.parity import cell_errors, solution_errors
 
@@ -55,16 +56,16 @@ def test_s1_full_size_matches_reference(s1):
     init = np.column_stack([np.ones(nsim), s1.a0 + 0.5 * (s1.mmax - s1.a0) * rng.random(nsim)])
     rs = rng.random(4 * nsim * s1.nt)
     s1.sim(init, "own_shocks", randstream=rs)
-    sr = orc.simulate(Mr, Dr, init, rs, 0)
+    ours, sr, period = paired(s1.sims, orc.simulate(Mr, Dr, init, rs, 0))
     both = ~np.isnan(sr)
-    assert np.array_equal(np.isnan(s1.sims), np.isnan(sr))
+    assert np.array_equal(np.isnan(ours), np.isnan(sr))
     # identical discrete choices except where cash is within 1e-9 of a threshold
-    diff = (s1.sims[:, :, 4] != sr[:, :, 4]) & both[:, :, 4]
+    diff = (ours[:, :, 4] != sr[:, :, 4]) & both[:, :, 4]
     for i, t in zip(*np.nonzero(diff)):
-        assert np.min(np.abs(Dr[0][t][:, 1] - sr[i, t, 0])) < 1e-9
+        assert np.min(np.abs(Dr[0][period[i, t]][:, 1] - sr[i, t, 0])) < 1e-9
     ok = both & ~np.repeat(diff[:, :, None], sr.shape[2], axis=2)
     fin = ok & np.isfinite(sr)
-    assert np.max(np.abs(s1.sims[fin] - sr[fin]) / np.maximum(1, np.abs(sr[fin]))) < TOL
+    assert np.max(np.abs(ours[fin] - sr[fin]) / np.maximum(1, np.abs(sr[fin]))) < TOL
 
 
 def test_s5_retirement1_2000_points(s1):
@@ -281,13 +282,13 @@ def test_lecture_model2_at_the_authors_largest_configuration():
     init = np.column_stack([np.full(nsim, 2.0), rng.uniform(1.0, 60.0, nsim)])  # everybody starts working
     rs = rng.random(4 * nsim * m.nt)
     m.sim(init, "own_shocks", randstream=rs)
-    sr = orc.simulate(Mr, Dr, init, rs, 0)
-    assert np.array_equal(np.isnan(m.sims), np.isnan(sr))
+    ours, sr, _ = paired(m.sims, orc.simulate(Mr, Dr, init, rs, 0))
+    assert np.array_equal(np.isnan(ours), np.isnan(sr))
     both = ~np.isnan(sr)
-    diff = ((m.sims[:, :, 4] != sr[:, :, 4]) | (m.sims[:, :, 5] != sr[:, :, 5])) & both[:, :, 4]
+    diff = ((ours[:, :, 4] != sr[:, :, 4]) | (ours[:, :, 5] != sr[:, :, 5])) & both[:, :, 4]
     assert diff.sum() == 0
     fin = both & np.isfinite(sr)
-    assert np.max(np.abs(m.sims[fin] - sr[fin]) / np.maximum(1, np.abs(sr[fin]))) < TOL
+    assert np.max(np.abs(ours[fin] - sr[fin]) / np.maximum(1, np.abs(sr[fin]))) < TOL
     # retirement is absorbing: once ist == 0 (retired) it stays 0
     ist = m.sims[:, :, 5]
     assert np.all(np.diff(ist, axis=1) <= 0)
@@ -369,7 +370,7 @@ def test_continuous_states_match_reference(variant, kw):
     reference addresses correctly; its value column is never assigned on this branch and is left out."""
     m = _solve(examples.EXTRA[variant](**kw))
     orc = oracle_for(m)
-    assert orc.kind == "reference"
+    assert orc.kind in ("reference", "stored")
     Mr, Dr = orc.solve()
     e = solution_errors(m.M, m.D, Mr, Dr)
     assert e["C"] < TOL and e["V"] < TOL and e["TH"] < 1e-8 and e["Dseq"] and e["rowdiff"] == 0, e
@@ -471,7 +472,7 @@ def test_mortality_ends_records_and_keeps_the_moment_counts():
     out of the moment sums and counts (the kernel's "clean tile" fast path must hand over to the NaN-aware one)."""
     m = _solve(examples.retirement_mortal(T=30, ngridm=300, ngridmax=700, nthrhmax=300, ny=10))
     orc = oracle_for(m)
-    assert orc.kind == "reference"
+    assert orc.kind in ("reference", "stored")
     Mr, Dr = orc.solve()
     e = solution_errors(m.M, m.D, Mr, Dr)
     assert e["C"] < TOL and e["V"] < TOL and e["Dseq"], e
@@ -510,7 +511,7 @@ def test_shock_dependent_transitions_match_reference():
     m = _solve(examples.retirement_jobloss(T=20, ngridm=400, ngridmax=1000, nthrhmax=100, ny=12))
     assert m.optim["optim_TRPRnoSH"] is False
     orc = oracle_for(m)
-    assert orc.kind == "reference"
+    assert orc.kind in ("reference", "stored")
     Mr, Dr = orc.solve()
     e = solution_errors(m.M, m.D, Mr, Dr)
     assert e["C"] < TOL and e["V"] < TOL and e["TH"] < 1e-8 and e["Dseq"] and e["rowdiff"] == 0, e
@@ -576,7 +577,7 @@ def test_late_zero_consumption_resends_match_reference():
     other grid sizes and horizons make the reference abort with its own errors, so this one configuration is the GPU's
     parity evidence for the path: S1b at BASELINE size takes 494 re-sends on the host emulator but none on the GPU.)"""
     m = examples.deaton_meanstest()
-    Mr, Dr = oracle_for(m).solve()
+    Mr, Dr = oracle_for(m, whole=True).solve()
     m.compile()
     sol = m._capi().solve(m)
     assert sol.status(0)[0] == 0, sol.status(0)
