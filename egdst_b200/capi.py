@@ -226,6 +226,8 @@ class ModelLibrary:
         L.egdst_call.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, _dp, C.c_int, C.c_int, _dp]
         L.egdst_sim_moments.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, _dp, C.c_int, C.c_longlong, C.c_ulonglong, _dp]
         L.egdst_sim_moments_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, vp, C.c_int, C.c_longlong, C.c_ulonglong, vp]
+        L.egdst_test_envelope2.argtypes = [C.POINTER(EgdstDesc), C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, C.c_int, C.c_double,
+                                           _dp, _dp, _dp, _ip]
         if L.egdst_abi_version() != ABI_VERSION:
             raise RuntimeError("ABI version mismatch in %s" % path)
 
@@ -397,7 +399,6 @@ class ModelLibrary:
         cap = int(model.ngridmax) + 8
         oX, oC, oV = np.zeros(cap), np.zeros(cap), np.zeros(cap)
         n = C.c_int(0)
-        self.L.egdst_test_envelope2.argtypes = [C.POINTER(EgdstDesc), C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, C.c_int, C.c_double, _dp, _dp, _dp, _ip]
         rc = self.L.egdst_test_envelope2(C.byref(d.c), it, 0, idd, _ptr(X), _ptr(Cc), _ptr(V), X.size, float(evfa0), _ptr(oX), _ptr(oC), _ptr(oV), C.byref(n))
         if rc:
             self._raise(rc)

@@ -11,6 +11,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <atomic>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -71,6 +72,20 @@ static int fail(int code, const std::string &msg) { g_err = msg; return code; }
         cudaError_t e_ = (call);                                                                       \
         if (e_ != cudaSuccess) return fail(2, std::string("CUDA error: ") + cudaGetErrorString(e_) + " at " #call); \
     } while (0)
+// error-accumulating form (cudaError_t ce in scope): once a call has failed, the following ones are skipped
+#define EGDST_TRY(call) do { if (ce == cudaSuccess) ce = (call); } while (0)
+
+// grow-only device buffer of n elements: reallocated, without its contents, when n does not fit
+template <class T>
+static cudaError_t grow(T **p, size_t *cap, size_t n) {
+    if (*p && n <= *cap) return cudaSuccess;
+    if (*p) cudaFree(*p);
+    *p = 0;
+    *cap = 0;
+    const cudaError_t e = cudaMalloc((void **)p, (n ? n : 1) * sizeof(T));
+    if (e == cudaSuccess) *cap = n;
+    return e;
+}
 
 static const char *status_text(int code) {
     switch (code) {  // wording of the reference's error() sites
@@ -95,39 +110,74 @@ static const char *status_text(int code) {
     }
 }
 
+enum { SCOPE_GRID = 0, SCOPE_CTA, SCOPE_WARP };  // work partitions of the solve kernel (egdst_period.cuh)
+
+// Test hooks, read from the environment when a solution object is created (read_hooks).  None is set in production.
+struct EgdstHooks {
+    int scope;                  // EGDST_SOLVE_SCOPE: "grid", "warp", any other value CTA; -1: chosen by the shape
+    int warpG, warpGSet;        // EGDST_WARP_G: warps per CTA of the WARP scope (when set, no fall-back to the CTA scope)
+    int egmP;                   // EGDST_EGM_P: grid points per work item of the EGM phase
+    int tabcap;                 // EGDST_TABCAP: lookup-table capacity; cells with more rows take the table-free path
+    int solveFrom, solveTo;     // EGDST_SOLVE_FROM/_TO: solve these periods only, the cells of later ones are imported
+};
+
+static EgdstHooks read_hooks() {
+    auto num = [](const char *v, int unset) { return v ? atoi(v) : unset; };
+    const char *scope = getenv("EGDST_SOLVE_SCOPE"), *warpG = getenv("EGDST_WARP_G");
+    EgdstHooks h;
+    h.scope = !scope ? -1 : strcmp(scope, "grid") == 0 ? SCOPE_GRID : strcmp(scope, "warp") == 0 ? SCOPE_WARP : SCOPE_CTA;
+    h.warpG = num(warpG, 0);
+    h.warpGSet = warpG != 0;
+    h.egmP = num(getenv("EGDST_EGM_P"), 0);
+    h.tabcap = num(getenv("EGDST_TABCAP"), 0);
+    h.solveFrom = num(getenv("EGDST_SOLVE_FROM"), -1);
+    h.solveTo = num(getenv("EGDST_SOLVE_TO"), -1);
+    return h;
+}
+
+// How the solve kernel is launched for one object (plan_solve)
+struct SolvePlan {
+    int scope = SCOPE_GRID;
+    int ctas = 0, block = 0, warps = 0;  // CTAs (one resident wave), threads per CTA (per warp in the WARP scope), warps per CTA
+    size_t smem = 0;                     // dynamic shared memory
+    int syncOff = -1, groupBytes = 0;    // per-vector state in shared memory (CTA and WARP scopes), bytes per warp (WARP)
+    int egmP = 0, chC = 0, chE = 0;      // grid points per EGM work item; scan windows per job of the EGM phase and of the merge
+    int itStart = 0, itStop = 0;         // periods solved
+};
+
 struct egdst_solution {
-    EgdstDev P;
-    int device;
-    std::vector<void *> owned;  // device allocations
-    double *d_qraw;             // quadrature as passed (weights, abscissas)
-    double *d_stm, *d_states, *d_decisions, *d_bparams, *d_q;
-    int nsd, ncell, nslot;
-    EgdstDev *d_self; // copy of P in global memory (smoothing mode)
-    int ncell_all;  // ncell, plus the ncell*nd choice-specific cells of the smoothing mode
+    EgdstDev P{};
+    int device = 0;
+    int dims[12] = {};    // shape signature for re-use
+    double dkey[2] = {};  // mmax, a0: the geometry of the lookup tables (mbits, lutcap) is derived from them at creation
+    EgdstHooks hooks{};   // in effect at creation; part of the re-use key, since the plan and tabcap depend on them
+    SolvePlan plan;
+    int nsd = 0, ncell = 0, nslot = 0;
+    int ncell_all = 0;    // ncell, plus the ncell*nd choice-specific cells of the smoothing mode
+    size_t bytes = 0;     // device bytes of the allocations made at creation (cache policy)
+    double *d_qraw = 0;   // quadrature as passed (weights, abscissas)
+    double *d_stm = 0, *d_states = 0, *d_decisions = 0, *d_bparams = 0, *d_q = 0;
+    EgdstDev *d_self = 0; // copy of P in global memory (smoothing mode)
+    int *d_moff = 0, *d_toff = 0;
+    unsigned long long *d_phase = 0;  // per-phase device time of profiled solves
+    unsigned char *tab_base = 0;      // lookup tables (one allocation)
+    // grow-only buffers (grow)
+    double *d_pack = 0; size_t pack_cap = 0;                // export / import staging
+    double *d_momscratch = 0; size_t momscratch_cap = 0;    // per-CTA moment slices of the wide simulator variant
+    EgdstCellHdr *d_hdr = 0; size_t hdr_cap = 0;            // simulator cell headers
+    // every device allocation, by the field that holds it
+    std::vector<void **> owned{(void **)&d_pack, (void **)&d_momscratch, (void **)&d_hdr};
+    // state of the current owner (adopt)
     std::vector<int> h_mlen, h_thlen, h_status;
-    bool sizes_valid;
-    double *d_pack;  // export staging
-    size_t pack_cap;
-    int *d_moff, *d_toff;
-    int neq;
-    unsigned long long *d_phase;  // per-phase device time of profiled solves
-    int grid_ctas;  // CTAs of the solve kernel (one resident wave), 0 = not sized yet
-    bool cta_scope; // sweeps of many small models: one CTA (or warp) per parameter vector
-    int warp_groups; // > 0: WARP scope with this many warps (vectors) per CTA
-    int chC_alloc;  // scan windows per job the allocation provides
-    size_t bytes;   // device bytes owned (workspace cache policy)
-    void *tab_base; size_t tab_bytes;  // lookup tables (one allocation)
+    bool sizes_valid = false;
     std::vector<double> h_params;  // host copy of the parameter matrix of the last solve (simulator kernel arguments)
-    EgdstCellHdr *d_hdr; std::vector<EgdstCellHdr> h_hdr; int hdr_ivec;  // simulator cell headers (kernel argument), -1 = stale
-    double *d_momscratch; size_t momscratch_cap;  // per-CTA moment slices of the wide simulator variant
-    int dims[12];   // shape signature for re-use
-    double dkey[2]; // mmax, a0: the geometry of the lookup tables (mbits, lutcap) is derived from them at creation
+    std::vector<EgdstCellHdr> h_hdr; int hdr_ivec = -1;  // simulator cell headers (kernel argument), -1 = stale
 };
 
 template <class T>
 static cudaError_t dalloc(egdst_solution *s, T **p, size_t n) {
     cudaError_t e = cudaMalloc((void **)p, (n ? n : 1) * sizeof(T));
-    if (e == cudaSuccess) { s->owned.push_back((void *)*p); s->bytes += (n ? n : 1) * sizeof(T); }
+    if (e == cudaSuccess) { s->owned.push_back((void **)p); s->bytes += (n ? n : 1) * sizeof(T); }
     return e;
 }
 
@@ -138,10 +188,7 @@ static egdst_solution *g_cached = 0;
 static const size_t EGDST_CACHE_MAX_BYTES = (size_t)2 << 30;
 static void destroy_solution(egdst_solution *s) {
     cudaSetDevice(s->device);
-    for (void *p : s->owned) cudaFree(p);
-    if (s->d_pack) cudaFree(s->d_pack);
-    if (s->d_momscratch) cudaFree(s->d_momscratch);
-    if (s->d_hdr) cudaFree(s->d_hdr);
+    for (void **p : s->owned) if (*p) cudaFree(*p);
     delete s;
 }
 
@@ -191,50 +238,38 @@ static int check_device(int device) {
     return 0;
 }
 
-static int create_solution(const egdst_desc *d, int nvec, egdst_solution **out) {
-    egdst_ctx cx;
-    int rc = fill_ctx(d, &cx);
-    if (rc) return rc;
-    if ((rc = check_device(d->device))) return rc;
-    const bool smooth = d->sigma_eps > 0.0;  // taste-shock smoothing: choice-specific cells next to the solution cells
-    if (smooth && d->nd > EGDST_SMOOTH_MAXND) return fail(2, "sigma_eps > 0 supports at most 8 decisions");
-    if (d->sigma_eps < 0.0 || d->sigma_eps != d->sigma_eps) return fail(2, "sigma_eps must be >= 0");
-    const int dims[12] = {d->device, nvec, d->T - d->t0 + 1, d->nst, d->nd, d->ngridm, d->ngridmax, d->nthrhmax, d->ny, d->nnst, d->nnd, smooth ? 1 : 0};
-    {
-        std::lock_guard<std::mutex> lk(g_cache_mu);
-        if (g_cached && memcmp(g_cached->dims, dims, sizeof(dims)) == 0 && g_cached->dkey[0] == d->mmax && g_cached->dkey[1] == d->a0) {
-            egdst_solution *s = g_cached;
-            g_cached = 0;
-            // nothing of the previous owner survives: sizes, status, parameter values, simulator headers
-            s->sizes_valid = false; s->hdr_ivec = -1; s->neq = d->neq;
-            s->h_params.clear();
-            std::fill(s->h_status.begin(), s->h_status.end(), 0);
-            std::fill(s->h_mlen.begin(), s->h_mlen.end(), 0);
-            std::fill(s->h_thlen.begin(), s->h_thlen.end(), 0);
-            const double *stm = s->d_stm, *states = s->d_states, *decisions = s->d_decisions;
-            s->P.cx = cx; s->P.cx.stm = stm; s->P.cx.states = states; s->P.cx.decisions = decisions;
-            s->P.bparams = 0;
-            s->P.sigmaEps = d->sigma_eps;
-            cudaMemset(s->P.units, 0, sizeof(unsigned long long) * 2 * nvec);
-            *out = s;
-            return 0;
-        }
-    }
-    egdst_solution *s = new egdst_solution();
-    s->bytes = 0; memcpy(s->dims, dims, sizeof(dims)); s->dkey[0] = d->mmax; s->dkey[1] = d->a0;
-    s->d_momscratch = 0; s->momscratch_cap = 0; s->d_hdr = 0; s->hdr_ivec = -1;
-    s->grid_ctas = 0; s->cta_scope = false; s->warp_groups = 0;
-    s->device = d->device; s->sizes_valid = false; s->d_pack = 0; s->pack_cap = 0; s->neq = d->neq;
+static inline int imin(int a, int b) { return a < b ? a : b; }
+
+// the model of d (validated by fill_ctx into cx) becomes the model of s
+static void set_model(egdst_solution *s, const egdst_desc *d, egdst_ctx cx) {
+    cx.stm = s->d_stm; cx.states = s->d_states; cx.decisions = s->d_decisions;
+    s->P.cx = cx;
+    s->P.sigmaEps = d->sigma_eps;
+}
+
+// hand s to a new owner: nothing of a previous owner (sizes, status, parameter values, simulator headers) survives
+static void adopt(egdst_solution *s, const egdst_desc *d, const egdst_ctx &cx) {
+    set_model(s, d, cx);
+    s->P.bparams = 0;
+    cudaMemset(s->P.units, 0, sizeof(unsigned long long) * 2 * s->P.nvec);
+    s->h_mlen.assign(s->ncell, 0);
+    s->h_thlen.assign(s->ncell, 0);
+    s->h_status.assign(4 * s->P.nvec, 0);
+    s->sizes_valid = false;
+    s->h_params.clear();
+    s->hdr_ivec = -1;
+}
+
+// every device array of a new object of the shape of d with nvec parameter vectors (s->P.cx: the model of d)
+static int alloc_solution(egdst_solution *s, const egdst_desc *d, int nvec) {
     EgdstDev &P = s->P;
-    memset(&P, 0, sizeof(P));
-    P.cx = cx;
     P.NT = d->T - d->t0 + 1; P.nvec = nvec; P.rowcap = d->ngridmax + 2; P.gcap = d->ngridmax; P.N = d->ngridm;
     const int nst = d->nst, nd = d->nd;
     s->ncell = nvec * P.NT * nst; s->nsd = nvec * nst * nd; s->nslot = s->nsd + nvec * nst;
-    s->ncell_all = smooth ? s->ncell * (1 + nd) : s->ncell;
-    P.ncellMain = s->ncell; P.sigmaEps = d->sigma_eps;
+    s->ncell_all = d->sigma_eps > 0.0 ? s->ncell * (1 + nd) : s->ncell;
+    P.ncellMain = s->ncell;
     P.envcap = (nd > 2 ? nd : 2) * P.gcap + 2;
-#define DA(ptr, n) do { cudaError_t e_ = dalloc(s, &(ptr), (size_t)(n)); if (e_ != cudaSuccess) { destroy_solution(s); return fail(2, std::string("cudaMalloc failed: ") + cudaGetErrorString(e_)); } } while (0)
+#define DA(ptr, n) do { cudaError_t e_ = dalloc(s, &(ptr), (size_t)(n)); if (e_ != cudaSuccess) return fail(2, std::string("cudaMalloc failed: ") + cudaGetErrorString(e_)); } while (0)
     DA(s->d_stm, 2 * d->nnst); DA(s->d_states, nst * d->nnst); DA(s->d_decisions, nd * d->nnd);
     DA(s->d_bparams, (size_t)nvec * EGDST_NPARAM_); DA(s->d_qraw, 2 * d->ny); DA(s->d_q, 2 * d->ny);
     DA(P.tabOk, s->ncell_all);
@@ -247,15 +282,14 @@ static int create_solution(const egdst_desc *d, int nvec, egdst_solution **out) 
     DA(P.outX, (size_t)s->nsd * P.envcap); DA(P.outC, (size_t)s->nsd * P.envcap); DA(P.outV, (size_t)s->nsd * P.envcap);
     // lookup tables (egdst_tables.cuh): capacity 2*ngridm+64 intervals per cell, about two buckets per grid row
     P.tabcap = P.rowcap - 1 < 2 * P.N + 64 ? P.rowcap - 1 : 2 * P.N + 64;
-    if (getenv("EGDST_TABCAP")) { const int c = atoi(getenv("EGDST_TABCAP")); if (c >= 1 && c < P.tabcap) P.tabcap = c; }  // test hook: cells with more rows take the table-free path
+    if (s->hooks.tabcap >= 1 && s->hooks.tabcap < P.tabcap) P.tabcap = s->hooks.tabcap;
     {
         const double span = 2.0 * (d->mmax - d->a0) + 2.0;
         const double octaves = log2(span > 2.0 ? span : 2.0);
         int mbits = 3;
         // buckets per grid row: an index entry resolves up to three rows of a bucket by itself, so about one bucket
         // per row keeps the index small (the simulator wants every period's tables L2-resident next to its output stream)
-        static const double density = getenv("EGDST_LUT_DENSITY") ? atof(getenv("EGDST_LUT_DENSITY")) : 1.0;
-        while (mbits < 16 && (double)(1 << mbits) * octaves < density * (double)(P.N + 1)) mbits++;
+        while (mbits < 16 && (double)(1 << mbits) * octaves < (double)(P.N + 1)) mbits++;
         P.mbits = mbits;
         P.lutcap = (int)(octaves * (double)(1 << mbits)) + 2;
     }
@@ -263,16 +297,14 @@ static int create_solution(const egdst_desc *d, int nvec, egdst_solution **out) 
         const size_t lutbytes = ((sizeof(EgdstLutEntry) * (size_t)s->ncell_all * (P.lutcap + 1) + 255) / 256) * 256;
         const size_t ivlbytes = ((sizeof(EgdstRow) * (size_t)s->ncell_all * (P.tabcap + 1) + 255) / 256) * 256;
         const size_t topbytes = sizeof(EgdstCellTop) * (size_t)s->ncell_all;
-        unsigned char *base = 0;
-        DA(base, lutbytes + ivlbytes + topbytes);
-        P.tabLut = (EgdstLutEntry *)base; P.tabRow = (EgdstRow *)(base + lutbytes); P.tabTop = (EgdstCellTop *)(base + lutbytes + ivlbytes);
-        s->tab_base = base; s->tab_bytes = lutbytes + ivlbytes + topbytes;
+        DA(s->tab_base, lutbytes + ivlbytes + topbytes);
+        P.tabLut = (EgdstLutEntry *)s->tab_base; P.tabRow = (EgdstRow *)(s->tab_base + lutbytes); P.tabTop = (EgdstCellTop *)(s->tab_base + lutbytes + ivlbytes);
     }
     // chained scans: one state word per work item of a job plus the seed's slot (EGM phase: at least 8 grid points per
-    // item), one per chunk of EGDST_BLOCK union positions (envelope merge)
+    // item), one per chunk of union positions (envelope merge); the allocation serves the narrowest team (a warp),
+    // plan_solve sets the values of the scope
     P.chC = (P.N - 1 + 7) / 8 + 2;
-    s->chC_alloc = P.chC;
-    P.chE = (P.envcap + 31) / 32 + 1;  // allocation: the narrowest group (a warp); launch_solve sets the value of the scope
+    P.chE = (P.envcap + 31) / 32 + 1;
     // a point of the secondary envelope ranks itself against every run (~10^2 in the zig-zag periods of S1): with few
     // jobs, 8 threads share the runs of a point
     P.envA1parts = (nvec * nst * nd < 148) ? 8 : 1;
@@ -282,165 +314,176 @@ static int create_solution(const egdst_desc *d, int nvec, egdst_solution **out) 
     cudaMemset(s->d_phase, 0, sizeof(unsigned long long) * EGDST_NPHASE);
     DA(s->d_self, 1); DA(P.status, 4 * nvec); DA(P.units, 2 * nvec); DA(s->d_moff, s->ncell + 1); DA(s->d_toff, s->ncell + 1);
 #undef DA
-    cudaMemset(P.units, 0, sizeof(unsigned long long) * 2 * nvec);
-    P.cx.stm = s->d_stm; P.cx.states = s->d_states; P.cx.decisions = s->d_decisions;
     P.qw = s->d_q; P.qz = s->d_q + d->ny;
-    s->h_mlen.assign(s->ncell, 0); s->h_thlen.assign(s->ncell, 0); s->h_status.assign(4 * nvec, 0);
+    return 0;
+}
+
+// The launch of the solve kernel, chosen once per object.  Scope (egdst_period.cuh): sweeps of many small models run
+// a CTA (or a warp) per parameter vector, which walks its vector through all periods on its own; everything else is a
+// cooperative launch of exactly one resident wave whose CTAs share every phase of every period.
+static int plan_solve(egdst_solution *s) {
+    const EgdstDev &P = s->P;
+    const EgdstHooks &h = s->hooks;
+    SolvePlan &pl = s->plan;
+    const int nvec = P.nvec, N = P.N;
+    int sms = 1;  // the host emulator runs one CTA
+#ifndef EGDST_HOSTEMU
+    int dev = 0;
+    CK(cudaGetDevice(&dev));
+    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    // small models, many of them: a CTA (or warp) per vector keeps all of a vector's arrays in its SM's L1/L2
+    // neighbourhood and needs neither launches nor inter-CTA waits
+    if (nvec >= 2 * sms && N <= 4 * EGDST_BLOCK) pl.scope = nvec >= 8 * sms ? SCOPE_WARP : SCOPE_CTA;
+#endif
+    if (h.scope >= 0) pl.scope = h.scope;
+    // per-CTA table of quadrature shocks and node probabilities (models whose shocks cannot depend on savings)
+    const size_t shbytes = (size_t)2 * P.cx.nst * P.cx.ny * sizeof(double);
+    const size_t shtab = (EGDST_SHOCK_INDEP_A && shbytes <= EGDST_SHOCKTAB_BYTES) ? shbytes : 0;
+    // CTA and WARP scopes: a team of B threads takes the whole grid of a decision at a time (few scan windows), and the
+    // vector's small state fits shared memory; returns the bytes of that state
+    auto team = [&](int B) {
+        pl.block = B;
+        pl.chE = (P.envcap + B - 1) / B + 1;
+        pl.egmP = B < N - 1 ? B : (N - 1 < 8 ? 8 : N - 1);
+        if (h.egmP >= 8 && h.egmP <= B) pl.egmP = h.egmP;
+        pl.chC = imin(P.chC, (N - 1 + pl.egmP - 1) / pl.egmP + 2);
+        EgdstDev Q = P;
+        Q.chC = pl.chC;
+        Q.chE = pl.chE;
+        return egdst_cta_sync_bytes(Q);
+    };
+    if (pl.scope == SCOPE_WARP) {
+        const size_t sb = team(32);
+        pl.syncOff = (int)((EgdstScratch<32>::bytes + shtab + 15) / 16 * 16);
+        pl.groupBytes = (int)((pl.syncOff + sb + 127) / 128 * 128);
+        // as many warps per CTA as shared memory allows, and no more than spreads the vectors over all SMs
+        pl.warps = imin(imin((200 * 1024) / pl.groupBytes, EGDST_WARP_GROUPS), (nvec + sms - 1) / sms);
+        if (h.warpG >= 1 && h.warpG <= pl.warps) pl.warps = h.warpG;
+        pl.smem = (size_t)pl.groupBytes * pl.warps;
+        if (pl.warps < 4 && !h.warpGSet) pl.scope = SCOPE_CTA;  // too few warps per SM to hide anything
+    }
+    if (pl.scope == SCOPE_CTA) {
+        const size_t sb = team(EGDST_CTA_BLOCK);
+        pl.warps = 0;
+        pl.smem = EgdstScratch<EGDST_CTA_BLOCK>::bytes + shtab;
+        pl.syncOff = -1;
+        if (sb <= 6144) { pl.syncOff = (int)((pl.smem + 15) / 16 * 16); pl.smem = pl.syncOff + sb; }
+    }
+    if (pl.scope == SCOPE_GRID) {
+        pl.block = EGDST_BLOCK;
+        pl.chE = (P.envcap + EGDST_BLOCK - 1) / EGDST_BLOCK + 1;
+        pl.chC = P.chC;
+        pl.smem = EgdstScratch<EGDST_BLOCK>::bytes + shtab;
+    }
+    int occ = 1;
+#ifndef EGDST_HOSTEMU
+    const void *kern = pl.scope == SCOPE_WARP ? (const void *)egdst_k_solve_warps
+                       : pl.scope == SCOPE_CTA ? (const void *)egdst_k_solve_cta : (const void *)egdst_k_solve_grid;
+    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+    if (pl.scope != SCOPE_WARP && (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, pl.block, pl.smem) != cudaSuccess || occ < 1)) occ = 1;
+#endif
+    pl.ctas = sms * occ;
+    if (pl.scope != SCOPE_GRID) {
+        pl.ctas = imin(pl.ctas, pl.warps ? (nvec + pl.warps - 1) / pl.warps : nvec);  // no more CTAs than vectors to take
+    } else {
+        // grid points per work item of the EGM phase: the items of one period fill the grid exactly once (no tail wave)
+        const long long jobs = (long long)nvec * P.cx.nst * P.cx.nd;
+        int egmP = (int)(((long long)(N - 1) * jobs + pl.ctas - 1) / pl.ctas);
+        if (egmP < 8) egmP = 8;
+        if (egmP > EGDST_BLOCK) egmP = EGDST_BLOCK;
+        if (egmP > N - 1 && N - 1 >= 1) egmP = N - 1 < 8 ? 8 : N - 1;
+        if (h.egmP >= 8 && h.egmP <= EGDST_BLOCK) egmP = h.egmP;
+        pl.egmP = egmP;
+    }
+    if ((N - 1 + pl.egmP - 1) / pl.egmP + 2 > pl.chC) return fail(2, "internal: scan state too small for the EGM items");
+    pl.itStart = h.solveFrom >= 0 && h.solveFrom < P.NT - 1 ? h.solveFrom : P.NT - 1;
+    pl.itStop = h.solveTo >= 0 && h.solveTo <= pl.itStart ? h.solveTo : 0;
+    return 0;
+}
+
+static int create_solution(const egdst_desc *d, int nvec, egdst_solution **out) {
+    egdst_ctx cx;
+    int rc = fill_ctx(d, &cx);
+    if (rc) return rc;
+    if ((rc = check_device(d->device))) return rc;
+    const bool smooth = d->sigma_eps > 0.0;  // taste-shock smoothing: choice-specific cells next to the solution cells
+    if (smooth && d->nd > EGDST_SMOOTH_MAXND) return fail(2, "sigma_eps > 0 supports at most 8 decisions");
+    if (d->sigma_eps < 0.0 || d->sigma_eps != d->sigma_eps) return fail(2, "sigma_eps must be >= 0");
+    const int dims[12] = {d->device, nvec, d->T - d->t0 + 1, d->nst, d->nd, d->ngridm, d->ngridmax, d->nthrhmax, d->ny, d->nnst, d->nnd, smooth ? 1 : 0};
+    const EgdstHooks hooks = read_hooks();
+    egdst_solution *s = 0;
+    {
+        std::lock_guard<std::mutex> lk(g_cache_mu);
+        if (g_cached && memcmp(g_cached->dims, dims, sizeof(dims)) == 0 && g_cached->dkey[0] == d->mmax && g_cached->dkey[1] == d->a0 &&
+            memcmp(&g_cached->hooks, &hooks, sizeof(hooks)) == 0) {
+            s = g_cached;
+            g_cached = 0;
+        }
+    }
+    if (!s) {
+        s = new egdst_solution();
+        s->device = d->device; memcpy(s->dims, dims, sizeof(dims)); s->dkey[0] = d->mmax; s->dkey[1] = d->a0; s->hooks = hooks;
+        s->P.cx = cx;
+        if ((rc = alloc_solution(s, d, nvec)) || (rc = plan_solve(s))) { destroy_solution(s); return rc; }
+    }
+    adopt(s, d, cx);
     *out = s;
     return 0;
 }
 
-static inline int imin(int a, int b) { return a < b ? a : b; }
-
-// One backward-induction pass = one kernel on `st`.  Scope (egdst_period.cuh): sweeps of many small models run one CTA
-// per parameter vector (every CTA walks its vector through all periods on its own); everything else is a cooperative
-// launch of exactly one resident wave whose CTAs share every phase of every period.
+// One backward-induction pass = one kernel on `st`, launched as planned (plan_solve)
 static int launch_solve(egdst_solution *s, cudaStream_t st) {
     EgdstDev &P = s->P;
-    // test hook: keep the cells of the periods after EGDST_SOLVE_FROM (an imported solution) and solve from there down
-    P.itStart = P.NT - 1;
-    P.itStop = 0;
-    if (getenv("EGDST_SOLVE_FROM")) { const int k = atoi(getenv("EGDST_SOLVE_FROM")); if (k >= 0 && k < P.NT - 1) P.itStart = k; }
-    if (getenv("EGDST_SOLVE_TO")) { const int k = atoi(getenv("EGDST_SOLVE_TO")); if (k >= 0 && k <= P.itStart) P.itStop = k; }
+    const SolvePlan &pl = s->plan;
+    P.itStart = pl.itStart;
+    P.itStop = pl.itStop;
     CK(cudaMemsetAsync(P.status, 0, sizeof(int) * 4 * P.nvec, st));
     CK(cudaMemsetAsync(P.units, 0, sizeof(unsigned long long) * 2 * P.nvec, st));
+    CK(cudaMemsetAsync(P.bar, 0, sizeof(unsigned) * 4, st));
     if (P.itStart == P.NT - 1) {
         CK(cudaMemsetAsync(P.mlen, 0, sizeof(int) * s->ncell_all, st));
         CK(cudaMemsetAsync(P.thlen, 0, sizeof(int) * s->ncell, st));
+        CK(cudaMemsetAsync(P.tabOk, 1, sizeof(int) * s->ncell_all, st));  // non-zero: usable; cleared by the table build of a cell whose grid steps back
     }
-    CK(cudaMemsetAsync(P.bar, 0, sizeof(unsigned) * 4, st));
-    if (P.itStart == P.NT - 1) CK(cudaMemsetAsync(P.tabOk, 1, sizeof(int) * s->ncell_all, st));  // non-zero: usable; cleared by the table build of a cell whose grid steps back
-    const int nst = P.cx.nst, nd = P.cx.nd, nvec = P.nvec, N = P.N;
-    int B = EGDST_BLOCK;
-    P.priSync0 = nvec * nst * nd;
-    // per-CTA table of quadrature shocks and node probabilities (models whose shocks cannot depend on savings)
-    const size_t shbytes = (size_t)2 * nst * P.cx.ny * sizeof(double);
-    const size_t shtab = (EGDST_SHOCK_INDEP_A && shbytes <= EGDST_SHOCKTAB_BYTES) ? shbytes : 0;
-    size_t shsmem = 0;  // dynamic shared memory: phase scratch + shock table (+ the per-vector state of the CTA and WARP scopes)
-    int syncOff = -1, groupBytes = 0;
-    int dev = 0, sms = 1, occ = 1;
-    const bool first = !s->grid_ctas;
-    if (first) {
-        // small models, many of them: a CTA (or warp) per vector keeps all of a vector's arrays in its SM's L1/L2
-        // neighbourhood and needs neither launches nor inter-CTA waits
-        const char *scope_env = getenv("EGDST_SOLVE_SCOPE");  // test hook: "grid" / "cta" / "warp"
-#ifndef EGDST_HOSTEMU
-        CK(cudaGetDevice(&dev));
-        CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-        s->cta_scope = nvec >= 2 * sms && N <= 4 * B;
-        s->warp_groups = s->cta_scope && nvec >= 8 * sms ? EGDST_WARP_GROUPS : 0;
-#else
-        s->cta_scope = false; s->warp_groups = 0;
-#endif
-        if (scope_env) { s->cta_scope = strcmp(scope_env, "grid") != 0; s->warp_groups = strcmp(scope_env, "warp") == 0 ? EGDST_WARP_GROUPS : 0; }
-    }
-    for (bool again = true; again;) {
-        again = false;
-        B = s->cta_scope ? (s->warp_groups ? 32 : EGDST_CTA_BLOCK) : EGDST_BLOCK;
-        P.chE = (P.envcap + B - 1) / B + 1;
-        P.chC = s->chC_alloc;
-        if (!s->cta_scope) { shsmem = EgdstScratch<EGDST_BLOCK>::bytes + shtab; break; }
-        // a CTA takes the whole grid of a decision at a time: few scan windows, and the vector's small state fits shared memory
-        int p = B < N - 1 ? B : (N - 1 < 8 ? 8 : N - 1);
-        if (getenv("EGDST_EGM_P")) { const int q = atoi(getenv("EGDST_EGM_P")); if (q >= 8 && q <= B) p = q; }  // test hook
-        P.egmP = p;
-        const int need = (N - 1 + p - 1) / p + 2;
-        if (need < P.chC) P.chC = need;
-        const size_t sb = egdst_cta_sync_bytes(P);
-        if (s->warp_groups) {
-            syncOff = (int)((EgdstScratch<32>::bytes + shtab + 15) / 16 * 16);
-            groupBytes = (int)((syncOff + sb + 127) / 128 * 128);
-            if (first) {
-                // as many warps per CTA as shared memory allows, and no more than spreads the vectors over all SMs
-                int g = (int)((200 * 1024) / groupBytes);
-                if (g > EGDST_WARP_GROUPS) g = EGDST_WARP_GROUPS;
-                const int even = (nvec + sms - 1) / sms;
-                if (even < g) g = even;
-                if (getenv("EGDST_WARP_G")) { const int q = atoi(getenv("EGDST_WARP_G")); if (q >= 1 && q <= g) g = q; }  // test hook
-                if (g < 4 && !getenv("EGDST_WARP_G")) { s->warp_groups = 0; again = true; continue; }  // too few warps per SM to hide anything: CTA scope
-                s->warp_groups = g;
-            }
-            shsmem = (size_t)groupBytes * s->warp_groups;
-        } else {
-            shsmem = EgdstScratch<EGDST_CTA_BLOCK>::bytes + shtab;
-            static const char *nosm = getenv("EGDST_CTA_SYNC_GLOBAL");  // measurement hook
-            syncOff = -1;
-            if (sb <= 6144 && !nosm) { syncOff = (int)((shsmem + 15) / 16 * 16); shsmem = syncOff + sb; }
-        }
-    }
-    if (first) {
-#ifndef EGDST_HOSTEMU
-        if (s->warp_groups) {
-            CK(cudaFuncSetAttribute(egdst_k_solve_warps, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shsmem));
-            occ = 1;
-        } else if (s->cta_scope) {
-            CK(cudaFuncSetAttribute(egdst_k_solve_cta, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shsmem));
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, egdst_k_solve_cta, EGDST_CTA_BLOCK, shsmem) != cudaSuccess || occ < 1) occ = 1;
-        } else {
-            CK(cudaFuncSetAttribute(egdst_k_solve_grid, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shsmem));
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, egdst_k_solve_grid, B, shsmem) != cudaSuccess || occ < 1) occ = 1;
-        }
-#endif
-        s->grid_ctas = sms * occ;
-        const int owners = s->warp_groups ? (nvec + s->warp_groups - 1) / s->warp_groups : nvec;
-        if (s->cta_scope && s->grid_ctas > owners) s->grid_ctas = owners;
-        if (getenv("EGDST_SOLVE_CTAS")) { const int g = atoi(getenv("EGDST_SOLVE_CTAS")); if (g >= 1 && g < s->grid_ctas) s->grid_ctas = g; }  // test hook
-    }
-    (void)dev;
-    if (!s->cta_scope) {
-        // grid points per work item of the EGM phase: the items of one period fill the grid exactly once (no tail wave)
-        const int G = s->grid_ctas;
-        long long jobs = (long long)nvec * nst * nd;
-        int egmP = (int)(((long long)(N - 1) * jobs + G - 1) / G);
-        if (egmP < 8) egmP = 8;
-        if (egmP > B) egmP = B;
-        if (egmP > N - 1 && N - 1 >= 1) egmP = N - 1 < 8 ? 8 : N - 1;
-        if (getenv("EGDST_EGM_P")) { const int p = atoi(getenv("EGDST_EGM_P")); if (p >= 8 && p <= B) egmP = p; }  // test hook
-        P.egmP = egmP;
-    }
+    P.priSync0 = P.nvec * P.cx.nst * P.cx.nd;
+    P.egmP = pl.egmP; P.chC = pl.chC; P.chE = pl.chE;
     P.self = s->d_self;
     P.phase_ns = g_prof_on ? s->d_phase : 0;  // measurement aid: in-kernel phase timers while profiling is enabled
-    if ((N - 1 + P.egmP - 1) / P.egmP + 2 > P.chC) return fail(2, "internal: scan state too small for the EGM items");
     if (EGDST_SMOOTHING) CK(cudaMemcpyAsync(s->d_self, &P, sizeof(EgdstDev), cudaMemcpyHostToDevice, st));  // read by egdst_smooth_node
+    switch (pl.scope) {
+    case SCOPE_WARP: KLAUNCH(KC_SOLVE, egdst_k_solve_warps, dim3(pl.ctas), dim3(32, pl.warps), pl.smem, st, P, pl.syncOff, pl.groupBytes); break;
+    case SCOPE_CTA: KLAUNCH(KC_SOLVE, egdst_k_solve_cta, dim3(pl.ctas), dim3(pl.block), pl.smem, st, P, pl.syncOff); break;
+    default: {
 #ifndef EGDST_HOSTEMU
-    prof_begin(KC_SOLVE, st);
-    if (s->warp_groups) {
-        egdst_k_solve_warps<<<s->grid_ctas, dim3(32, s->warp_groups), shsmem, st>>>(P, syncOff, groupBytes);
-    } else if (s->cta_scope) {
-        egdst_k_solve_cta<<<s->grid_ctas, B, shsmem, st>>>(P, syncOff);
-    } else {
         void *args[] = {(void *)&P};
-        CK(cudaLaunchCooperativeKernel((const void *)egdst_k_solve_grid, dim3(s->grid_ctas), dim3(B), args, shsmem, st));
-    }
-    prof_end(st);
+        prof_begin(KC_SOLVE, st);
+        CK(cudaLaunchCooperativeKernel((const void *)egdst_k_solve_grid, dim3(pl.ctas), dim3(pl.block), args, pl.smem, st));
+        prof_end(st);
 #else
-    if (s->warp_groups) { KLAUNCH(KC_SOLVE, egdst_k_solve_warps, dim3(s->grid_ctas), dim3(32, s->warp_groups), shsmem, st, P, syncOff, groupBytes); }
-    else if (s->cta_scope) { KLAUNCH(KC_SOLVE, egdst_k_solve_cta, dim3(s->grid_ctas), dim3(B), shsmem, st, P, syncOff); }
-    else { KLAUNCH(KC_SOLVE, egdst_k_solve_grid, dim3(1), dim3(B), shsmem, st, P); }
+        KLAUNCH(KC_SOLVE, egdst_k_solve_grid, dim3(pl.ctas), dim3(pl.block), pl.smem, st, P);
 #endif
+    }
+    }
     CK(cudaGetLastError());
     return 0;
 }
 
-// one backward-induction pass; asynchronous
+// the model tables of d (stm, states, decisions) to the device copies of s
+static cudaError_t upload_tables(egdst_solution *s, const egdst_desc *d, cudaStream_t st) {
+    cudaError_t ce = cudaSuccess;
+    EGDST_TRY(cudaMemcpyAsync(s->d_stm, d->stm, sizeof(double) * 2 * d->nnst, cudaMemcpyHostToDevice, st));
+    EGDST_TRY(cudaMemcpyAsync(s->d_states, d->states, sizeof(double) * d->nst * d->nnst, cudaMemcpyHostToDevice, st));
+    EGDST_TRY(cudaMemcpyAsync(s->d_decisions, d->decisions, sizeof(double) * d->nd * d->nnd, cudaMemcpyHostToDevice, st));
+    return ce;
+}
+
+// one backward-induction pass of the model in s->P.cx (d: its descriptor); asynchronous
 static int run_solve(egdst_solution *s, const egdst_desc *d, const double *params) {
     EgdstDev &P = s->P;
-    egdst_ctx cx;
-    int rc = fill_ctx(d, &cx);
-    if (rc) return rc;
     if (d->ny > 1 && !d->quadrature) return fail(2, "quadrature missing");
-    if (d->ngridm != P.N || d->ngridmax != P.gcap || d->T - d->t0 + 1 != P.NT || d->nst != P.cx.nst || d->nd != P.cx.nd ||
-        d->ny != P.cx.ny || d->nthrhmax != P.cx.nthrhmax)
-        return fail(2, "egdst_resolve: dimensions differ from the solution object");
     CK(cudaSetDevice(s->device));
-    cx.stm = s->d_stm; cx.states = s->d_states; cx.decisions = s->d_decisions;
-    P.cx = cx;
-    if ((d->sigma_eps > 0.0) != (s->ncell_all > s->ncell)) return fail(2, "egdst_resolve: sigma_eps switches the smoothing mode on or off; solve anew");
-    P.sigmaEps = d->sigma_eps;
     cudaStream_t st = g_stream;
-    CK(cudaMemcpyAsync(s->d_stm, d->stm, sizeof(double) * 2 * d->nnst, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(s->d_states, d->states, sizeof(double) * d->nst * d->nnst, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(s->d_decisions, d->decisions, sizeof(double) * d->nd * d->nnd, cudaMemcpyHostToDevice, st));
+    CK(upload_tables(s, d, st));
     // parameter values always travel through the device array (one row per vector), never through the kernel
     // arguments: the argument block then depends on the shape only
     if (!params && P.nvec != 1) return fail(2, "egdst_resolve: a batched solution needs the parameter matrix");
@@ -452,7 +495,7 @@ static int run_solve(egdst_solution *s, const egdst_desc *d, const double *param
         CK(cudaMemcpyAsync(s->d_qraw, d->quadrature, sizeof(double) * 2 * d->ny, cudaMemcpyHostToDevice, st));
         KLAUNCH(KC_SETUP, egdst_k_quadrature, dim3((d->ny + 127) / 128), dim3(128), 0, st, s->d_qraw, s->d_q, d->ny);
     }
-    rc = launch_solve(s, st);
+    int rc = launch_solve(s, st);
     if (rc) return rc;
     s->sizes_valid = false;
     s->hdr_ivec = -1;
@@ -516,6 +559,34 @@ __global__ void egdst_k_unpack(EgdstDev P, const int *moff, const int *toff, con
     if (threadIdx.x == 0 && n > 0) P.evf[cell] = src[3 * n];
 }
 
+// offsets of the cells in the packed layout (rows mlen, thresholds thlen) to the device, and a pack buffer that holds
+// the layout's nm M values and nd2 D values
+static int pack_layout(egdst_solution *s, const int *mlen, const int *thlen, size_t *nm, size_t *nd2) {
+    std::vector<int> moff(s->ncell + 1, 0), toff(s->ncell + 1, 0);
+    for (int c = 0; c < s->ncell; c++) { moff[c + 1] = moff[c] + mlen[c]; toff[c + 1] = toff[c] + thlen[c]; }
+    *nm = (size_t)4 * moff[s->ncell];
+    *nd2 = (size_t)2 * toff[s->ncell];
+    CK(grow(&s->d_pack, &s->pack_cap, *nm + *nd2));
+    CK(cudaMemcpyAsync(s->d_moff, moff.data(), sizeof(int) * (s->ncell + 1), cudaMemcpyHostToDevice, g_stream));
+    CK(cudaMemcpyAsync(s->d_toff, toff.data(), sizeof(int) * (s->ncell + 1), cudaMemcpyHostToDevice, g_stream));
+    return 0;
+}
+
+// sum over the vectors of row `row` of P.units (0: solve work units, 1: re-sends); -1 on error
+static long long units_sum(egdst_solution *s, int row) {
+    if (!s) return -1;
+    if (cudaSetDevice(s->device) != cudaSuccess) return -1;
+    std::vector<unsigned long long> u(s->P.nvec, 0ULL);
+    if (cudaMemcpyAsync(u.data(), s->P.units + (size_t)row * s->P.nvec, sizeof(unsigned long long) * s->P.nvec, cudaMemcpyDeviceToHost, g_stream) != cudaSuccess) return -1;
+    if (cudaStreamSynchronize(g_stream) != cudaSuccess) return -1;
+    long long tot = 0;
+    for (unsigned long long x : u) tot += (long long)x;
+    return tot;
+}
+
+// frees a scratch or failed solution object (egdst_free_solution) on every return that does not release it
+typedef std::unique_ptr<egdst_solution, void (*)(egdst_solution *)> SolutionGuard;
+
 extern "C" {
 
 int egdst_abi_version(void) { return EGDST_ABI_VERSION; }
@@ -544,13 +615,10 @@ int egdst_solve_batch(const egdst_desc *d, const double *params, int nvec, egdst
     egdst_solution *s = 0;
     int rc = create_solution(d, nvec, &s);
     if (rc) return rc;
-    rc = run_solve(s, d, params);
-    if (rc) { egdst_free_solution(s); return rc; }
-    rc = fetch_sizes(s);
-    if (rc) { egdst_free_solution(s); return rc; }
-    *out = s;
+    SolutionGuard guard(s, egdst_free_solution);
+    if ((rc = run_solve(s, d, params)) || (rc = fetch_sizes(s))) return rc;
     rc = status_rc(s);
-    if (rc == 2) { egdst_free_solution(s); *out = 0; }
+    if (rc != 2) *out = guard.release();
     return rc;
 }
 
@@ -558,6 +626,15 @@ int egdst_solve(const egdst_desc *d, egdst_solution **out) { return egdst_solve_
 
 int egdst_resolve(egdst_solution *s, const egdst_desc *d, const double *params) {
     if (!s) return fail(2, "null solution");
+    egdst_ctx cx;
+    int rc = fill_ctx(d, &cx);
+    if (rc) return rc;
+    const EgdstDev &P = s->P;
+    if (d->ngridm != P.N || d->ngridmax != P.gcap || d->T - d->t0 + 1 != P.NT || d->nst != P.cx.nst || d->nd != P.cx.nd ||
+        d->ny != P.cx.ny || d->nthrhmax != P.cx.nthrhmax)
+        return fail(2, "egdst_resolve: dimensions differ from the solution object");
+    if ((d->sigma_eps > 0.0) != (s->ncell_all > s->ncell)) return fail(2, "egdst_resolve: sigma_eps switches the smoothing mode on or off; solve anew");
+    set_model(s, d, cx);
     return run_solve(s, d, params);
 }
 
@@ -572,20 +649,10 @@ int egdst_solution_sizes(egdst_solution *s, int *mlen, int *thlen) {
 
 int egdst_solution_export(egdst_solution *s, double *Mbuf, double *Dbuf) {
     if (!s || !Mbuf || !Dbuf) return fail(2, "invalid arguments");
+    size_t nm = 0, nd2 = 0;
     int rc = fetch_sizes(s);
-    if (rc) return rc;
-    std::vector<int> moff(s->ncell + 1, 0), toff(s->ncell + 1, 0);
-    for (int c = 0; c < s->ncell; c++) { moff[c + 1] = moff[c] + s->h_mlen[c]; toff[c + 1] = toff[c] + s->h_thlen[c]; }
-    const size_t nm = (size_t)4 * moff[s->ncell], nd2 = (size_t)2 * toff[s->ncell];
+    if (rc || (rc = pack_layout(s, s->h_mlen.data(), s->h_thlen.data(), &nm, &nd2))) return rc;
     cudaStream_t st = g_stream;
-    if (nm + nd2 > s->pack_cap) {
-        if (s->d_pack) cudaFree(s->d_pack);
-        s->d_pack = 0; s->pack_cap = 0;
-        CK(cudaMalloc((void **)&s->d_pack, sizeof(double) * (nm + nd2 + 1)));
-        s->pack_cap = nm + nd2;
-    }
-    CK(cudaMemcpyAsync(s->d_moff, moff.data(), sizeof(int) * (s->ncell + 1), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(s->d_toff, toff.data(), sizeof(int) * (s->ncell + 1), cudaMemcpyHostToDevice, st));
     KLAUNCH(KC_OTHER, egdst_k_pack, dim3(s->ncell), dim3(EGDST_BLOCK), 0, st, s->P, s->d_moff, s->d_toff, s->d_pack, s->d_pack + nm, s->ncell);
     CK(cudaMemcpyAsync(Mbuf, s->d_pack, sizeof(double) * nm, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(Dbuf, s->d_pack + nm, sizeof(double) * nd2, cudaMemcpyDeviceToHost, st));
@@ -625,31 +692,13 @@ int egdst_solution_status(egdst_solution *s, int ivec, int *it, int *ist, int *i
 
 int egdst_solution_nvec(const egdst_solution *s) { return s ? s->P.nvec : 0; }
 
-long long egdst_solution_units(egdst_solution *s) {
-    // the solve work unit (SURVEY 8d): every EGM grid point stored for an (it, ist, id) -- the mgridvecs
-    // quadruples of egdst_solver.c:646-650, terminal period included; counted on the device by the kernels.
-    if (!s) return -1;
-    if (cudaSetDevice(s->device) != cudaSuccess) return -1;
-    std::vector<unsigned long long> u(s->P.nvec, 0ULL);
-    if (cudaMemcpyAsync(u.data(), s->P.units, sizeof(unsigned long long) * s->P.nvec, cudaMemcpyDeviceToHost, g_stream) != cudaSuccess) return -1;
-    if (cudaStreamSynchronize(g_stream) != cudaSuccess) return -1;
-    long long tot = 0;
-    for (unsigned long long x : u) tot += (long long)x;
-    return tot;
-}
+// the solve work unit (SURVEY 8d): every EGM grid point stored for an (it, ist, id) -- the mgridvecs
+// quadruples of egdst_solver.c:646-650, terminal period included; counted on the device by the kernels.
+long long egdst_solution_units(egdst_solution *s) { return units_sum(s, 0); }
 
-long long egdst_solution_resends(egdst_solution *s) {
-    // diagnostic: zero-consumption re-sends requested by grid points after the seed stage (egdst_solver.c:1080-1099)
-    // that the last solve handled, over all vectors
-    if (!s) return -1;
-    if (cudaSetDevice(s->device) != cudaSuccess) return -1;
-    std::vector<unsigned long long> u(s->P.nvec, 0ULL);
-    if (cudaMemcpyAsync(u.data(), s->P.units + s->P.nvec, sizeof(unsigned long long) * s->P.nvec, cudaMemcpyDeviceToHost, g_stream) != cudaSuccess) return -1;
-    if (cudaStreamSynchronize(g_stream) != cudaSuccess) return -1;
-    long long tot = 0;
-    for (unsigned long long x : u) tot += (long long)x;
-    return tot;
-}
+// diagnostic: zero-consumption re-sends requested by grid points after the seed stage (egdst_solver.c:1080-1099)
+// that the last solve handled, over all vectors
+long long egdst_solution_resends(egdst_solution *s) { return units_sum(s, 1); }
 
 int egdst_solution_phase_ms(egdst_solution *s, double *ms) {
     // device time per phase of the solve kernel (terminal, seed, egm, resend, envelope2, rank, merge, tables), accumulated over
@@ -674,13 +723,10 @@ int egdst_test_envelope2(const egdst_desc *d, int it, int ist, int id, const dou
     egdst_solution *s = 0;
     int rc = create_solution(d, 1, &s);
     if (rc) return rc;
-    EgdstDev P = s->P;
+    SolutionGuard scratch(s, egdst_free_solution);
+    const EgdstDev &P = s->P;
     cudaStream_t st = g_stream;
-    cudaError_t ce = cudaSuccess;
-#define EGDST_TRY(call) do { if (ce == cudaSuccess) ce = (call); } while (0)
-    EGDST_TRY(cudaMemcpyAsync(s->d_stm, d->stm, sizeof(double) * 2 * d->nnst, cudaMemcpyHostToDevice, st));
-    EGDST_TRY(cudaMemcpyAsync(s->d_states, d->states, sizeof(double) * d->nst * d->nnst, cudaMemcpyHostToDevice, st));
-    EGDST_TRY(cudaMemcpyAsync(s->d_decisions, d->decisions, sizeof(double) * d->nd * d->nnd, cudaMemcpyHostToDevice, st));
+    cudaError_t ce = upload_tables(s, d, st);
     // the decision's slot is sd = 0 of the scratch object; its decision index travels in the view (ist = 0 => sd = id):
     // place the points in the slot of (ist 0, id) so that the analytic segment uses the right decision
     const size_t off = (size_t)id * P.gcap;
@@ -691,7 +737,6 @@ int egdst_test_envelope2(const egdst_desc *d, int it, int ist, int id, const dou
     EGDST_TRY(cudaMemcpyAsync(P.evfa0 + id, &evfa0, sizeof(double), cudaMemcpyHostToDevice, st));
     int nres = 0;
     if (ce == cudaSuccess) {
-        P.bparams = 0;
         KLAUNCH(KC_OTHER, egdst_k_env2_only, dim3(1), dim3(EGDST_BLOCK), EgdstScratch<EGDST_BLOCK>::bytes, st, P, it, n, id);
         EGDST_TRY(cudaGetLastError());
         EGDST_TRY(cudaMemcpyAsync(&nres, P.ptN + id, sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -703,14 +748,9 @@ int egdst_test_envelope2(const egdst_desc *d, int it, int ist, int id, const dou
         EGDST_TRY(cudaMemcpyAsync(outV, P.ptV + off, sizeof(double) * nres, cudaMemcpyDeviceToHost, st));
         EGDST_TRY(cudaStreamSynchronize(st));
     }
-#undef EGDST_TRY
-    if (ce != cudaSuccess) { egdst_free_solution(s); return fail(2, std::string("CUDA error in egdst_test_envelope2: ") + cudaGetErrorString(ce)); }
+    if (ce != cudaSuccess) return fail(2, std::string("CUDA error in egdst_test_envelope2: ") + cudaGetErrorString(ce));
     *nout = nres;
-    s->sizes_valid = false;
-    rc = fetch_sizes(s);
-    if (!rc) rc = status_rc(s);
-    egdst_free_solution(s);
-    return rc;
+    return (rc = fetch_sizes(s)) ? rc : status_rc(s);
 }
 
 void egdst_free_solution(egdst_solution *s) {
@@ -729,31 +769,19 @@ int egdst_solution_import(const egdst_desc *d, const int *mlen, const int *thlen
     egdst_solution *s = 0;
     int rc = create_solution(d, 1, &s);
     if (rc) return rc;
-    std::vector<int> moff(s->ncell + 1, 0), toff(s->ncell + 1, 0);
+    SolutionGuard guard(s, egdst_free_solution);
     for (int c = 0; c < s->ncell; c++) {
-        if (mlen[c] > s->P.rowcap || thlen[c] > d->nthrhmax) { egdst_free_solution(s); return fail(2, "imported cell exceeds ngridmax/nthrhmax"); }
-        if (mlen[c] < 0 || mlen[c] == 1 || thlen[c] < 0 || (mlen[c] == 0) != (thlen[c] == 0)) { egdst_free_solution(s); return fail(2, "imported cell has an invalid number of rows"); }
-        moff[c + 1] = moff[c] + mlen[c]; toff[c + 1] = toff[c] + thlen[c];
+        if (mlen[c] > s->P.rowcap || thlen[c] > d->nthrhmax) return fail(2, "imported cell exceeds ngridmax/nthrhmax");
+        if (mlen[c] < 0 || mlen[c] == 1 || thlen[c] < 0 || (mlen[c] == 0) != (thlen[c] == 0)) return fail(2, "imported cell has an invalid number of rows");
     }
-    const size_t nm = (size_t)4 * moff[s->ncell], nd2 = (size_t)2 * toff[s->ncell];
+    size_t nm = 0, nd2 = 0;
+    if ((rc = pack_layout(s, mlen, thlen, &nm, &nd2))) return rc;
     cudaStream_t st = g_stream;
-    if (nm + nd2 > s->pack_cap || !s->d_pack) {
-        if (s->d_pack) cudaFree(s->d_pack);
-        s->d_pack = 0; s->pack_cap = 0;
-        if (cudaMalloc((void **)&s->d_pack, sizeof(double) * (nm + nd2 + 1)) != cudaSuccess) { egdst_free_solution(s); return fail(2, "cudaMalloc failed"); }
-        s->pack_cap = nm + nd2;
-    }
-    cudaError_t ce = cudaSuccess;
-#define EGDST_TRY(call) do { if (ce == cudaSuccess) ce = (call); } while (0)
+    cudaError_t ce = upload_tables(s, d, st);
     EGDST_TRY(cudaMemcpyAsync(s->d_pack, Mbuf, sizeof(double) * nm, cudaMemcpyHostToDevice, st));
     EGDST_TRY(cudaMemcpyAsync(s->d_pack + nm, Dbuf, sizeof(double) * nd2, cudaMemcpyHostToDevice, st));
     EGDST_TRY(cudaMemcpyAsync(s->P.mlen, mlen, sizeof(int) * s->ncell, cudaMemcpyHostToDevice, st));
     EGDST_TRY(cudaMemcpyAsync(s->P.thlen, thlen, sizeof(int) * s->ncell, cudaMemcpyHostToDevice, st));
-    EGDST_TRY(cudaMemcpyAsync(s->d_moff, moff.data(), sizeof(int) * (s->ncell + 1), cudaMemcpyHostToDevice, st));
-    EGDST_TRY(cudaMemcpyAsync(s->d_toff, toff.data(), sizeof(int) * (s->ncell + 1), cudaMemcpyHostToDevice, st));
-    EGDST_TRY(cudaMemcpyAsync(s->d_stm, d->stm, sizeof(double) * 2 * d->nnst, cudaMemcpyHostToDevice, st));
-    EGDST_TRY(cudaMemcpyAsync(s->d_states, d->states, sizeof(double) * d->nst * d->nnst, cudaMemcpyHostToDevice, st));
-    EGDST_TRY(cudaMemcpyAsync(s->d_decisions, d->decisions, sizeof(double) * d->nd * d->nnd, cudaMemcpyHostToDevice, st));
     EGDST_TRY(cudaMemsetAsync(s->P.status, 0, sizeof(int) * 4, st));
     EGDST_TRY(cudaMemsetAsync(s->P.tabOk, 1, sizeof(int) * s->ncell_all, st));  // imported cells: usable unless egdst_k_tabonly finds a grid that steps back
     if (ce == cudaSuccess) {
@@ -763,15 +791,12 @@ int egdst_solution_import(const egdst_desc *d, const int *mlen, const int *thlen
         EGDST_TRY(cudaGetLastError());
     }
     EGDST_TRY(cudaStreamSynchronize(st));
-#undef EGDST_TRY
-    if (ce != cudaSuccess) { egdst_free_solution(s); return fail(2, std::string("CUDA error in import: ") + cudaGetErrorString(ce)); }
+    if (ce != cudaSuccess) return fail(2, std::string("CUDA error in import: ") + cudaGetErrorString(ce));
     memcpy(s->h_mlen.data(), mlen, sizeof(int) * s->ncell);
     memcpy(s->h_thlen.data(), thlen, sizeof(int) * s->ncell);
-    std::fill(s->h_status.begin(), s->h_status.end(), 0);
     s->h_params.assign(d->params, d->params + EGDST_NPARAM);  // the imported model's own parameter values
-    s->P.bparams = 0;
     s->sizes_valid = true;
-    *out = s;
+    *out = guard.release();
     return 0;
 }
 

@@ -370,10 +370,6 @@ EGDST_DEV void egdst_eval_nodes(const egdst_ctx *cx, const EgdstDev &P, int ivec
                     acc.evf += pb * fb.v1;
                     continue;
                 }
-#ifdef EGDST_HOSTEMU
-                if (getenv("EGDST_DEBUG_SLOW") && curr->it == atoi(getenv("EGDST_DEBUG_SLOW")))
-                    printf("slow it=%d id=%d A=%.6f qa=%d cash=%.9f/%.9f ok=%d/%d ia=%d ib=%d c1=%.3g/%.3g n1=%d top=%.9f\n", curr->it, curr->id, A, qa, fa.cash, fb.cash, (int)fa.ok, (int)fb.ok, ia, ib, fa.c1, fb.c1, t.n1, top.g1);
-#endif
                 // general path, one node after the other
                 if (pa != 0.0) { next.shock = sa; if (!egdst_eval_node(cx, P, t, tab, curr, next, keep, qa, pa, acc)) break; }
                 if (pb != 0.0) {
@@ -956,9 +952,6 @@ EGDST_DEV void egdst_ph_resend(const EgdstDev &P, int it, const EgdstTeam &T, in
         if (kept > P.gcap) kept = P.gcap;
         const double baseA = seed[8], baseM = seed[9];
         if (threadIdx.x == 0) { S.A = egdst_agrid(&cx, &curr, seed, nl, N); S.calls = (int)seed[7]; S.go = 1; }
-#ifdef EGDST_HOSTEMU
-        if (threadIdx.x == 0 && getenv("EGDST_DEBUG_RESEND")) printf("re-send after the seed stage: it=%d ist=%d id=%d at grid point %d (A=%.12g), %d points kept before it\n", it, ist, id, nl, S.A, kept);
-#endif
         egdst_cta_sync();
         EgdstLims L; L.lim1 = seed[0]; L.lim2 = seed[1]; L.lim3 = seed[2]; L.lim3p = seed[3]; L.k3 = seed[4]; L.lim2p = 0;
         double lastA = 0, aM = 0;
