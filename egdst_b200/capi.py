@@ -163,12 +163,11 @@ class Solution:
     def units(self) -> int:
         return int(self.lib.L.egdst_solution_units(self.handle))
 
-    PHASES = ("terminal", "seed", "egm", "resend", "envelope2", "rank", "merge", "tables",
-              "egm.setup", "egm.nodes", "egm.combine", "egm.lookback", "egm.write", "egm.epilogue", "-", "--")
+    PHASES = ("terminal", "seed", "egm", "resend", "envelope2", "rank", "merge", "tables")
 
     def phase_ms(self):
         """{phase: ms} of the solve kernel, accumulated over profiled solves of this object (reading resets)."""
-        ms = (C.c_double * 16)()
+        ms = (C.c_double * len(self.PHASES))()
         n = self.lib.L.egdst_solution_phase_ms(self.handle, ms)
         return {self.PHASES[i]: float(ms[i]) for i in range(max(n, 0))}
 

@@ -29,7 +29,7 @@
 
 #define EGDST_FULL 0xffffffffu
 #define EGDST_SEEDW 12
-#define EGDST_NPHASE 16  /* terminal, seed, egm, resend, envelope2, rank, merge, tables; then the steps of the last EGM work item */
+#define EGDST_NPHASE 8  /* terminal, seed, egm, resend, envelope2, rank, merge, tables */
 #define EGDST_SHOCKTAB_BYTES (40 * 1024)  /* per-CTA table of quadrature shocks and node probabilities (dynamic shared memory) */
 #ifdef EGDST_HOSTEMU
 #define EGDST_SOLVE_MINB 1

@@ -45,6 +45,14 @@ EGDST_DEV int egdst_optimd(double m, const double *__restrict__ th, const double
     if (nth <= 1) return (int)dd[0];  // the reference reads grid[1] here (SURVEY 8a quirks); one threshold => one choice
     return (int)dd[egdst_bracket(m, th, nth, 1)];
 }
+// The decision of policy() for the simulator and call() (egdst_simulator.c:145-199): a linear scan for the last
+// threshold <= m (the first decision below every threshold).  The reference's solver uses the bisection of optimd
+// instead; the two agree on increasing thresholds but not on others, so each path keeps its reference's rule.
+EGDST_DEV int egdst_policy_decision(double m, const double *th, const double *dd, int nth) {
+    int ith = 0;
+    while (ith < nth && m >= th[ith]) ith++;
+    return (int)dd[ith > 0 ? ith - 1 : 0];
+}
 
 // linear interpolation / extrapolation on interval i (egdst_lib.c:175)
 EGDST_DEV double egdst_lerp(double x, double g0, double g1, double f0, double f1) {

@@ -216,18 +216,13 @@ __global__ void __launch_bounds__(EGDST_BLOCK, EGDST_SOLVE_MINB) egdst_k_env2_on
     egdst_cta_sync();
     const int sd = id;  // ist = 0
     const double *X = P.ptX + (size_t)sd * P.gcap, *V = P.ptV + (size_t)sd * P.gcap;
-    int *runStart = P.runStart + (size_t)sd * (P.gcap + 1), *foldList = P.foldList + (size_t)sd * (P.gcap + 1);
+    int *foldList = P.foldList + (size_t)sd * (P.gcap + 1);
     for (int p = 1 + threadIdx.x; p < n; p += blockDim.x)
         if (X[p - 1] > X[p] || V[p - 1] > V[p]) { const int k = atomicAdd(&s_nf, 1); foldList[k] = p; }
     egdst_cta_sync();
     const int nf = s_nf;
-    for (int i = threadIdx.x; i < nf; i += blockDim.x) {
-        const int v = foldList[i];
-        int r = 0;
-        for (int j = 0; j < nf; j++) r += foldList[j] < v ? 1 : 0;
-        runStart[r + 1] = v;
-    }
-    if (threadIdx.x == 0) { runStart[0] = 0; runStart[nf + 1] = n; P.ptN[sd] = n; P.nfold[sd] = nf; P.active[sd] = 1; }
+    egdst_fold_runs(P, sd, nf, n);
+    if (threadIdx.x == 0) P.active[sd] = 1;
     for (int k = threadIdx.x; k < P.cx.nst * P.cx.nd; k += blockDim.x) if (k != sd) { P.active[k] = 0; P.nfold[k] = 0; P.ptN[k] = 0; }
     egdst_cta_sync();
     if (nf == 0) return;

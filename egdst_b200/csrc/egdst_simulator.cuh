@@ -110,8 +110,10 @@ struct EgdstSimArgs {
 EGDST_DEV bool egdst_sim_interval(const EgdstDev &P, int cell, int nm, bool tabok, double cash, unsigned long long l2keep, EgdstInterval &iv) {
     if (nm < 2) return false;
     if (tabok && egdst_cell_fits_tab(P, nm)) {
-        egdst_lookup_tab<true>(P, cell, egdst_cell_rows(P, cell), cash, nm, iv, l2keep);
-    } else {  // oversized cell: plain columns
+        egdst_cell_lookup<true>(P, cell, true, cash, nm, iv, l2keep);
+    } else {
+        // cells without tables: the same bracket as egdst_cell_lookup, but y = 0 (egdst_sim_weights divides here), because
+        // the record's own reciprocal costs a PB == 2 instantiation of egdst_k_simulate spill space
         const double *Mg = egdst_colM(P, cell), *Cg = egdst_colC(P, cell), *Vg = egdst_colV(P, cell);
         const int i = egdst_bracket(cash, Mg, nm, 0);
         iv.g0 = Mg[i]; iv.g1 = Mg[i + 1]; iv.c0 = Cg[i]; iv.c1 = Cg[i + 1]; iv.v0 = Vg[i]; iv.v1 = Vg[i + 1]; iv.y = 0.0;
@@ -138,11 +140,7 @@ EGDST_DEV bool egdst_sim_policy_cell(const EgdstDev &P, const egdst_ctx &cx, int
     double wl, wr;
     egdst_sim_weights(iv, pv.cash, wl, wr);
     c = iv.c1 * wl + iv.c0 * wr;
-    const int nth = P.thlen[cell];
-    const double *th = P.thTH + (size_t)cell * cx.nthrhmax, *dd = P.thD + (size_t)cell * cx.nthrhmax;
-    int ith = 0;
-    while (ith < nth && pv.cash >= th[ith]) ith++;
-    pv.id = (int)dd[ith > 0 ? ith - 1 : 0];
+    pv.id = egdst_policy_decision(pv.cash, P.thTH + (size_t)cell * cx.nthrhmax, P.thD + (size_t)cell * cx.nthrhmax, P.thlen[cell]);
     egdst_fill_decision(&cx, &pv);
     const double evf = P.evf[cell];
     if (pv.cash < M1 && evf > -EGDST_INF) vf = utility(&cx, &pv, c) + discount(&cx, &pv) * evf;
@@ -390,16 +388,8 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
                     c = iv.c1 * wl + iv.c0 * wr;
                     cur.savings = cur.cash - c;
                     const int nth = HDR ? hc->nth : P.thlen[cell];
-                    if (HDR && nth <= EGDST_SIM_TH8) {
-                        int ith = 0;
-                        while (ith < nth && cur.cash >= hc->th[ith]) ith++;
-                        cur.id = (int)hc->dd[ith > 0 ? ith - 1 : 0];
-                    } else {
-                        const double *th = P.thTH + (size_t)cell * cx.nthrhmax, *dd = P.thD + (size_t)cell * cx.nthrhmax;
-                        int ith = 0;
-                        while (ith < nth && cur.cash >= th[ith]) ith++;
-                        cur.id = (int)dd[ith > 0 ? ith - 1 : 0];
-                    }
+                    if (HDR && nth <= EGDST_SIM_TH8) cur.id = egdst_policy_decision(cur.cash, hc->th, hc->dd, nth);
+                    else cur.id = egdst_policy_decision(cur.cash, P.thTH + (size_t)cell * cx.nthrhmax, P.thD + (size_t)cell * cx.nthrhmax, nth);
                     egdst_fill_decision(&cx, &cur);
                     const double evf = HDR ? hc->evf : P.evf[cell];  // == V(row 0)
                     const double M1 = HDR ? hc->M1 : egdst_colM(P, cell)[1];

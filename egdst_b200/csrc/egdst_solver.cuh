@@ -31,20 +31,26 @@ struct EgdstNext {
     double M1, Mlast, Clast;  // M[1], M[n1], C[n1]
 };
 
-EGDST_DEV EgdstNext egdst_next_tables(const EgdstDev &P, int ivec, int it1, int ist1) {
-    int cell = egdst_cell(P, ivec, it1, ist1);
+// The tables of a cell with at least two rows after row 0, without thresholds: decision cells of the smoothing mode have
+// none (thlen and thTH are sized for the solution cells only).
+EGDST_DEV EgdstNext egdst_cell_tables(const EgdstDev &P, int cell) {
     EgdstNext t;
     t.M = egdst_colM(P, cell);
     t.C = egdst_colC(P, cell);
     t.V = egdst_colV(P, cell);
     t.n1 = P.mlen[cell] - 1;
-    t.th = P.thTH + (size_t)cell * P.cx.nthrhmax;
-    t.dd = P.thD + (size_t)cell * P.cx.nthrhmax;
-    t.nth = P.thlen[cell];
+    t.th = 0; t.dd = 0; t.nth = 0;
     t.evf = P.evf[cell];
     t.cell = cell;
     t.ivl = egdst_cell_rows(P, cell);
     t.M1 = t.M[1]; t.Mlast = t.M[t.n1]; t.Clast = t.C[t.n1];
+    return t;
+}
+EGDST_DEV EgdstNext egdst_next_tables(const EgdstDev &P, int ivec, int it1, int ist1) {
+    EgdstNext t = egdst_cell_tables(P, egdst_cell(P, ivec, it1, ist1));
+    t.th = P.thTH + (size_t)t.cell * P.cx.nthrhmax;
+    t.dd = P.thD + (size_t)t.cell * P.cx.nthrhmax;
+    t.nth = P.thlen[t.cell];
     return t;
 }
 
@@ -83,8 +89,8 @@ EGDST_DEV void egdst_fill_shocktab(const egdst_ctx *cx, const EgdstDev &P, const
 
 // One quadrature node of the expectation (egdst_solver.c:547-573), all cases: table-free cells, extrapolation on either
 // side of the grid, the credit-constrained branch of the value function, decision-dependent marginal utility, aborts.
-// Returns false when the evaluation ends at this node (acc.bad* say why).  Kept out of line: the hot loop of
-// egdst_eval_nodes handles the common case itself and must not pay this function's registers.
+// Returns false when the evaluation ends at this node (acc.bad* say why).  The hot loop of egdst_eval_nodes takes the
+// common cases through egdst_fast_lookup / egdst_fast_interp and calls this for the rest.
 EGDST_DEV bool egdst_eval_node(const egdst_ctx *cx, const EgdstDev &P, const EgdstNext &t, bool tab, const PeriodVars *curr, PeriodVars &next,
                                     int keep, int q, double pr1, EgdstAcc &acc) {
     acc.checksum += pr1;
@@ -92,12 +98,7 @@ EGDST_DEV bool egdst_eval_node(const egdst_ctx *cx, const EgdstDev &P, const Egd
     // one bracket lookup serves consumption (rows 0..n1) and value (rows 1..n1): the second bracket of the
     // reference is max(i,1) of the first (same strictly increasing grid); rows i, i+1 come as one record
     EgdstInterval iv;
-    int i;
-    if (tab) i = egdst_lookup_tab(P, t.cell, t.ivl, next.cash, t.n1 + 1, iv);
-    else {
-        i = egdst_bracket(next.cash, t.M, t.n1 + 1, 0); iv.g0 = t.M[i]; iv.g1 = t.M[i + 1]; iv.c0 = t.C[i]; iv.c1 = t.C[i + 1]; iv.v0 = t.V[i]; iv.v1 = t.V[i + 1];
-        iv.y = egdst_div_safe(iv.g1 - iv.g0) ? 1.0 / (iv.g1 - iv.g0) : 0.0;
-    }
+    const int i = egdst_cell_lookup(P, t.cell, tab, next.cash, t.n1 + 1, iv);
     // the reference's quotients are kept bit for bit (two divisions per interpolation, egdst_lib.c:175): next to its
     // instability boundary (SURVEY 0, fact 7) a plain reciprocal-multiply variant drifted 1e-2 away in C, so the
     // shared-reciprocal form below is the exactly rounded one (egdst_div_by)
@@ -120,8 +121,7 @@ EGDST_DEV bool egdst_eval_node(const egdst_ctx *cx, const EgdstDev &P, const Egd
             v1 = utility(cx, &next, next.cash - cx->a0) + discount(cx, &next) * t.evf;  // egdst_solver.c:763
         } else {
             if (i < 1) {  // value table starts at row 1 (row 0 of V is evf(a0), not a value)
-                if (tab) iv = egdst_load_interval(t.ivl + 1);
-                else { iv.g0 = t.M[1]; iv.g1 = t.M[2]; iv.v0 = t.V[1]; iv.v1 = t.V[2]; iv.y = egdst_div_safe(iv.g1 - iv.g0) ? 1.0 / (iv.g1 - iv.g0) : 0.0; }
+                iv = egdst_cell_interval(P, t.cell, tab, 1);
                 w = iv.g1 - iv.g0;
                 y = iv.y;
             }
@@ -149,17 +149,6 @@ EGDST_DEV bool egdst_eval_node(const egdst_ctx *cx, const EgdstDev &P, const Egd
 // credit-constrained branch below the first endogenous point, transformed extrapolation of the value above the grid.
 #define EGDST_SMOOTH_MAXND 8
 #if EGDST_SMOOTHING
-EGDST_DEV EgdstNext egdst_choice_tables(const EgdstDev &P, int dcell) {
-    EgdstNext t;
-    t.M = egdst_colM(P, dcell); t.C = egdst_colC(P, dcell); t.V = egdst_colV(P, dcell);
-    t.n1 = P.mlen[dcell] - 1;
-    t.th = 0; t.dd = 0; t.nth = 0;
-    t.evf = P.evf[dcell];
-    t.cell = dcell;
-    t.ivl = egdst_cell_rows(P, dcell);
-    t.M1 = t.n1 >= 1 ? t.M[1] : 0.0; t.Mlast = t.n1 >= 1 ? t.M[t.n1] : 0.0; t.Clast = t.n1 >= 1 ? t.C[t.n1] : 0.0;
-    return t;
-}
 // Out of line, with scalar arguments and the kernel-argument block read from its copy in global memory (P.self): the
 // reference-parity kernels must not pay registers, local memory or instruction-cache space for this mode (a by-reference
 // call would pin the caller's context structs to local memory).
@@ -182,17 +171,12 @@ EGDST_NOINLINE EgdstSmoothOut egdst_smooth_node(const EgdstDev *Pg, int ivec, in
         vd[d1] = -EGDST_INF; md[d1] = 0.0; vl[d1] = -EGDST_INF;
         const int dcell = egdst_dcell(P, cell1, d1);
         if (P.mlen[dcell] < 3) continue;  // decision not available in (it+1, ist1)
-        const EgdstNext t = egdst_choice_tables(P, dcell);
+        const EgdstNext t = egdst_cell_tables(P, dcell);
         vl[d1] = t.V[t.n1];
         above = above || cash > t.Mlast;
         const bool tab = egdst_cell_has_tab(P, t.cell, t.n1 + 1);
         EgdstInterval iv;
-        int i;
-        if (tab) i = egdst_lookup_tab(P, t.cell, t.ivl, cash, t.n1 + 1, iv);
-        else {
-            i = egdst_bracket(cash, t.M, t.n1 + 1, 0); iv.g0 = t.M[i]; iv.g1 = t.M[i + 1]; iv.c0 = t.C[i]; iv.c1 = t.C[i + 1]; iv.v0 = t.V[i]; iv.v1 = t.V[i + 1];
-            iv.y = egdst_div_safe(iv.g1 - iv.g0) ? 1.0 / (iv.g1 - iv.g0) : 0.0;
-        }
+        const int i = egdst_cell_lookup(P, t.cell, tab, cash, t.n1 + 1, iv);
         double w = iv.g1 - iv.g0, y = iv.y;
         double c1 = y != 0.0 ? egdst_lerp_y(cash, iv.g0, iv.g1, iv.c0, iv.c1, w, y) : egdst_lerp(cash, iv.g0, iv.g1, iv.c0, iv.c1);
         if (cash > t.Mlast) c1 = MAX(c1, t.Clast);
@@ -204,8 +188,7 @@ EGDST_NOINLINE EgdstSmoothOut egdst_smooth_node(const EgdstDev *Pg, int ivec, in
             v1 = utility(cx, &next, cash - cx->a0) + discount(cx, &next) * t.evf;
         } else {
             if (i < 1) {
-                if (tab) iv = egdst_load_interval(t.ivl + 1);
-                else { iv.g0 = t.M[1]; iv.g1 = t.M[2]; iv.v0 = t.V[1]; iv.v1 = t.V[2]; iv.y = egdst_div_safe(iv.g1 - iv.g0) ? 1.0 / (iv.g1 - iv.g0) : 0.0; }
+                iv = egdst_cell_interval(P, t.cell, tab, 1);
                 w = iv.g1 - iv.g0; y = iv.y;
             }
             v1 = egdst_linter_extrap_iv(cx, &next, cash, iv.g0, iv.g1, iv.v0, iv.v1, t.M1, t.Mlast, w, y);
@@ -214,8 +197,7 @@ EGDST_NOINLINE EgdstSmoothOut egdst_smooth_node(const EgdstDev *Pg, int ivec, in
                 // the chord it continues: the reference continues the last interval of the MERGED cell, so every decision's value
                 // is continued from that abscissa (g0m) -- the limit sigma -> 0 is then the reference's extrapolation exactly
                 EgdstInterval jv;
-                if (tab) egdst_lookup_tab(P, t.cell, t.ivl, g0m, t.n1 + 1, jv);
-                else { const int j = egdst_bracket(g0m, t.M, t.n1 + 1, 0); jv.g0 = t.M[j]; jv.g1 = t.M[j + 1]; jv.v0 = t.V[j]; jv.v1 = t.V[j + 1]; }
+                egdst_cell_lookup(P, t.cell, tab, g0m, t.n1 + 1, jv);
                 const double vg = egdst_lerp(g0m, jv.g0, jv.g1, jv.v0, jv.v1);
                 v1 = egdst_linter_extrap_iv(cx, &next, cash, g0m, t.Mlast, vg, t.V[t.n1], t.M1, t.Mlast, t.Mlast - g0m, 0.0);
             }
@@ -267,24 +249,8 @@ EGDST_NOINLINE EgdstSmoothOut egdst_smooth_node(const EgdstDev *Pg, int ivec, in
 struct EgdstFastNode { double cash, c1, v1; bool ok; };
 EGDST_DEV void egdst_fast_lookup(const EgdstDev &P, const EgdstNext &t, const EgdstCellTop &top, double cash, int &i, bool &ok) {
     if (cash > top.g1) { i = -1; ok = top.y != 0.0 && top.yt != 0.0 && cash > P.cx.a0; return; }
-    int b = egdst_lut_key(cash, P.cx.a0, P.mbits);
-    b = b < 0 ? 0 : (b > P.lutcap - 1 ? P.lutcap - 1 : b);
-    const EgdstLutEntry *lut = egdst_cell_lut(P, t.cell) + b;
-#ifdef EGDST_HOSTEMU
-    const EgdstLutEntry e = *lut;
-#else
-    EgdstLutEntry e;
-    const int4 r0 = *reinterpret_cast<const int4 *>(lut);
-    const double2 r1 = *(reinterpret_cast<const double2 *>(lut) + 1);
-    e.l = r0.x; e.cnt = r0.y; e.m0 = __hiloint2double(r0.w, r0.z); e.m1 = r1.x; e.m2 = r1.y;
-#endif
-    i = e.l - 1 + (e.m0 <= cash ? 1 : 0) + (e.m1 <= cash ? 1 : 0) + (e.m2 <= cash ? 1 : 0);
-    if (e.cnt > 3 && e.m2 <= cash) {  // crowded bucket (the grid is dense around its focal point): bisect its remaining rows
-        int l = e.l + 3, h = e.l + e.cnt;
-        while (l < h) { const int mid = (l + h) >> 1; if (t.M[mid] <= cash) l = mid + 1; else h = mid; }
-        i = l - 1;
-    }
-    ok = i >= 1 && i <= t.n1 - 1;  // rows i, i+1 exist and belong to the value grid
+    i = egdst_lut_rank(P, t.cell, t.M, cash);
+    ok = i >= 1 && i <= t.n1 - 1;  // rows i, i+1 exist and belong to the value grid (no clamp: others take the general path)
 }
 EGDST_DEV void egdst_fast_interp(const egdst_ctx *cx, const PeriodVars *next, const EgdstNext &t, const EgdstCellTop &top, int i, double cash, EgdstFastNode &f) {
     const double big = 1e290;
@@ -539,14 +505,66 @@ EGDST_DEV void egdst_seed_publish(const EgdstDev &P, int sd, double *seed, const
     P.scanC[(size_t)sd * P.chC] = EGDST_SCAN_INC | egdst_scan_pack(kept, stop);
 }
 
+// The adraw loop from savings point S.A on (egdst_solver.c:1032-1099), serial in A, parallel over nodes: the CTA
+// evaluates the point; thread 0 classifies it, replaces a point whose consumption vanished by its zero-consumption re-send
+// (egdst_resend_point), stores a point with a finite M as row `slot` of the grid (if slot < P.gcap), and goes on while
+// the point asks for a re-send.  On return S.go is 0 (done) or -1 (failed), and thread 0 holds the last point, its M,
+// evf(a0) (-inf after an abort) and the limits L of the closed-form grid after it (the first ones when L.k3 == 0).
+struct EgdstAdraw { double lastA, aM, evfa0; int stored, storedAny; };  // stored: by the last evaluation / by any
+EGDST_DEV EgdstAdraw egdst_adraw(const egdst_ctx *cx, const EgdstDev &P, int it, int ivec, int ist, int id, const PeriodVars *curr, double beta,
+                                 int slot, double baseA, double baseM, EgdstLims &L, EgdstSeedShared &S, const double *shk, const double *shp) {
+    const size_t row = (size_t)egdst_sd(P, ivec, ist, id) * P.gcap + slot;
+    EgdstAdraw r; r.lastA = cx->a0; r.aM = 0; r.evfa0 = 0.0; r.stored = 0; r.storedAny = 0;
+    while (true) {
+        egdst_block_eval(cx, P, ivec, curr, S.A, 1, S, shk, shp);
+        if (threadIdx.x == 0) {
+            r.lastA = S.A;
+            r.stored = 0;
+            int resend = 0, fatal = 0;
+            if (S.badq == EGDST_NOBAD && fabs(S.checksum - 1) > cx->tolerance) {
+                egdst_fail(P, ivec, EGDST_ERR_CHECKSUM, it, ist, id); fatal = 1;
+            } else if (S.badq != EGDST_NOBAD) {
+                r.evfa0 = -EGDST_INF;
+                r.aM = S.badcash;
+                if (S.badtype == EGDST_PT_C1NEG) {
+                    r.aM = cx->a0 - 1;
+                    int fail = 0;
+                    r.lastA = egdst_resend_point(cx, P, ivec, curr, it, r.lastA, S.badq, S.badshock, S.badcash, &fail);
+                    if (fail) { egdst_fail(P, ivec, EGDST_ERR_CASHINVERSE, it, ist, id); fatal = 1; }
+                }
+            } else {
+                r.aM = r.lastA + utility_marginal_inverse(cx, curr, beta * S.rhs);
+                if (isfinite(r.aM)) {
+                    if (fabs(r.lastA - cx->a0) < cx->tolerance && r.evfa0 > -EGDST_INF) r.evfa0 = S.evf;
+                    if (slot < P.gcap) {
+                        P.ptX[row] = r.aM; P.ptC[row] = r.aM - r.lastA; P.ptV[row] = utility(cx, curr, r.aM - r.lastA) + beta * S.evf;
+                        r.stored = 1; r.storedAny = 1;
+                    }
+                }
+            }
+            if (!fatal) {
+                // adraw, ngenerated==1 branch (egdst_solver.c:1032-1099)
+                if (L.k3 == 0) egdst_lims_first(cx, curr, r.aM, r.lastA, baseA, baseM, P.N, L);
+                if (r.aM <= cx->a0 - 1 + cx->tolerance) {
+                    egdst_lims_resend(cx, curr, r.lastA, baseA, baseM, L);
+                    resend = 1;
+                    if (++S.calls >= cx->ngridmax) { egdst_fail(P, ivec, EGDST_ERR_ADRAW_LOOP, it, ist, id); resend = 0; fatal = 1; }
+                }
+            }
+            S.A = r.lastA;
+            S.go = fatal ? -1 : resend;
+        }
+        egdst_cta_sync();
+        if (S.go != 1) return r;
+    }
+}
+
 EGDST_DEV void egdst_seed_job(const EgdstDev &P, int it, int ivec, int ist, int id, EgdstSeedShared &S, double *shsm, int useTab) {
     egdst_ctx cx; egdst_load_ctx(P, ivec, cx);
     const int sd = egdst_sd(P, ivec, ist, id);
     PeriodVars curr; curr.it = it; curr.ist = ist; curr.id = id; curr.cash = 0; curr.savings = 0; curr.shock = 0;
     const int act = (feasible(&cx, &curr) == 1) && (inchoiceset(&cx, &curr) == 1);
-    const int N = P.N;
     double *seed = P.seed + (size_t)sd * EGDST_SEEDW;
-    double *X = P.ptX + (size_t)sd * P.gcap, *Cc = P.ptC + (size_t)sd * P.gcap, *V = P.ptV + (size_t)sd * P.gcap;
     egdst_cta_sync();  // S and the shock table of the previous job are free
     if (threadIdx.x == 0) {
         P.active[sd] = act;
@@ -606,54 +624,14 @@ EGDST_DEV void egdst_seed_job(const EgdstDev &P, int it, int ivec, int ist, int 
         if (S.go != 0) break;
     }
     if (S.go != 1) return;
-    // stage 1 (+ re-sends): serial in A, parallel over nodes
+    // stage 1 (+ re-sends): the point a0 becomes row 0 of the grid
     EgdstLims L; L.lim1 = 0; L.lim2 = 0; L.lim3 = 0; L.lim2p = 0; L.lim3p = 0; L.k3 = 0;
-    double lastA = cx.a0, aM = 0, evfa0 = 0.0;
-    int stored = 0;
-    while (true) {
-        egdst_block_eval(&cx, P, ivec, &curr, S.A, 1, S, shk, shp);
-        if (threadIdx.x == 0) {
-            lastA = S.A;
-            int resend = 0, fatal = 0;
-            if (S.badq == EGDST_NOBAD && fabs(S.checksum - 1) > cx.tolerance) {
-                egdst_fail(P, ivec, EGDST_ERR_CHECKSUM, it, ist, id); fatal = 1;
-            } else if (S.badq != EGDST_NOBAD) {
-                evfa0 = -EGDST_INF;
-                aM = S.badcash;
-                if (S.badtype == EGDST_PT_C1NEG) {
-                    aM = cx.a0 - 1;
-                    int fail = 0;
-                    lastA = egdst_resend_point(&cx, P, ivec, &curr, it, lastA, S.badq, S.badshock, S.badcash, &fail);
-                    if (fail) { egdst_fail(P, ivec, EGDST_ERR_CASHINVERSE, it, ist, id); fatal = 1; }
-                }
-            } else {
-                aM = lastA + utility_marginal_inverse(&cx, &curr, beta * S.rhs);
-                if (isfinite(aM)) {
-                    if (fabs(lastA - cx.a0) < cx.tolerance && evfa0 > -EGDST_INF) evfa0 = S.evf;
-                    X[0] = aM; Cc[0] = aM - lastA; V[0] = utility(&cx, &curr, aM - lastA) + beta * S.evf;
-                    stored = 1;
-                }
-            }
-            if (!fatal) {
-                // adraw, ngenerated==1 branch (egdst_solver.c:1032-1099)
-                if (L.k3 == 0) egdst_lims_first(&cx, &curr, aM, lastA, baseA, baseM, N, L);
-                if (aM <= cx.a0 - 1 + cx.tolerance) {
-                    egdst_lims_resend(&cx, &curr, lastA, baseA, baseM, L);
-                    resend = 1;
-                    if (++S.calls >= cx.ngridmax) { egdst_fail(P, ivec, EGDST_ERR_ADRAW_LOOP, it, ist, id); resend = 0; fatal = 1; }
-                }
-            }
-            S.A = lastA;
-            S.go = fatal ? -1 : resend;
-        }
-        egdst_cta_sync();
-        if (S.go != 1) break;
-    }
+    const EgdstAdraw r = egdst_adraw(&cx, P, it, ivec, ist, id, &curr, beta, 0, baseA, baseM, L, S, shk, shp);
     if (threadIdx.x == 0) {
-        P.evfa0[sd] = evfa0;
+        P.evfa0[sd] = r.evfa0;
         if (S.go == 0) {
-            egdst_seed_publish(P, sd, seed, L, lastA, 1, S.calls, baseA, baseM, stored, (aM < cx.mmax) ? 0 : 1, 0);
-            if (stored) atomicAdd(P.units + ivec, 1ULL);
+            egdst_seed_publish(P, sd, seed, L, r.lastA, 1, S.calls, baseA, baseM, r.storedAny, (r.aM < cx.mmax) ? 0 : 1, 0);
+            if (r.storedAny) atomicAdd(P.units + ivec, 1ULL);
         }
     }
 }
@@ -712,11 +690,30 @@ struct EgdstEgmShared {
     unsigned long long excl;
 };
 
+// The runs of the point list of sd (n points, nf folds at the positions in its fold list, unordered): runStart = 0, the
+// fold positions in ascending order, n; and the counts.  All threads of the CTA; the list may have been written by other
+// CTAs, so it is read past L1.
+EGDST_DEV void egdst_fold_runs(const EgdstDev &P, int sd, int nf, int n) {
+    const int *foldList = P.foldList + (size_t)sd * (P.gcap + 1);
+    int *runStart = P.runStart + (size_t)sd * (P.gcap + 1);
+    for (int i = threadIdx.x; i < nf; i += blockDim.x) {  // rank sort (folds are rare)
+        const int v = EGDST_LDCG(foldList + i);
+        int r = 0;
+        for (int j = 0; j < nf; j++) r += EGDST_LDCG(foldList + j) < v ? 1 : 0;
+        runStart[r + 1] = v;
+    }
+    if (threadIdx.x == 0) {
+        runStart[0] = 0;
+        runStart[nf + 1] = n;
+        P.ptN[sd] = n;
+        P.nfold[sd] = nf;
+    }
+}
+
 EGDST_DEV void egdst_egm_epilogue(const EgdstDev &P, int it, int ivec, int ist, int id, int sd, int nitems, int slot) {
     // last item of this (ist,id): folds on item boundaries, ordering of the fold list, counts
     const volatile unsigned long long *st = P.scanC + (size_t)sd * P.chC;
     const double *X = P.ptX + (size_t)sd * P.gcap, *V = P.ptV + (size_t)sd * P.gcap;
-    int *runStart = P.runStart + (size_t)sd * (P.gcap + 1);
     int *foldList = P.foldList + (size_t)sd * (P.gcap + 1);
     const unsigned long long tot = egdst_scan_inclusive(st, nitems);
     const int kept = egdst_scan_lo(tot);
@@ -732,36 +729,16 @@ EGDST_DEV void egdst_egm_epilogue(const EgdstDev &P, int it, int ivec, int ist, 
     egdst_cta_sync();
     int nf = *((volatile int *)(P.foldCnt + sd));
     if (nf > P.gcap - 1) nf = P.gcap - 1;
-    for (int i = threadIdx.x; i < nf; i += blockDim.x) {  // rank sort (folds are rare)
-        const int v = EGDST_LDCG(foldList + i);
-        int r = 0;
-        for (int j = 0; j < nf; j++) r += EGDST_LDCG(foldList + j) < v ? 1 : 0;
-        runStart[r + 1] = v;
-    }
+    egdst_fold_runs(P, sd, nf, nvd);
     if (threadIdx.x == 0) {
         if (kept >= P.cx.ngridmax) egdst_fail(P, ivec, EGDST_ERR_GRIDSPACE, it, ist, id);
-        runStart[0] = 0;
-        runStart[nf + 1] = nvd;
-        P.ptN[sd] = nvd;
-        P.nfold[sd] = nf;
         if (nf > 0) atomicAdd(P.flags + 8 * slot + 3, 1);  // the period needs the secondary envelope
     }
 }
 
-#ifndef EGDST_HOSTEMU
-#define EGDST_EGM_TIC(k) do { if (tic && threadIdx.x == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_)); P.phase_ns[8 + (k)] += t_ - tprev; tprev = t_; } } while (0)
-#else
-#define EGDST_EGM_TIC(k)
-#endif
 template <int BS>
 EGDST_DEV void egdst_ph_egm(const EgdstDev &P, int it, const EgdstTeam &T, int pass, void *scratch, double *shsm) {
     EgdstEgmShared<BS> &E = *reinterpret_cast<EgdstEgmShared<BS> *>(scratch);
-    // measurement aid: the steps of the team's last work item (the longest look-back), from the start of the phase
-    unsigned long long tprev = 0ULL;
-    bool tic = false;
-#ifndef EGDST_HOSTEMU
-    if (P.phase_ns && threadIdx.x == 0) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(tprev));
-#endif
     const int N = P.N, B = blockDim.x, Pp = P.egmP, nsl = B / Pp;
     const int jpv = P.cx.nst * P.cx.nd;
     const int nitems = (N - 1 + Pp - 1) / Pp;  // items per (ist,id): the grid points 1..N-1 (a re-seeded pass covers fewer)
@@ -776,7 +753,6 @@ EGDST_DEV void egdst_ph_egm(const EgdstDev &P, int it, const EgdstTeam &T, int p
         egdst_item(T, w, jpv, ivec, jy, item);
         const int ist = jy / P.cx.nd, id = jy % P.cx.nd;
         const int sd = egdst_sd(P, ivec, ist, id);
-        tic = P.phase_ns != 0 && w == nwork - 1;
         if (!P.active[sd]) continue;  // uniform per CTA
         const double *seed = P.seed + (size_t)sd * EGDST_SEEDW;
         volatile unsigned long long *st = P.scanC + (size_t)sd * P.chC;
@@ -809,11 +785,6 @@ EGDST_DEV void egdst_ph_egm(const EgdstDev &P, int it, const EgdstTeam &T, int p
         }
         if (threadIdx.x == 0) { E.evmin[0] = 0x7fffffff; E.evmin[1] = 0x7fffffff; }
         egdst_cta_sync();
-        EGDST_EGM_TIC(0);  // set-up: context, shock table
-#ifndef EGDST_HOSTEMU
-        unsigned long long tstart = 0ULL;
-        if (P.phase_ns && threadIdx.x == 0) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(tstart));
-#endif
         // the loop guard of adraw (egdst_solver.c:963-978): the call that would return point n is call seed[7]+n
         const bool valid = s < nsl && n < N && (int)seed[7] + n < cx.ngridmax;
         double A = 0.0;
@@ -825,13 +796,6 @@ EGDST_DEV void egdst_ph_egm(const EgdstDev &P, int it, const EgdstTeam &T, int p
         E.rhs[threadIdx.x] = a.rhs; E.evf[threadIdx.x] = a.evf; E.chk[threadIdx.x] = a.checksum;
         E.q[threadIdx.x] = a.badq; E.t[threadIdx.x] = a.badtype; E.cash[threadIdx.x] = a.badcash;
         egdst_cta_sync();
-        EGDST_EGM_TIC(1);  // node loop
-#ifndef EGDST_HOSTEMU
-        if (P.phase_ns && threadIdx.x == 0 && it == P.NT / 2) {  // measurement aid: the slowest node loop of the middle period and its item
-            unsigned long long t_; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t_));
-            atomicMax(P.phase_ns + 14, ((t_ - tstart) << 20) | (unsigned long long)w);
-        }
-#endif
         // threads 0..Pp-1 own the points of the item, in order
         int flag = EGDST_PT_NONE;
         double M = 0, c = 0, v = 0;
@@ -875,13 +839,11 @@ EGDST_DEV void egdst_ph_egm(const EgdstDev &P, int it, const EgdstTeam &T, int p
         int woff = egdst_block_excl_scan(lane == 0 ? __popc(bal) : 0, E.sh, &total);
         woff = __shfl_sync(EGDST_FULL, woff, 0);
         int err = 0;
-        EGDST_EGM_TIC(2);  // combine, Euler inversion, stop rule, block scan
         if (warp == 0) {
             const unsigned long long e = egdst_lookback<1>(st, item + 1, egdst_scan_pack(total, lim != 0x7fffffff ? 1 : 0), &err);
             if (lane == 0) E.excl = e;
         }
         egdst_cta_sync();
-        EGDST_EGM_TIC(3);  // look-back
         const unsigned long long excl = E.excl;
         if (!egdst_scan_hi(excl)) {  // the grid did not end in an earlier item: this item's points count
             if (in && flag == EGDST_PT_CHECKSUM) egdst_fail(P, ivec, EGDST_ERR_CHECKSUM, it, ist, id);
@@ -911,9 +873,7 @@ EGDST_DEV void egdst_ph_egm(const EgdstDev &P, int it, const EgdstTeam &T, int p
         egdst_cta_sync();
         if (threadIdx.x == 0) E.last = (atomicAdd(P.tickC + 2 * sd + 1, 1) == nitems - 1);
         egdst_cta_sync();
-        EGDST_EGM_TIC(4);  // writes, folds, completion count
         if (E.last) { __threadfence(); egdst_egm_epilogue(P, it, ivec, ist, id, sd, nitems, T.slot); }
-        EGDST_EGM_TIC(5);  // epilogue (if this item finished last)
     }
 }
 
@@ -940,7 +900,7 @@ EGDST_DEV void egdst_ph_resend(const EgdstDev &P, int it, const EgdstTeam &T, in
         egdst_ctx cx; egdst_load_ctx(P, ivec, cx);
         PeriodVars curr; curr.it = it; curr.ist = ist; curr.id = id; curr.cash = 0; curr.savings = 0; curr.shock = 0;
         double *seed = P.seed + (size_t)sd * EGDST_SEEDW;
-        double *X = P.ptX + (size_t)sd * P.gcap, *Cc = P.ptC + (size_t)sd * P.gcap, *V = P.ptV + (size_t)sd * P.gcap;
+        const double *X = P.ptX + (size_t)sd * P.gcap, *V = P.ptV + (size_t)sd * P.gcap;
         const int nitems = (N - 1 + P.egmP - 1) / P.egmP;
         const double beta = discount(&cx, &curr);
         const double *shk = 0, *shp = 0;
@@ -953,47 +913,13 @@ EGDST_DEV void egdst_ph_resend(const EgdstDev &P, int it, const EgdstTeam &T, in
         const double baseA = seed[8], baseM = seed[9];
         if (threadIdx.x == 0) { S.A = egdst_agrid(&cx, &curr, seed, nl, N); S.calls = (int)seed[7]; S.go = 1; }
         egdst_cta_sync();
+        // the limits of the published seed (k3 >= 1: egdst_adraw does not take the first ones again)
         EgdstLims L; L.lim1 = seed[0]; L.lim2 = seed[1]; L.lim3 = seed[2]; L.lim3p = seed[3]; L.k3 = seed[4]; L.lim2p = 0;
-        double lastA = 0, aM = 0;
-        int stored = 0;
-        while (true) {
-            egdst_block_eval(&cx, P, ivec, &curr, S.A, 1, S, shk, shp);
-            if (threadIdx.x == 0) {
-                lastA = S.A;
-                int resend = 0, fatal = 0;
-                stored = 0;
-                if (S.badq == EGDST_NOBAD && fabs(S.checksum - 1) > cx.tolerance) {
-                    egdst_fail(P, ivec, EGDST_ERR_CHECKSUM, it, ist, id); fatal = 1;
-                } else if (S.badq != EGDST_NOBAD) {
-                    aM = S.badcash;
-                    if (S.badtype == EGDST_PT_C1NEG) {
-                        aM = cx.a0 - 1;
-                        int fail = 0;
-                        lastA = egdst_resend_point(&cx, P, ivec, &curr, it, lastA, S.badq, S.badshock, S.badcash, &fail);
-                        if (fail) { egdst_fail(P, ivec, EGDST_ERR_CASHINVERSE, it, ist, id); fatal = 1; }
-                    }
-                } else {
-                    aM = lastA + utility_marginal_inverse(&cx, &curr, beta * S.rhs);
-                    if (isfinite(aM) && kept < P.gcap) {
-                        X[kept] = aM; Cc[kept] = aM - lastA; V[kept] = utility(&cx, &curr, aM - lastA) + beta * S.evf;
-                        stored = 1;
-                    }
-                }
-                if (!fatal && aM <= cx.a0 - 1 + cx.tolerance) {
-                    egdst_lims_resend(&cx, &curr, lastA, baseA, baseM, L);
-                    resend = 1;
-                    if (++S.calls >= cx.ngridmax) { egdst_fail(P, ivec, EGDST_ERR_ADRAW_LOOP, it, ist, id); resend = 0; fatal = 1; }
-                }
-                S.A = lastA;
-                S.go = fatal ? -1 : resend;
-            }
-            egdst_cta_sync();
-            if (S.go != 1) break;
-        }
+        const EgdstAdraw r = egdst_adraw(&cx, P, it, ivec, ist, id, &curr, beta, kept, baseA, baseM, L, S, shk, shp);
         if (threadIdx.x == 0) {
             P.evfa0[sd] = -EGDST_INF;  // egdst_solver.c:596
             atomicAdd(P.units + P.nvec + ivec, 1ULL);  // diagnostic: re-sends after the seed stage handled in this solve
-            if (stored) {
+            if (r.stored) {
                 if (kept > 0 && (X[kept - 1] > X[kept] || V[kept - 1] > V[kept])) {
                     const int k = atomicAdd(P.foldCnt + sd, 1); if (k <= P.gcap) P.foldList[(size_t)sd * (P.gcap + 1) + k] = kept;
                 }
@@ -1001,8 +927,8 @@ EGDST_DEV void egdst_ph_resend(const EgdstDev &P, int it, const EgdstTeam &T, in
                 atomicAdd(P.units + ivec, 1ULL);
             }
             // the grid goes on after the re-sent point (which took the place of point nl) unless it ended there
-            const int stop = (S.go == -1 || !(aM < cx.mmax)) ? 1 : 0;
-            egdst_seed_publish(P, sd, seed, L, lastA, nl + 1, S.calls, baseA, baseM, kept, stop, pass + 1);
+            const int stop = (S.go == -1 || !(r.aM < cx.mmax)) ? 1 : 0;
+            egdst_seed_publish(P, sd, seed, L, r.lastA, nl + 1, S.calls, baseA, baseM, kept, stop, pass + 1);
             for (int c = 1; c < P.chC; c++) P.scanC[(size_t)sd * P.chC + c] = 0ULL;
             P.tickC[2 * sd + 1] = 0;
             P.lateN[sd] = 0x7fffffff;

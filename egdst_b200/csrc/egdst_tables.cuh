@@ -250,12 +250,11 @@ EGDST_DEV EgdstInterval egdst_load_interval_keep(const EgdstRow *p, unsigned lon
 #endif
 }
 
-// Bracket AND interval record of x in a cell that has tables (egdst_cell_has_tab).  Same bracket as
-// egdst_bracket(x, M, n, 0) on a strictly increasing grid: (#rows <= x) - 1 clamped to [0, n-2].  KEEP: load with the
-// evict_last hint `pol`.  Two dependent gathers: the 32-byte index entry, then rows i and i+1 (64 contiguous bytes).
+// Index entry of x's bucket and the rank it gives: (#rows <= x) - 1, where crowded buckets (more than three rows: the
+// grid is dense around a focal point or holds double points) bisect their remaining rows of M.  Not clamped.  KEEP:
+// load with the evict_last hint `pol`.
 template <bool KEEP = false>
-EGDST_DEV int egdst_lookup_tab(const EgdstDev &P, int cell, const EgdstRow *ivl, double x, int n, EgdstInterval &iv,
-                               unsigned long long pol = 0ULL) {
+EGDST_DEV int egdst_lut_rank(const EgdstDev &P, int cell, const double *M, double x, unsigned long long pol = 0ULL) {
     int b = egdst_lut_key(x, P.cx.a0, P.mbits);
     b = b < 0 ? 0 : (b > P.lutcap - 1 ? P.lutcap - 1 : b);
     const EgdstLutEntry *lut = egdst_cell_lut(P, cell);
@@ -274,14 +273,45 @@ EGDST_DEV int egdst_lookup_tab(const EgdstDev &P, int cell, const EgdstRow *ivl,
     }
 #endif
     int i = e.l - 1 + (e.m0 <= x ? 1 : 0) + (e.m1 <= x ? 1 : 0) + (e.m2 <= x ? 1 : 0);
-    if (e.cnt > 3 && e.m2 <= x) {  // crowded bucket (double points next to a dense stretch): bisect its remaining rows
-        const double *M = egdst_colM(P, cell);
+    if (e.cnt > 3 && e.m2 <= x) {
         int l = e.l + 3, h = e.l + e.cnt;
         while (l < h) { const int mid = (l + h) >> 1; if (M[mid] <= x) l = mid + 1; else h = mid; }
         i = l - 1;
     }
-    i = i > n - 2 ? n - 2 : i;
-    i = i < 0 ? 0 : i;
-    iv = KEEP ? egdst_load_interval_keep(ivl + i, pol) : egdst_load_interval(ivl + i);
+    return i;
+}
+
+// The record of rows i and i+1 of a cell: from the row table when the cell's tables may be used (tab,
+// egdst_cell_has_tab), otherwise from the columns, with y filled as the table rows fill it (RN(1/w), 0 where the width
+// is degenerate: plain divisions).  KEEP: load with the evict_last hint `pol`.
+template <bool KEEP = false>
+EGDST_DEV EgdstInterval egdst_cell_interval(const EgdstDev &P, int cell, bool tab, int i, unsigned long long pol = 0ULL) {
+    if (tab) {
+        const EgdstRow *r = egdst_cell_rows(P, cell) + i;
+        return KEEP ? egdst_load_interval_keep(r, pol) : egdst_load_interval(r);
+    }
+    const double *M = egdst_colM(P, cell), *C = egdst_colC(P, cell), *V = egdst_colV(P, cell);
+    EgdstInterval iv;
+    iv.g0 = M[i]; iv.g1 = M[i + 1]; iv.c0 = C[i]; iv.c1 = C[i + 1]; iv.v0 = V[i]; iv.v1 = V[i + 1];
+    iv.y = egdst_div_safe(iv.g1 - iv.g0) ? 1.0 / (iv.g1 - iv.g0) : 0.0;
+    iv.pad = 0.0;
+    return iv;
+}
+
+// Bracket i of x in a cell of n rows and the record of rows i and i+1.  With tables, two dependent gathers (the index
+// entry, then 64 contiguous bytes of rows); without, the reference's bisection (egdst_bracket).  On a strictly
+// increasing grid both give (#rows <= x) - 1 clamped to [0, n-2].
+template <bool KEEP = false>
+EGDST_DEV int egdst_cell_lookup(const EgdstDev &P, int cell, bool tab, double x, int n, EgdstInterval &iv, unsigned long long pol = 0ULL) {
+    const double *M = egdst_colM(P, cell);
+    int i;
+    if (tab) {
+        i = egdst_lut_rank<KEEP>(P, cell, M, x, pol);
+        i = i > n - 2 ? n - 2 : i;
+        i = i < 0 ? 0 : i;
+    } else {
+        i = egdst_bracket(x, M, n, 0);
+    }
+    iv = egdst_cell_interval<KEEP>(P, cell, tab, i, pol);
     return i;
 }

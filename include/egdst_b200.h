@@ -95,7 +95,7 @@ long long egdst_solution_units(egdst_solution *s);
  * (egdst_solver.c:1080-1099) the last solve went through */
 long long egdst_solution_resends(egdst_solution *s);
 /* measurement aid: device time in ms per phase of the solve kernel -- terminal, seed, egm, resend, envelope2, rank,
- * merge, tables, then six steps of the last work item of the EGM phase (16 entries) -- accumulated over this object's solves while egdst_profile_enable(1) was in effect;
+ * merge, tables (8 entries) -- accumulated over this object's solves while egdst_profile_enable(1) was in effect;
  * reading resets the counters.  Returns the number of entries. */
 int egdst_solution_phase_ms(egdst_solution *s, double *ms);
 /* diagnostic: the secondary upper envelope (envelope2, egdst_solver.c:776-913) of n EGM points (M, C, V_d) of decision

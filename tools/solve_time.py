@@ -33,8 +33,3 @@ ph = sol.phase_ms()
 for k, v in ph.items():
     print("  phase %-10s %8.3f ms/solve  %6.1f us/period" % (k, v / 3, v / 3 / max(m.nt - 1, 1) * 1e3))
 print("  resends handled:", sol.resends())
-import ctypes as C
-raw = (C.c_double * 16)()
-lib.profile_enable(True); lib.resolve(sol, m); torch.cuda.synchronize(); lib.L.egdst_solution_phase_ms(sol.handle, raw); lib.profile_enable(False)
-packed = int(round(raw[14] * 1e6))
-print("  slowest EGM node loop in the middle period: %.1f us at work item %d (of %d x %d)" % ((packed >> 20) / 1e3, packed & 0xFFFFF, m.nd, -1))
