@@ -163,10 +163,9 @@ struct egdst_solution {
     unsigned char *tab_base = 0;      // lookup tables (one allocation)
     // grow-only buffers (grow)
     double *d_pack = 0; size_t pack_cap = 0;                // export / import staging
-    double *d_momscratch = 0; size_t momscratch_cap = 0;    // per-CTA moment slices of the wide simulator variant
     EgdstCellHdr *d_hdr = 0; size_t hdr_cap = 0;            // simulator cell headers
     // every device allocation, by the field that holds it
-    std::vector<void **> owned{(void **)&d_pack, (void **)&d_momscratch, (void **)&d_hdr};
+    std::vector<void **> owned{(void **)&d_pack, (void **)&d_hdr};
     // state of the current owner (adopt)
     std::vector<int> h_mlen, h_thlen, h_status;
     bool sizes_valid = false;

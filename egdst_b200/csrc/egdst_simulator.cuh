@@ -29,11 +29,12 @@
 #ifndef EGDST_SIM_MINBLOCKS
 #define EGDST_SIM_MINBLOCKS 4
 #endif
-// CTA width of the two-periods-per-write variant: the unpadded 2*NSO-double rows of 16 warps fill two CTAs per SM
+// CTA width of the two-periods-per-write variant: two CTAs of 12 warps per SM leave each thread 80 registers, which the
+// pipelined period loop needs, and room for the per-CTA moment accumulators next to the staged rows
 #ifdef EGDST_HOSTEMU
 #define EGDST_SIM_WIDE 128
 #else
-#define EGDST_SIM_WIDE 512
+#define EGDST_SIM_WIDE 384
 #endif
 
 // the sims array is written once and never re-read by the kernel: evict-first (st.global.cs) keeps the policy
@@ -102,7 +103,6 @@ struct EgdstSimArgs {
     double *moments;           // [3, nsimout, nt]      (template OUT & 2)
     int nsimout;
     int mom_smem;              // 1: per-CTA moment accumulators for all periods live in shared memory (flushed at the end)
-    double *momscratch;        // or: per-CTA slices [nt*nsimout*3 doubles + nt ints] of a zeroed global scratch (egdst_k_momreduce)
     double param[EGDST_NPARAM_];  // parameter values of the vector (template HDR: single-vector launches)
 };
 
@@ -120,6 +120,9 @@ EGDST_DEV bool egdst_sim_interval(const EgdstDev &P, int cell, int nm, bool tabo
     }
     return true;
 }
+// Whether the policy lookup of a cell of nm rows goes through its tables (tabok: egdst_cell_has_tab's flag), as in
+// egdst_sim_interval; the pipelined period order then gathers the index entry of cash (egdst_lut_entry) a period ahead.
+EGDST_DEV bool egdst_sim_tab(const EgdstDev &P, int nm, bool tabok) { return nm >= 2 && tabok && egdst_cell_fits_tab(P, nm); }
 // One division for the weights of both interpolations (the reference divides four times, egdst_lib.c:175): the
 // reciprocal comes with the record.  The exactly rounded quotients of the solver (egdst_div_by) are not needed here:
 // the difference is in the last bit and no discrete branch of the simulator depends on it.
@@ -149,6 +152,63 @@ EGDST_DEV bool egdst_sim_policy_cell(const EgdstDev &P, const egdst_ctx &cx, int
 }
 #endif
 
+// One step of an agent's path from period cur.it into period `it` (egdst_simulator.c:259-309): survival, the next
+// discrete state by inverse-CDF sampling over trpr, shock, cash in hand and the equations of the new period, from the
+// uniforms (rrr, rrr1, rrr2) of period `it`.  False: the agent dies (the rest of its record stays NaN).
+EGDST_DEV bool egdst_sim_transition(const egdst_ctx &cx, const PeriodVars &cur, PeriodVars &nx, int it, double rrr, double rrr1, double rrr2,
+                                    double &mu, double &sigma, double *eqs) {
+    if (rrr2 > survival(&cx, &cur)) return false;
+    nx = cur;
+    nx.it = it;
+    nx.savings = cur.savings;
+    int chosen = -1, lastfeas = -1;
+    for (int ist1 = 0; ist1 < cx.nst; ist1++) {
+#if EGDST_NCONT > 0
+        {   // continuous states are carried by value: only the cells at their first grid point stand
+            // for the discrete part of the state (egdst_simulator.c:268-271)
+            bool first = true;
+#pragma unroll
+            for (int k = 0; k < EGDST_NCONT; k++) {
+                const int j0 = egdst_contvar[k];
+                if ((ist1 / (int)cx.stm[cx.nnst + j0]) % (int)cx.stm[j0] != 0) first = false;
+            }
+            if (!first) continue;
+        }
+#endif
+        nx.ist = ist1;
+        egdst_fill_state(&cx, &nx);
+#if EGDST_NCONT > 0
+        trpr_cont(&cx, &cur, &nx);  // exact next-period values of the continuous states
+#endif
+        if (!feasible(&cx, &nx)) continue;
+        lastfeas = ist1;
+        double pr;
+#if EGDST_OPT_TRPRNOSH
+        pr = trpr(&cx, &cur, &nx, 0);
+#else
+        mu = mu_param(&cx, &cur, &nx); sigma = sigma_param(&cx, &cur, &nx);
+        nx.shock = (sigma <= 0) ? egdst_expectation(&cx, &cur, &nx) : egdst_cdfinv(rrr1, mu, sigma);
+        pr = trpr(&cx, &cur, &nx, 0);
+#endif
+        rrr -= pr;
+        if (rrr <= 0) { chosen = ist1; break; }
+    }
+    if (chosen < 0) chosen = lastfeas < 0 ? 0 : lastfeas;  // the reference runs off the end here
+    nx.ist = chosen;
+    egdst_fill_state(&cx, &nx);
+#if EGDST_NCONT > 0
+    trpr_cont(&cx, &cur, &nx);
+#endif
+#if EGDST_OPT_TRPRNOSH
+    // shocks for the shock-independent case (egdst_simulator.c:292-298)
+    mu = mu_param(&cx, &cur, &nx); sigma = sigma_param(&cx, &cur, &nx);
+    nx.shock = (sigma <= 0) ? egdst_expectation(&cx, &cur, &nx) : egdst_cdfinv(rrr1, mu, sigma);
+#endif
+    nx.cash = cashinhand(&cx, &cur, &nx);
+    eqs_sim(&cx, &cur, &nx, eqs);
+    return true;
+}
+
 // Dynamic shared memory layout of egdst_k_simulate:
 //   tile[warps][32*TS]                PB staged records per agent of the warp's tile
 //   mom[nt][nso][3] + clean[nt]       (mom_smem) per-CTA moment accumulators, flushed once at the end
@@ -158,12 +218,16 @@ EGDST_DEV bool egdst_sim_policy_cell(const EgdstDev &P, const egdst_ctx &cx, int
 //   HDR     single-vector launch whose per-cell headers and parameter values travel in the kernel arguments
 //   PB      periods per write of the sims array:
 //     1  one record (8*nso bytes) per agent and store pass; rows padded to an odd stride (conflict-free staging and
-//        column walks), 8 warps per CTA, 4 CTAs/SM, moments in shared memory
+//        column walks), 8 warps per CTA, 4 CTAs/SM at 64 registers, the plain period order (below)
 //     2  two consecutive periods of an agent are staged side by side and written together (nt even): the output
 //        stream is 1.5e5 concurrent per-agent runs, and DRAM takes runs of 16*nso bytes much better than runs of 8*nso
-//        (tools/micro/wpat.cu).  The unpadded 2*nso-double rows of 16 warps fill two CTAs per SM exactly, so rows are
-//        column-rotated by (lane/4)%4 instead of padded, and moments accumulate in a per-CTA slice of a global scratch
-//        with fire-and-forget reductions (summed by egdst_k_momreduce)
+//        (tools/micro/wpat.cu).  Rows are unpadded and column-rotated by (lane/4)%4 instead; 12 warps per CTA, 2
+//        CTAs/SM at 80 registers, the software-pipelined period order, moments always in shared memory
+// Period order: PB == 2 (NCONT == 0) runs the transition into period it+1 and the index-entry gather of its cell
+// during period it, before the value, utility, moments and store pass of period it, so that the gather's latency
+// overlaps that work.  PB == 1 and the continuous-state branch keep the plain order (transition into period it, then
+// its policy): pipelined, PB == 1 spills at 64 registers, and at 80 registers the occupancy lost costs more than the
+// overlap gains.
 template <bool PHILOX, int OUT, bool HDR, int PB>
 __global__ void __launch_bounds__(PB == 2 ? EGDST_SIM_WIDE : EGDST_SIM_BLOCK, PB == 2 ? 2 : EGDST_SIM_MINBLOCKS)
 egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimHdrs H) {
@@ -174,6 +238,7 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
     constexpr int TS = SWZ ? W : (W | 1);
     constexpr int WPB = (PB == 2 ? EGDST_SIM_WIDE : EGDST_SIM_BLOCK) / 32;
     constexpr bool SIMS = (OUT & 1) != 0, MOM = (OUT & 2) != 0;
+    constexpr bool PIPE = PB == 2 && EGDST_NCONT == 0;  // pipelined period order
     // position of column j in the row of the agent staged by lane l: rotated rows spread a column over the banks
 #define EGDST_TILE_POS(l, j) ((l) * TS + (SWZ ? (((j) + (((l) >> 2) & 3) >= W) ? (j) + (((l) >> 2) & 3) - W : (j) + (((l) >> 2) & 3)) : (j)))
     // blockIdx.y walks the parameter vectors of a batched sweep: same agents and shocks under every vector,
@@ -195,10 +260,7 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
     double *tile = egdst_sim_smem + (size_t)w * 32 * TS;
     double *smom = egdst_sim_smem + (size_t)WPB * 32 * TS;                    // [nt][NSO][3] when mom_smem
     int *clean_s = reinterpret_cast<int *>(smom + (size_t)nt * NSO * 3);      // [nt] clean tiles per period
-    const bool momsm = MOM && PB == 1 && S.mom_smem;
-    // PB == 2: this CTA's slice of the global scratch
-    double *gslice = (MOM && PB == 2) ? S.momscratch + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * ((size_t)nt * NSO * 3 + nt) : (double *)0;
-    int *clean_g = reinterpret_cast<int *>(gslice + (size_t)nt * NSO * 3);
+    const bool momsm = MOM && S.mom_smem;
     const double NaN = EGDST_NAN;
     const int ntiles = (S.nsim + 31) / 32;
 #ifndef EGDST_HOSTEMU
@@ -231,8 +293,9 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
             if (ist0 < 0 || ist0 >= cx.nst || m0 < cx.a0 || m0 > cx.mmax) state = 1;  // egdst_simulator.c:215-216
             else { cur.ist = ist0; cur.cash = m0; egdst_fill_state(&cx, &cur); if (!feasible(&cx, &cur)) state = 1; }
         }
-        // the uniforms of period it+1 are drawn during period it: the Philox rounds are independent of the agent's
-        // state, so their integer pipeline work overlaps the table-gather latency of the current period
+        // Uniforms are drawn one period ahead of the transition that uses them: the Philox rounds are independent of
+        // the agent's state, so their integer pipeline work overlaps the table gathers.  The plain order steps into
+        // period it during period it and draws the uniforms of it+1; the pipelined order steps into it+1 and draws it+2.
         unsigned pr0 = 0, pr1 = 0, pr2 = 0, pr3 = 0;
         const unsigned long long gid = (unsigned long long)(S.agent0 + isim);
         if (PHILOX && nt > 1)
@@ -245,179 +308,218 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
         const int na = S.nsim - tileidx * 32 < 32 ? S.nsim - tileidx * 32 : 32;
         const bool vecok = VEC && (((size_t)sims & 15) == 0);
         double *wdst = SIMS ? sims + (size_t)tileidx * 32 * rowpitch + (vecok ? (size_t)wa0 * rowpitch + 2 * wk : 0) : (double *)0;
+#if EGDST_NCONT == 0
+        // PIPE: the index entry of the next record's cell (tabnext: its lookup goes through the tables), gathered one
+        // period ahead so that it is in flight while the value, utility, moments and store pass of a period run
+        EgdstLutEntry ent;
+        bool tabnext = false;
+        auto lookup_begin = [&](int p, const PeriodVars &v) {
+            const int cell = egdst_cell(P, ivec, p, v.ist);
+            const int nmraw = HDR ? H.h[p * cx.nst + v.ist].n : P.mlen[cell];
+            const int nm = HDR ? (nmraw & ~EGDST_HDR_NOTAB) : nmraw;
+            const bool tabok = HDR ? (nmraw & EGDST_HDR_NOTAB) == 0 : P.tabOk[cell] != 0;
+            tabnext = egdst_sim_tab(P, nm, tabok);
+            if (tabnext) ent = egdst_lut_entry<true>(P, cell, v.cash, l2keep);
+        };
+        if (PIPE && state == 0) {  // period 0 has no transition into it
+            eqs_sim(&cx, &cur, (const PeriodVars *)0, eqs);
+            lookup_begin(0, cur);
+        }
+#endif
         for (int it = 0; it < nt; it++) {
             const unsigned cr0 = pr0, cr1 = pr1, cr2 = pr2;
-            if (PHILOX && it > 0 && it + 1 < nt)
-                egdst_philox4x32((unsigned)gid, (unsigned)(gid >> 32), (unsigned)(it + 1), 0u, (unsigned)S.seed, (unsigned)(S.seed >> 32), pr0, pr1, pr2, pr3);
-            if (state == 0 && it > 0) {
-                PeriodVars nx = cur;
-                nx.it = it;
-                nx.savings = cur.savings;
-                double rrr, rrr1, rrr2;
-                if (!PHILOX) {
-                    const double *r3 = rs + (size_t)3 * (it - 1);
-                    rrr = r3[0]; rrr1 = r3[1]; rrr2 = r3[2];
-                } else {
-                    rrr = egdst_u01(cr0); rrr1 = egdst_u01(cr1); rrr2 = egdst_u01(cr2);
-                }
-                if (rrr2 > survival(&cx, &cur)) {
-                    state = 1;  // death: the rest of the record stays NaN
-                } else {
-                    int chosen = -1, lastfeas = -1;
-                    for (int ist1 = 0; ist1 < cx.nst; ist1++) {
-#if EGDST_NCONT > 0
-                        {   // continuous states are carried by value: only the cells at their first grid point stand
-                            // for the discrete part of the state (egdst_simulator.c:268-271)
-                            bool first = true;
-#pragma unroll
-                            for (int k = 0; k < EGDST_NCONT; k++) {
-                                const int j0 = egdst_contvar[k];
-                                if ((ist1 / (int)cx.stm[cx.nnst + j0]) % (int)cx.stm[j0] != 0) first = false;
-                            }
-                            if (!first) continue;
-                        }
-#endif
-                        nx.ist = ist1;
-                        egdst_fill_state(&cx, &nx);
-#if EGDST_NCONT > 0
-                        trpr_cont(&cx, &cur, &nx);  // exact next-period values of the continuous states
-#endif
-                        if (!feasible(&cx, &nx)) continue;
-                        lastfeas = ist1;
-                        double pr;
-#if EGDST_OPT_TRPRNOSH
-                        pr = trpr(&cx, &cur, &nx, 0);
-#else
-                        mu = mu_param(&cx, &cur, &nx); sigma = sigma_param(&cx, &cur, &nx);
-                        nx.shock = (sigma <= 0) ? egdst_expectation(&cx, &cur, &nx) : egdst_cdfinv(rrr1, mu, sigma);
-                        pr = trpr(&cx, &cur, &nx, 0);
-#endif
-                        rrr -= pr;
-                        if (rrr <= 0) { chosen = ist1; break; }
-                    }
-                    if (chosen < 0) chosen = lastfeas < 0 ? 0 : lastfeas;  // the reference runs off the end here
-                    nx.ist = chosen;
-                    egdst_fill_state(&cx, &nx);
-#if EGDST_NCONT > 0
-                    trpr_cont(&cx, &cur, &nx);
-#endif
-#if EGDST_OPT_TRPRNOSH
-                    // shocks for the shock-independent case (egdst_simulator.c:292-298)
-                    mu = mu_param(&cx, &cur, &nx); sigma = sigma_param(&cx, &cur, &nx);
-                    nx.shock = (sigma <= 0) ? egdst_expectation(&cx, &cur, &nx) : egdst_cdfinv(rrr1, mu, sigma);
-#endif
-                    nx.cash = cashinhand(&cx, &cur, &nx);
-                    eqs_sim(&cx, &cur, &nx, eqs);
-                    cur = nx;
-                }
-            } else if (state == 0) {
-                eqs_sim(&cx, &cur, (const PeriodVars *)0, eqs);
-            }
-#if EGDST_NCONT > 0
-            if (state == 0) {
-                // Continuous states (egdst_simulator.c:309-365): consumption and value are the multilinear mix of the
-                // policies of the 2^NCONT surrounding grid cells (weights <= 0 are skipped, as there); the recorded
-                // cell and discrete decision are those of the corner at which the cumulated weight passes one half.
-                // The reference never assigns the value column on this branch (policy(...,0) skips it); here it is
-                // the same mix of the corner values.  At it == 0 the cell index of `init` may point at any grid point
-                // of a continuous state: its grid part is removed before the corners are addressed (the reference
-                // adds the corner offset on top of it and leaves the table, egdst_simulator.c:313).
-                int j1[EGDST_NCONT], stride[EGDST_NCONT];
-                double wlo[EGDST_NCONT], whi[EGDST_NCONT];
-                int base = cur.ist;
-#pragma unroll
-                for (int k = 0; k < EGDST_NCONT; k++) {
-                    const int j0 = egdst_contvar[k], n = (int)cx.stm[j0];
-                    const double *g = egdst_contgrid(k);
-                    const double x = cur.st[j0];
-                    stride[k] = (int)cx.stm[cx.nnst + j0];
-                    base -= ((cur.ist / stride[k]) % n) * stride[k];
-                    j1[k] = egdst_gridcell(x, g, n);
-                    wlo[k] = (g[j1[k] + 1] - x) / (g[j1[k] + 1] - g[j1[k]]);
-                    whi[k] = (x - g[j1[k]]) / (g[j1[k] + 1] - g[j1[k]]);
-                }
-                double wc = 0, wvf = 0, rr = .5;
-                int ist1 = -1, id1 = 0, istlast = -1, idlast = 0;
-                bool ok = true;
-                for (int ii = 0; ii < (1 << EGDST_NCONT) && ok; ii++) {
-                    double wt = 1;
-                    int ist = base;
-#pragma unroll
-                    for (int k = 0; k < EGDST_NCONT; k++) {
-                        const int up = (ii >> k) & 1;
-                        wt *= up ? whi[k] : wlo[k];
-                        ist += stride[k] * (j1[k] + up);
-                    }
-                    if (!(wt > 0)) continue;
-                    PeriodVars pv = cur;
-                    pv.ist = ist;
-                    double cc, vv;
-                    ok = egdst_sim_policy_cell(P, cx, egdst_cell(P, ivec, it, ist), pv, l2keep, cc, vv);
-                    if (!ok) break;
-                    wc += cc * wt;
-                    wvf += vv * wt;
-                    rr -= wt;
-                    istlast = ist; idlast = pv.id;
-                    if (rr < 0 && ist1 == -1) { ist1 = ist; id1 = pv.id; }
-                }
-                if (!ok || istlast < 0) state = 1;
-                else {
-                    if (ist1 < 0) { ist1 = istlast; id1 = idlast; }
-                    c = MIN(wc, cur.cash - cx.a0);
-                    cur.savings = cur.cash - c;
-                    vf = wvf;
-                    cur.ist = ist1;
-                    cur.id = id1;
-                    egdst_fill_decision(&cx, &cur);
-                    uu = utility(&cx, &cur, c); bb = discount(&cx, &cur);
-                }
-            }
-#else
-            if (state == 0) {
-                // policy (egdst_simulator.c:145-199)
-                const int cell = egdst_cell(P, ivec, it, cur.ist);
-                const EgdstCellHdr *hc = H.h + it * cx.nst + cur.ist;
-                const int nmraw = HDR ? hc->n : P.mlen[cell];
-                const int nm = HDR ? (nmraw & ~EGDST_HDR_NOTAB) : nmraw;
-                const bool tabok = HDR ? (nmraw & EGDST_HDR_NOTAB) == 0 : P.tabOk[cell] != 0;
-                EgdstInterval iv;
-                if (!egdst_sim_interval(P, cell, nm, tabok, cur.cash, l2keep, iv)) { state = 1; }
-                else {
-                    double wl, wr;
-                    egdst_sim_weights(iv, cur.cash, wl, wr);
-                    c = iv.c1 * wl + iv.c0 * wr;
-                    cur.savings = cur.cash - c;
-                    const int nth = HDR ? hc->nth : P.thlen[cell];
-                    if (HDR && nth <= EGDST_SIM_TH8) cur.id = egdst_policy_decision(cur.cash, hc->th, hc->dd, nth);
-                    else cur.id = egdst_policy_decision(cur.cash, P.thTH + (size_t)cell * cx.nthrhmax, P.thD + (size_t)cell * cx.nthrhmax, nth);
-                    egdst_fill_decision(&cx, &cur);
-                    const double evf = HDR ? hc->evf : P.evf[cell];  // == V(row 0)
-                    const double M1 = HDR ? hc->M1 : egdst_colM(P, cell)[1];
-                    uu = utility(&cx, &cur, c); bb = discount(&cx, &cur);  // output columns 9, 10; shared with the exact value below
-                    if (cur.cash < M1 && evf > -EGDST_INF) vf = uu + bb * evf;
-                    else vf = iv.v1 * wl + iv.v0 * wr;
-                }
-            }
-#endif
-            // stage the record of this period (PB == 2: odd periods go to the second half of the agent's row)
+            if (PHILOX && (PIPE ? it + 2 < nt : it > 0 && it + 1 < nt))
+                egdst_philox4x32((unsigned)gid, (unsigned)(gid >> 32), (unsigned)(it + (PIPE ? 2 : 1)), 0u, (unsigned)S.seed, (unsigned)(S.seed >> 32), pr0, pr1, pr2, pr3);
+            // the record of this period is staged in the tile (PB == 2: odd periods go to the second half of the agent's row)
             const int half = (PB == 2) ? (it & 1) : 0;
             const int hoff = half * NSO;
 #define EGDST_REC(j) tile[EGDST_TILE_POS(lane, hoff + (j))]
-            if (state == 0) {
-                EGDST_REC(0) = cur.cash; EGDST_REC(1) = c; EGDST_REC(2) = cur.savings; EGDST_REC(3) = vf; EGDST_REC(4) = (double)cur.id; EGDST_REC(5) = (double)cur.ist;
-                EGDST_REC(6) = mu; EGDST_REC(7) = sigma; EGDST_REC(8) = cur.shock; EGDST_REC(9) = uu; EGDST_REC(10) = bb;
+            int rstate;  // state of this period's record; PIPE: `state` moves on to the next period
+            if (!PIPE) {
+                if (state == 0 && it > 0) {
+                    double rrr, rrr1, rrr2;
+                    if (!PHILOX) {
+                        const double *r3 = rs + (size_t)3 * (it - 1);
+                        rrr = r3[0]; rrr1 = r3[1]; rrr2 = r3[2];
+                    } else {
+                        rrr = egdst_u01(cr0); rrr1 = egdst_u01(cr1); rrr2 = egdst_u01(cr2);
+                    }
+                    PeriodVars nx;
+                    if (!egdst_sim_transition(cx, cur, nx, it, rrr, rrr1, rrr2, mu, sigma, eqs)) state = 1;  // death: the rest of the record stays NaN
+                    else cur = nx;
+                } else if (state == 0) {
+                    eqs_sim(&cx, &cur, (const PeriodVars *)0, eqs);
+                }
+#if EGDST_NCONT > 0
+                if (state == 0) {
+                    // Continuous states (egdst_simulator.c:309-365): consumption and value are the multilinear mix of the
+                    // policies of the 2^NCONT surrounding grid cells (weights <= 0 are skipped, as there); the recorded
+                    // cell and discrete decision are those of the corner at which the cumulated weight passes one half.
+                    // The reference never assigns the value column on this branch (policy(...,0) skips it); here it is
+                    // the same mix of the corner values.  At it == 0 the cell index of `init` may point at any grid point
+                    // of a continuous state: its grid part is removed before the corners are addressed (the reference
+                    // adds the corner offset on top of it and leaves the table, egdst_simulator.c:313).
+                    int j1[EGDST_NCONT], stride[EGDST_NCONT];
+                    double wlo[EGDST_NCONT], whi[EGDST_NCONT];
+                    int base = cur.ist;
 #pragma unroll
-                for (int i = 0; i < EGDST_NNST; i++) EGDST_REC(11 + i) = cur.st[i];
+                    for (int k = 0; k < EGDST_NCONT; k++) {
+                        const int j0 = egdst_contvar[k], n = (int)cx.stm[j0];
+                        const double *g = egdst_contgrid(k);
+                        const double x = cur.st[j0];
+                        stride[k] = (int)cx.stm[cx.nnst + j0];
+                        base -= ((cur.ist / stride[k]) % n) * stride[k];
+                        j1[k] = egdst_gridcell(x, g, n);
+                        wlo[k] = (g[j1[k] + 1] - x) / (g[j1[k] + 1] - g[j1[k]]);
+                        whi[k] = (x - g[j1[k]]) / (g[j1[k] + 1] - g[j1[k]]);
+                    }
+                    double wc = 0, wvf = 0, rr = .5;
+                    int ist1 = -1, id1 = 0, istlast = -1, idlast = 0;
+                    bool ok = true;
+                    for (int ii = 0; ii < (1 << EGDST_NCONT) && ok; ii++) {
+                        double wt = 1;
+                        int ist = base;
 #pragma unroll
-                for (int i = 0; i < EGDST_NND; i++) EGDST_REC(11 + EGDST_NNST + i) = cur.dc[i];
+                        for (int k = 0; k < EGDST_NCONT; k++) {
+                            const int up = (ii >> k) & 1;
+                            wt *= up ? whi[k] : wlo[k];
+                            ist += stride[k] * (j1[k] + up);
+                        }
+                        if (!(wt > 0)) continue;
+                        PeriodVars pv = cur;
+                        pv.ist = ist;
+                        double cc, vv;
+                        ok = egdst_sim_policy_cell(P, cx, egdst_cell(P, ivec, it, ist), pv, l2keep, cc, vv);
+                        if (!ok) break;
+                        wc += cc * wt;
+                        wvf += vv * wt;
+                        rr -= wt;
+                        istlast = ist; idlast = pv.id;
+                        if (rr < 0 && ist1 == -1) { ist1 = ist; id1 = pv.id; }
+                    }
+                    if (!ok || istlast < 0) state = 1;
+                    else {
+                        if (ist1 < 0) { ist1 = istlast; id1 = idlast; }
+                        c = MIN(wc, cur.cash - cx.a0);
+                        cur.savings = cur.cash - c;
+                        vf = wvf;
+                        cur.ist = ist1;
+                        cur.id = id1;
+                        egdst_fill_decision(&cx, &cur);
+                        uu = utility(&cx, &cur, c); bb = discount(&cx, &cur);
+                    }
+                }
+#else
+                if (state == 0) {
+                    // policy (egdst_simulator.c:145-199)
+                    const int cell = egdst_cell(P, ivec, it, cur.ist);
+                    const EgdstCellHdr *hc = H.h + it * cx.nst + cur.ist;
+                    const int nmraw = HDR ? hc->n : P.mlen[cell];
+                    const int nm = HDR ? (nmraw & ~EGDST_HDR_NOTAB) : nmraw;
+                    const bool tabok = HDR ? (nmraw & EGDST_HDR_NOTAB) == 0 : P.tabOk[cell] != 0;
+                    EgdstInterval iv;
+                    if (!egdst_sim_interval(P, cell, nm, tabok, cur.cash, l2keep, iv)) { state = 1; }
+                    else {
+                        double wl, wr;
+                        egdst_sim_weights(iv, cur.cash, wl, wr);
+                        c = iv.c1 * wl + iv.c0 * wr;
+                        cur.savings = cur.cash - c;
+                        const int nth = HDR ? hc->nth : P.thlen[cell];
+                        if (HDR && nth <= EGDST_SIM_TH8) cur.id = egdst_policy_decision(cur.cash, hc->th, hc->dd, nth);
+                        else cur.id = egdst_policy_decision(cur.cash, P.thTH + (size_t)cell * cx.nthrhmax, P.thD + (size_t)cell * cx.nthrhmax, nth);
+                        egdst_fill_decision(&cx, &cur);
+                        const double evf = HDR ? hc->evf : P.evf[cell];  // == V(row 0)
+                        const double M1 = HDR ? hc->M1 : egdst_colM(P, cell)[1];
+                        uu = utility(&cx, &cur, c); bb = discount(&cx, &cur);  // output columns 9, 10; shared with the exact value below
+                        if (cur.cash < M1 && evf > -EGDST_INF) vf = uu + bb * evf;
+                        else vf = iv.v1 * wl + iv.v0 * wr;
+                    }
+                }
+#endif
+                if (state == 0) {
+                    EGDST_REC(0) = cur.cash; EGDST_REC(1) = c; EGDST_REC(2) = cur.savings; EGDST_REC(3) = vf; EGDST_REC(4) = (double)cur.id; EGDST_REC(5) = (double)cur.ist;
+                    EGDST_REC(6) = mu; EGDST_REC(7) = sigma; EGDST_REC(8) = cur.shock; EGDST_REC(9) = uu; EGDST_REC(10) = bb;
 #pragma unroll
-                for (int i = 0; i < EGDST_NREQ; i++) EGDST_REC(11 + EGDST_NNST + EGDST_NND + i) = eqs[i];
-            } else {
+                    for (int i = 0; i < EGDST_NNST; i++) EGDST_REC(11 + i) = cur.st[i];
 #pragma unroll
-                for (int j = 0; j < NSO; j++) EGDST_REC(j) = NaN;
+                    for (int i = 0; i < EGDST_NND; i++) EGDST_REC(11 + EGDST_NNST + i) = cur.dc[i];
+#pragma unroll
+                    for (int i = 0; i < EGDST_NREQ; i++) EGDST_REC(11 + EGDST_NNST + EGDST_NND + i) = eqs[i];
+                } else {
+#pragma unroll
+                    for (int j = 0; j < NSO; j++) EGDST_REC(j) = NaN;
+                }
+                rstate = state;
             }
+#if EGDST_NCONT == 0
+            else {
+                // Pipelined order: (1) the policy of period it from the index entry gathered during period it-1, and
+                // the record columns that do not wait for the value; (2) the transition into period it+1 and the
+                // index-entry gather of its cell; (3) value, utility and discount of period it.  Only independent
+                // work moves, every expression is the one of the plain order: the records are the same to the bit.
+                double evf = 0.0, vlin = 0.0;
+                bool vexact = false;
+                if (state == 0) {
+                    const int cell = egdst_cell(P, ivec, it, cur.ist);
+                    const EgdstCellHdr *hc = H.h + it * cx.nst + cur.ist;
+                    const int nm = HDR ? (hc->n & ~EGDST_HDR_NOTAB) : P.mlen[cell];
+                    EgdstInterval iv;
+                    if (nm < 2) { state = 1; }
+                    else {
+                        if (tabnext) egdst_cell_lookup_finish(P, cell, cur.cash, nm, ent, iv, l2keep);
+                        else egdst_sim_interval(P, cell, nm, false, cur.cash, l2keep, iv);
+                        double wl, wr;
+                        egdst_sim_weights(iv, cur.cash, wl, wr);
+                        c = iv.c1 * wl + iv.c0 * wr;
+                        cur.savings = cur.cash - c;
+                        const int nth = HDR ? hc->nth : P.thlen[cell];
+                        if (HDR && nth <= EGDST_SIM_TH8) cur.id = egdst_policy_decision(cur.cash, hc->th, hc->dd, nth);
+                        else cur.id = egdst_policy_decision(cur.cash, P.thTH + (size_t)cell * cx.nthrhmax, P.thD + (size_t)cell * cx.nthrhmax, nth);
+                        egdst_fill_decision(&cx, &cur);
+                        evf = HDR ? hc->evf : P.evf[cell];  // == V(row 0)
+                        const double M1 = HDR ? hc->M1 : egdst_colM(P, cell)[1];
+                        vexact = cur.cash < M1 && evf > -EGDST_INF;  // the value is exact below M[1], else interpolated
+                        vlin = iv.v1 * wl + iv.v0 * wr;
+                    }
+                }
+                rstate = state;
+                if (state == 0) {
+                    EGDST_REC(0) = cur.cash; EGDST_REC(1) = c; EGDST_REC(2) = cur.savings; EGDST_REC(4) = (double)cur.id; EGDST_REC(5) = (double)cur.ist;
+                    EGDST_REC(6) = mu; EGDST_REC(7) = sigma; EGDST_REC(8) = cur.shock;
+#pragma unroll
+                    for (int i = 0; i < EGDST_NNST; i++) EGDST_REC(11 + i) = cur.st[i];
+#pragma unroll
+                    for (int i = 0; i < EGDST_NND; i++) EGDST_REC(11 + EGDST_NNST + i) = cur.dc[i];
+#pragma unroll
+                    for (int i = 0; i < EGDST_NREQ; i++) EGDST_REC(11 + EGDST_NNST + EGDST_NND + i) = eqs[i];
+                } else {
+#pragma unroll
+                    for (int j = 0; j < NSO; j++) EGDST_REC(j) = NaN;
+                }
+                PeriodVars nx;
+                bool stepped = false;
+                if (state == 0 && it + 1 < nt) {
+                    double rrr, rrr1, rrr2;
+                    if (!PHILOX) {
+                        const double *r3 = rs + (size_t)3 * it;
+                        rrr = r3[0]; rrr1 = r3[1]; rrr2 = r3[2];
+                    } else {
+                        rrr = egdst_u01(cr0); rrr1 = egdst_u01(cr1); rrr2 = egdst_u01(cr2);
+                    }
+                    stepped = egdst_sim_transition(cx, cur, nx, it + 1, rrr, rrr1, rrr2, mu, sigma, eqs);
+                    if (!stepped) state = 1;  // death in period it+1; this period's record stands
+                    else lookup_begin(it + 1, nx);
+                }
+                if (rstate == 0) {
+                    uu = utility(&cx, &cur, c); bb = discount(&cx, &cur);
+                    vf = vexact ? uu + bb * evf : vlin;
+                    EGDST_REC(3) = vf; EGDST_REC(9) = uu; EGDST_REC(10) = bb;
+                }
+                if (stepped) cur = nx;
+            }
+#endif
 #undef EGDST_REC
-            const bool clean = MOM && __all_sync(EGDST_FULL, state == 0) && it > 0;  // no NaN record in the tile
+            const bool clean = MOM && __all_sync(EGDST_FULL, rstate == 0) && it > 0;  // no NaN record in the tile
             __syncwarp();
             if (SIMS && (PB == 1 || half == 1)) {
                 if (vecok) {
@@ -470,18 +572,11 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
                 }
                 // a clean tile adds 32 to the count of every column: one integer atomic per tile instead of NSO
                 // floating-point ones (clean_s[it], folded into the counts at the final flush)
-                const bool cntint = (momsm || PB == 2) && clean && __all_sync(EGDST_FULL, lane >= NSO || n == 32.0);
+                const bool cntint = momsm && clean && __all_sync(EGDST_FULL, lane >= NSO || n == 32.0);
                 if (momsm) {
                     if (cntint && lane == 0) atomicAdd(clean_s + it, 1);
                     if (lane < NSO && n > 0) {
                         double *d = smom + ((size_t)it * NSO + lane) * 3;
-                        atomicAdd(d + 0, s1); atomicAdd(d + 1, s2);
-                        if (!cntint) atomicAdd(d + 2, n);
-                    }
-                } else if (PB == 2) {
-                    if (cntint && lane == 0) atomicAdd(clean_g + it, 1);
-                    if (lane < NSO && n > 0) {
-                        double *d = gslice + ((size_t)it * NSO + lane) * 3;
                         atomicAdd(d + 0, s1); atomicAdd(d + 1, s2);
                         if (!cntint) atomicAdd(d + 2, n);
                     }
@@ -504,18 +599,3 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
 }
 #undef EGDST_TILE_POS
 
-// sums the per-CTA moment slices of the global scratch into the caller's moment buffer (adds, like the kernel's own
-// flush); the integer clean-tile counters become 32 agents per tile in every column's count
-__global__ void egdst_k_momreduce(const double *scratch, int nslices, int nt, int nso, double *moments) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    const int n = nt * nso * 3;
-    if (i >= n) return;
-    const size_t stride = (size_t)n + nt;
-    double acc = 0.0;
-    for (int c = 0; c < nslices; c++) {
-        const double *sl = scratch + (size_t)c * stride;
-        acc += sl[i];
-        if (i % 3 == 2) acc += 32.0 * reinterpret_cast<const int *>(sl + n)[i / (3 * nso)];
-    }
-    if (acc != 0.0) atomicAdd(moments + i, acc);
-}

@@ -250,11 +250,9 @@ EGDST_DEV EgdstInterval egdst_load_interval_keep(const EgdstRow *p, unsigned lon
 #endif
 }
 
-// Index entry of x's bucket and the rank it gives: (#rows <= x) - 1, where crowded buckets (more than three rows: the
-// grid is dense around a focal point or holds double points) bisect their remaining rows of M.  Not clamped.  KEEP:
-// load with the evict_last hint `pol`.
+// Index entry of x's bucket.  KEEP: load with the evict_last hint `pol`.
 template <bool KEEP = false>
-EGDST_DEV int egdst_lut_rank(const EgdstDev &P, int cell, const double *M, double x, unsigned long long pol = 0ULL) {
+EGDST_DEV EgdstLutEntry egdst_lut_entry(const EgdstDev &P, int cell, double x, unsigned long long pol = 0ULL) {
     int b = egdst_lut_key(x, P.cx.a0, P.mbits);
     b = b < 0 ? 0 : (b > P.lutcap - 1 ? P.lutcap - 1 : b);
     const EgdstLutEntry *lut = egdst_cell_lut(P, cell);
@@ -272,6 +270,11 @@ EGDST_DEV int egdst_lut_rank(const EgdstDev &P, int cell, const double *M, doubl
         e.l = r0.x; e.cnt = r0.y; e.m0 = __hiloint2double(r0.w, r0.z); e.m1 = r1.x; e.m2 = r1.y;
     }
 #endif
+    return e;
+}
+// The rank the index entry e of x's bucket gives: (#rows <= x) - 1, where crowded buckets (more than three rows: the
+// grid is dense around a focal point or holds double points) bisect their remaining rows of M.  Not clamped.
+EGDST_DEV int egdst_lut_entry_rank(const EgdstLutEntry &e, const double *M, double x) {
     int i = e.l - 1 + (e.m0 <= x ? 1 : 0) + (e.m1 <= x ? 1 : 0) + (e.m2 <= x ? 1 : 0);
     if (e.cnt > 3 && e.m2 <= x) {
         int l = e.l + 3, h = e.l + e.cnt;
@@ -279,6 +282,10 @@ EGDST_DEV int egdst_lut_rank(const EgdstDev &P, int cell, const double *M, doubl
         i = l - 1;
     }
     return i;
+}
+template <bool KEEP = false>
+EGDST_DEV int egdst_lut_rank(const EgdstDev &P, int cell, const double *M, double x, unsigned long long pol = 0ULL) {
+    return egdst_lut_entry_rank(egdst_lut_entry<KEEP>(P, cell, x, pol), M, x);
 }
 
 // The record of rows i and i+1 of a cell: from the row table when the cell's tables may be used (tab,
@@ -313,5 +320,17 @@ EGDST_DEV int egdst_cell_lookup(const EgdstDev &P, int cell, bool tab, double x,
         i = egdst_bracket(x, M, n, 0);
     }
     iv = egdst_cell_interval<KEEP>(P, cell, tab, i, pol);
+    return i;
+}
+
+// The second half of egdst_cell_lookup for a cell with tables, from the index entry e of x (egdst_lut_entry<true>):
+// the simulator's pipelined period loop issues the entry gather a period ahead of this.  The solver keeps the fused
+// egdst_cell_lookup: built on these halves, the grid-scope solve kernel gets a larger stack frame.
+EGDST_DEV int egdst_cell_lookup_finish(const EgdstDev &P, int cell, double x, int n, const EgdstLutEntry &e, EgdstInterval &iv,
+                                       unsigned long long pol) {
+    int i = egdst_lut_entry_rank(e, egdst_colM(P, cell), x);
+    i = i > n - 2 ? n - 2 : i;
+    i = i < 0 ? 0 : i;
+    iv = egdst_cell_interval<true>(P, cell, true, i, pol);
     return i;
 }
