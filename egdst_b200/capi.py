@@ -155,6 +155,13 @@ class Solution:
             self.lib._raise(rc)
         return buf.reshape(4, n.value).T.copy()
 
+    def set_choice_draws(self, on: bool):
+        """Smoothing mode only: simulations of this solution draw each period's decision from the choice probabilities
+        (on) or take the modal choice (off, the default).  See egdst_solution_set_choice_draws in include/egdst_b200.h."""
+        rc = self.lib.L.egdst_solution_set_choice_draws(self.handle, 1 if on else 0)
+        if rc:
+            self.lib._raise(rc)
+
     def status(self, ivec: int = 0):
         it, ist, idd = C.c_int(0), C.c_int(0), C.c_int(0)
         code = self.lib.L.egdst_solution_status(self.handle, ivec, C.byref(it), C.byref(ist), C.byref(idd))
@@ -182,7 +189,7 @@ class ModelLibrary:
     EXPORTS = ["egdst_abi_version", "egdst_model_key", "egdst_model_nparam", "egdst_model_neq", "egdst_last_error",
                "egdst_set_stream", "egdst_launch_count", "egdst_profile_classes", "egdst_profile_class_name",
                "egdst_profile_enable", "egdst_profile_read", "egdst_solve", "egdst_solve_batch", "egdst_resolve", "egdst_solution_sizes",
-               "egdst_solution_export", "egdst_solution_choice_cell", "egdst_solution_status", "egdst_solution_nvec", "egdst_solution_units", "egdst_solution_resends", "egdst_solution_phase_ms", "egdst_test_envelope2",
+               "egdst_solution_export", "egdst_solution_choice_cell", "egdst_solution_set_choice_draws", "egdst_solution_status", "egdst_solution_nvec", "egdst_solution_units", "egdst_solution_resends", "egdst_solution_phase_ms", "egdst_test_envelope2",
                "egdst_free_solution", "egdst_solution_import", "egdst_simulate", "egdst_simulate_philox",
                "egdst_simulate_device", "egdst_sim_moments", "egdst_sim_moments_device", "egdst_call", "egdst_shutdown"]
 
@@ -207,6 +214,7 @@ class ModelLibrary:
         L.egdst_solution_sizes.argtypes = [vp, _ip, _ip]
         L.egdst_solution_export.argtypes = [vp, _dp, _dp]
         L.egdst_solution_choice_cell.argtypes = [vp, C.c_int, C.c_int, C.c_int, C.c_int, _dp, C.c_int, _ip]
+        L.egdst_solution_set_choice_draws.argtypes = [vp, C.c_int]
         L.egdst_solution_status.argtypes = [vp, C.c_int, _ip, _ip, _ip]
         L.egdst_solution_nvec.argtypes = [vp]
         L.egdst_solution_units.argtypes = [vp]

@@ -171,6 +171,8 @@ struct egdst_solution {
     bool sizes_valid = false;
     std::vector<double> h_params;  // host copy of the parameter matrix of the last solve (simulator kernel arguments)
     std::vector<EgdstCellHdr> h_hdr; int hdr_ivec = -1;  // simulator cell headers (kernel argument), -1 = stale
+    bool choice_cells = false;  // the choice-specific cells hold a solve's result (an import leaves them empty)
+    bool choice_draws = false;  // simulations draw each period's decision from the choice probabilities
 };
 
 template <class T>
@@ -257,6 +259,8 @@ static void adopt(egdst_solution *s, const egdst_desc *d, const egdst_ctx &cx) {
     s->sizes_valid = false;
     s->h_params.clear();
     s->hdr_ivec = -1;
+    s->choice_cells = false;
+    s->choice_draws = false;
 }
 
 // every device array of a new object of the shape of d with nvec parameter vectors (s->P.cx: the model of d)
@@ -498,6 +502,7 @@ static int run_solve(egdst_solution *s, const egdst_desc *d, const double *param
     if (rc) return rc;
     s->sizes_valid = false;
     s->hdr_ivec = -1;
+    s->choice_cells = s->ncell_all > s->ncell;
     CK(cudaGetLastError());
     return 0;
 }

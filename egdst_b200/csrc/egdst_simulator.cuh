@@ -18,7 +18,7 @@
 // macro of the generated header (EGDST_OPT_TRPRNOSH ...): the period loop carries no run-time mode switches.
 #pragma once
 
-#include "egdst_tables.cuh"
+#include "egdst_solver.cuh"
 
 #define EGDST_NSIMOUT_MAX (11 + EGDST_NNST + EGDST_NND + EGDST_NREQ)
 #ifdef EGDST_HOSTEMU
@@ -214,7 +214,9 @@ EGDST_DEV bool egdst_sim_transition(const egdst_ctx &cx, const PeriodVars &cur, 
 //   mom[nt][nso][3] + clean[nt]       (mom_smem) per-CTA moment accumulators, flushed once at the end
 // Template parameters:
 //   PHILOX  uniforms from Philox4x32-10 (else: the caller's randstream, egdst_simulator.c:259-261)
-//   OUT     bit 0: write the sims array; bit 1: accumulate moments
+//   OUT     bit 0: write the sims array; bit 1: accumulate moments; bit 2 (smoothing images): choice draws, each period's
+//           decision drawn from the choice probabilities of the solve (egdst_choice_weights) and the record that of the
+//           drawn decision's choice cell; PB == 1 and !HDR only
 //   HDR     single-vector launch whose per-cell headers and parameter values travel in the kernel arguments
 //   PB      periods per write of the sims array:
 //     1  one record (8*nso bytes) per agent and store pass; rows padded to an odd stride (conflict-free staging and
@@ -237,8 +239,9 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
     constexpr bool SWZ = PB == 2;
     constexpr int TS = SWZ ? W : (W | 1);
     constexpr int WPB = (PB == 2 ? EGDST_SIM_WIDE : EGDST_SIM_BLOCK) / 32;
-    constexpr bool SIMS = (OUT & 1) != 0, MOM = (OUT & 2) != 0;
+    constexpr bool SIMS = (OUT & 1) != 0, MOM = (OUT & 2) != 0, DRAW = (OUT & 4) != 0;
     constexpr bool PIPE = PB == 2 && EGDST_NCONT == 0;  // pipelined period order
+    static_assert(!DRAW || (PB == 1 && !HDR && EGDST_SMOOTHING && EGDST_NCONT == 0), "choice draws: plain period order, choice cells in global memory");
     // position of column j in the row of the agent staged by lane l: rotated rows spread a column over the banks
 #define EGDST_TILE_POS(l, j) ((l) * TS + (SWZ ? (((j) + (((l) >> 2) & 3) >= W) ? (j) + (((l) >> 2) & 3) - W : (j) + (((l) >> 2) & 3)) : (j)))
     // blockIdx.y walks the parameter vectors of a batched sweep: same agents and shocks under every vector,
@@ -301,6 +304,13 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
         if (PHILOX && nt > 1)
             egdst_philox4x32((unsigned)gid, (unsigned)(gid >> 32), 1u, 0u, (unsigned)S.seed, (unsigned)(S.seed >> 32), pr0, pr1, pr2, pr3);
         const double *rs = PHILOX ? (const double *)0 : S.randstream + (S.rndtype == 1 ? 0 : (size_t)4 * nt * isim);
+        // DRAW: the choice uniform of period it is word 3 of the Philox block of (gid, it), whose words 0-2 feed the
+        // transition into it (period 0: a block of its own), or slot 3*(nt-1)+it of the agent's randstream block
+        unsigned pw3 = 0;
+        if (DRAW && PHILOX) {
+            unsigned q0, q1, q2;
+            egdst_philox4x32((unsigned)gid, (unsigned)(gid >> 32), 0u, 0u, (unsigned)S.seed, (unsigned)(S.seed >> 32), q0, q1, q2, pw3);
+        }
         // cooperative write of the tile: lane = (agent sub-index, 16-byte piece); running pointer over the periods
         constexpr bool VEC = (W & 1) == 0 && W <= 32;
         constexpr int SL = W / 2 <= 8 ? 8 : 16, APT = 32 / SL;
@@ -327,7 +337,7 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
         }
 #endif
         for (int it = 0; it < nt; it++) {
-            const unsigned cr0 = pr0, cr1 = pr1, cr2 = pr2;
+            const unsigned cr0 = pr0, cr1 = pr1, cr2 = pr2, cr3 = it > 0 ? pr3 : pw3;
             if (PHILOX && (PIPE ? it + 2 < nt : it > 0 && it + 1 < nt))
                 egdst_philox4x32((unsigned)gid, (unsigned)(gid >> 32), (unsigned)(it + (PIPE ? 2 : 1)), 0u, (unsigned)S.seed, (unsigned)(S.seed >> 32), pr0, pr1, pr2, pr3);
             // the record of this period is staged in the tile (PB == 2: odd periods go to the second half of the agent's row)
@@ -410,6 +420,46 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
                     }
                 }
 #else
+#if EGDST_SMOOTHING
+                if (DRAW) {
+                    if (state == 0) {
+                        // choice draw: P_d(cash) as the solve weighs decision d, d = the first available decision whose
+                        // cumulative probability reaches u, and the policy and value of d's choice cell by the rules of
+                        // the modal branch below (interpolation, exact value below M[1])
+                        const int cell = egdst_cell(P, ivec, it, cur.ist);
+                        EgdstChoiceVals cv;
+                        egdst_choice_values(P, &cx, cell, cur, cv);
+                        double pe[EGDST_SMOOTH_MAXND], ssum, wmax;
+                        for (int d = 0; d < cx.nd; d++) pe[d] = 0.0;
+                        egdst_choice_weights(cx.nd, cv, P.sigmaEps, ssum, wmax, [&](int d, double e) { pe[d] = e; });
+                        const double u = PHILOX ? egdst_u01(cr3) : rs[(size_t)3 * (nt - 1) + it];
+                        int dr = -1;
+                        double cum = 0.0;
+                        for (int d = 0; d < cx.nd; d++) {
+                            if (!(cv.avail >> d & 1u)) continue;
+                            cum += pe[d] / ssum;
+                            dr = d;  // the last available decision if rounding keeps the sum below u
+                            if (cum >= u) break;
+                        }
+                        if (dr < 0) { state = 1; }  // no decision available in (it, ist)
+                        else {
+                            const int dcell = egdst_dcell(P, cell, dr);
+                            EgdstInterval iv;
+                            egdst_sim_interval(P, dcell, P.mlen[dcell], P.tabOk[dcell] != 0, cur.cash, l2keep, iv);
+                            double wl, wr;
+                            egdst_sim_weights(iv, cur.cash, wl, wr);
+                            c = iv.c1 * wl + iv.c0 * wr;
+                            cur.savings = cur.cash - c;
+                            cur.id = dr;
+                            egdst_fill_decision(&cx, &cur);
+                            const double evf = P.evf[dcell], M1 = egdst_colM(P, dcell)[1];
+                            uu = utility(&cx, &cur, c); bb = discount(&cx, &cur);
+                            if (cur.cash < M1 && evf > -EGDST_INF) vf = uu + bb * evf;
+                            else vf = iv.v1 * wl + iv.v0 * wr;
+                        }
+                    }
+                } else
+#endif
                 if (state == 0) {
                     // policy (egdst_simulator.c:145-199)
                     const int cell = egdst_cell(P, ivec, it, cur.ist);

@@ -149,6 +149,82 @@ EGDST_DEV bool egdst_eval_node(const egdst_ctx *cx, const EgdstDev &P, const Egd
 // credit-constrained branch below the first endogenous point, transformed extrapolation of the value above the grid.
 #define EGDST_SMOOTH_MAXND 8
 #if EGDST_SMOOTHING
+// The choice-specific values at the cash x.cash of cell1 = (x.it, x.ist), by the rules above, with the caller's parameter
+// values in cx (the solve's, or a simulation launch's).  Per decision d: c[d], v[d] consumption and value at cash (v[d]
+// = -inf: not available, or no finite value), vl[d] the value at the bound of the unified grid.  avail: bit d set when
+// decision d is available (its cell has at least 3 rows); above: cash lies above some decision's grid; vmax: max of v.
+struct EgdstChoiceVals { double c[EGDST_SMOOTH_MAXND], v[EGDST_SMOOTH_MAXND], vl[EGDST_SMOOTH_MAXND], vmax; unsigned avail; bool above; };
+EGDST_DEV void egdst_choice_values(const EgdstDev &P, const egdst_ctx *cx, int cell1, PeriodVars x, EgdstChoiceVals &cv) {
+    const double cash = x.cash;
+    cv.vmax = -EGDST_INF; cv.avail = 0u; cv.above = false;
+    const int nm = P.mlen[cell1];
+    const double g0m = nm >= 3 ? egdst_colM(P, cell1)[nm - 2] : -EGDST_INF;  // second-to-last abscissa of the merged cell
+    for (int d1 = 0; d1 < cx->nd; d1++) {
+        cv.v[d1] = -EGDST_INF; cv.c[d1] = 0.0; cv.vl[d1] = -EGDST_INF;
+        const int dcell = egdst_dcell(P, cell1, d1);
+        if (P.mlen[dcell] < 3) continue;  // decision not available in (it, ist)
+        cv.avail |= 1u << d1;
+        const EgdstNext t = egdst_cell_tables(P, dcell);
+        cv.vl[d1] = t.V[t.n1];
+        cv.above = cv.above || cash > t.Mlast;
+        const bool tab = egdst_cell_has_tab(P, t.cell, t.n1 + 1);
+        EgdstInterval iv;
+        const int i = egdst_cell_lookup(P, t.cell, tab, cash, t.n1 + 1, iv);
+        double w = iv.g1 - iv.g0, y = iv.y;
+        double c1 = y != 0.0 ? egdst_lerp_y(cash, iv.g0, iv.g1, iv.c0, iv.c1, w, y) : egdst_lerp(cash, iv.g0, iv.g1, iv.c0, iv.c1);
+        if (cash > t.Mlast) c1 = MAX(c1, t.Clast);
+        cv.c[d1] = c1;
+        x.id = d1;
+        double v1;
+        if (cash < t.M1 && t.evf > -EGDST_INF) {
+            v1 = utility(cx, &x, cash - cx->a0) + discount(cx, &x) * t.evf;
+        } else {
+            if (i < 1) {
+                iv = egdst_cell_interval(P, t.cell, tab, 1);
+                w = iv.g1 - iv.g0; y = iv.y;
+            }
+            v1 = egdst_linter_extrap_iv(cx, &x, cash, iv.g0, iv.g1, iv.v0, iv.v1, t.M1, t.Mlast, w, y);
+            if (cash > t.Mlast && g0m > t.M1 && g0m < t.Mlast) {
+                // above the grid the value is extrapolated in the metric of the transform (egdst_lib.c:179-206), which depends on
+                // the chord it continues: the reference continues the last interval of the MERGED cell, so every decision's value
+                // is continued from that abscissa (g0m) -- the limit sigma -> 0 is then the reference's extrapolation exactly
+                EgdstInterval jv;
+                egdst_cell_lookup(P, t.cell, tab, g0m, t.n1 + 1, jv);
+                const double vg = egdst_lerp(g0m, jv.g0, jv.g1, jv.v0, jv.v1);
+                v1 = egdst_linter_extrap_iv(cx, &x, cash, g0m, t.Mlast, vg, t.V[t.n1], t.M1, t.Mlast, t.Mlast - g0m, 0.0);
+            }
+        }
+        cv.v[d1] = v1;
+        if (v1 > cv.vmax) cv.vmax = v1;
+    }
+}
+
+// The choice probabilities P_d = e_d / ssum of the values cv: f(d, e_d) is called for every decision with a weight, in
+// decision order, and ssum is the sum of the weights.  e_d = exp((w_d - wmax) / sigma), w_d = v_d, or above the unified
+// grid (all choice-specific tables end at its bound, egdst_ph_dsave) the value at the bound vl_d: the probabilities are
+// held at their values at the bound, because the reference holds the argmax of the bound there (it extrapolates the last
+// interval of the merged cell), so this is its limit as sigma -> 0; extrapolated choice-specific values are not compared
+// with each other.  False: no decision has a finite value, and every available decision weighs 1.
+template <class F>
+EGDST_DEV bool egdst_choice_weights(int nd, const EgdstChoiceVals &cv, double sig, double &ssum, double &wmax, F &&f) {
+    wmax = cv.vmax;
+    if (cv.above) { wmax = -EGDST_INF; for (int d1 = 0; d1 < nd; d1++) if (cv.v[d1] > -EGDST_INF && cv.vl[d1] > wmax) wmax = cv.vl[d1]; }
+    ssum = 0.0;
+    if (wmax > -EGDST_INF) {
+        for (int d1 = 0; d1 < nd; d1++) {
+            if (!(cv.v[d1] > -EGDST_INF)) continue;
+            const double wv = cv.above ? cv.vl[d1] : cv.v[d1];
+            if (!(wv > -EGDST_INF)) continue;
+            const double e = exp((wv - wmax) / sig);
+            ssum += e;
+            f(d1, e);
+        }
+    }
+    if (ssum > 0.0) return true;
+    for (int d1 = 0; d1 < nd; d1++) if (cv.avail >> d1 & 1u) { ssum += 1.0; f(d1, 1.0); }
+    return false;
+}
+
 // Out of line, with scalar arguments and the kernel-argument block read from its copy in global memory (P.self): the
 // reference-parity kernels must not pay registers, local memory or instruction-cache space for this mode (a by-reference
 // call would pin the caller's context structs to local memory).
@@ -160,78 +236,27 @@ EGDST_NOINLINE EgdstSmoothOut egdst_smooth_node(const EgdstDev *Pg, int ivec, in
     const egdst_ctx *cx = &cxs;
     PeriodVars next; next.it = it1; next.ist = ist1; next.id = 0; next.savings = savings; next.shock = shock; next.cash = cash;
     const int nd = cx->nd;
-    const int cell1 = egdst_cell(P, ivec, it1, ist1);
-    double vd[EGDST_SMOOTH_MAXND], md[EGDST_SMOOTH_MAXND], vl[EGDST_SMOOTH_MAXND];
-    double vmax = -EGDST_INF;
-    int nav = 0;
-    bool above = false;
-    const int nm = P.mlen[cell1];
-    const double g0m = nm >= 3 ? egdst_colM(P, cell1)[nm - 2] : -EGDST_INF;  // second-to-last abscissa of the merged cell
+    EgdstChoiceVals cv;
+    egdst_choice_values(P, cx, egdst_cell(P, ivec, it1, ist1), next, cv);
+    double md[EGDST_SMOOTH_MAXND];
     for (int d1 = 0; d1 < nd; d1++) {
-        vd[d1] = -EGDST_INF; md[d1] = 0.0; vl[d1] = -EGDST_INF;
-        const int dcell = egdst_dcell(P, cell1, d1);
-        if (P.mlen[dcell] < 3) continue;  // decision not available in (it+1, ist1)
-        const EgdstNext t = egdst_cell_tables(P, dcell);
-        vl[d1] = t.V[t.n1];
-        above = above || cash > t.Mlast;
-        const bool tab = egdst_cell_has_tab(P, t.cell, t.n1 + 1);
-        EgdstInterval iv;
-        const int i = egdst_cell_lookup(P, t.cell, tab, cash, t.n1 + 1, iv);
-        double w = iv.g1 - iv.g0, y = iv.y;
-        double c1 = y != 0.0 ? egdst_lerp_y(cash, iv.g0, iv.g1, iv.c0, iv.c1, w, y) : egdst_lerp(cash, iv.g0, iv.g1, iv.c0, iv.c1);
-        if (cash > t.Mlast) c1 = MAX(c1, t.Clast);
-        if (c1 <= 0) { o.bad = EGDST_PT_C1NEG; return o; }
+        md[d1] = 0.0;
+        if (!(cv.avail >> d1 & 1u)) continue;
+        if (cv.c[d1] <= 0) { o.bad = EGDST_PT_C1NEG; return o; }
         next.id = d1;
-        md[d1] = utility_marginal(cx, &next, c1);
-        double v1;
-        if (cash < t.M1 && t.evf > -EGDST_INF) {
-            v1 = utility(cx, &next, cash - cx->a0) + discount(cx, &next) * t.evf;
-        } else {
-            if (i < 1) {
-                iv = egdst_cell_interval(P, t.cell, tab, 1);
-                w = iv.g1 - iv.g0; y = iv.y;
-            }
-            v1 = egdst_linter_extrap_iv(cx, &next, cash, iv.g0, iv.g1, iv.v0, iv.v1, t.M1, t.Mlast, w, y);
-            if (cash > t.Mlast && g0m > t.M1 && g0m < t.Mlast) {
-                // above the grid the value is extrapolated in the metric of the transform (egdst_lib.c:179-206), which depends on
-                // the chord it continues: the reference continues the last interval of the MERGED cell, so every decision's value
-                // is continued from that abscissa (g0m) -- the limit sigma -> 0 is then the reference's extrapolation exactly
-                EgdstInterval jv;
-                egdst_cell_lookup(P, t.cell, tab, g0m, t.n1 + 1, jv);
-                const double vg = egdst_lerp(g0m, jv.g0, jv.g1, jv.v0, jv.v1);
-                v1 = egdst_linter_extrap_iv(cx, &next, cash, g0m, t.Mlast, vg, t.V[t.n1], t.M1, t.Mlast, t.Mlast - g0m, 0.0);
-            }
-        }
-        vd[d1] = v1;
-        if (v1 > vmax) vmax = v1;
-        nav++;
+        md[d1] = utility_marginal(cx, &next, cv.c[d1]);
     }
-    if (nav == 0 || (keep == 1 && !(vmax > -EGDST_INF))) { o.bad = EGDST_PT_EVFINF; return o; }  // the reference's evf = -inf abort (egdst_solver.c:596)
-    const double sig = P.sigmaEps;
-    // Above the unified grid (all choice-specific tables end at its bound, egdst_ph_dsave) the choice probabilities are
-    // held at their values at the bound, and the logsum moves with the probability-weighted extrapolated values: the
-    // reference holds the argmax of the bound there (it extrapolates the last interval of the merged cell), so this is
-    // its limit as sigma -> 0; extrapolated choice-specific values are not compared with each other.
-    double wmax = vmax;
-    if (above) { wmax = -EGDST_INF; for (int d1 = 0; d1 < nd; d1++) if (vd[d1] > -EGDST_INF && vl[d1] > wmax) wmax = vl[d1]; }
-    double ssum = 0.0, mu = 0.0, dv = 0.0;
-    if (wmax > -EGDST_INF) {
-        for (int d1 = 0; d1 < nd; d1++) {
-            if (!(vd[d1] > -EGDST_INF)) continue;
-            const double wv = above ? vl[d1] : vd[d1];
-            if (!(wv > -EGDST_INF)) continue;
-            const double e = exp((wv - wmax) / sig);
-            ssum += e; mu += e * md[d1];
-            if (above) dv += e * (vd[d1] - vl[d1]);
-        }
-    }
-    if (!(ssum > 0.0)) {  // keep == 0 with every value at -inf: the available decisions weigh equally
-        for (int d1 = 0; d1 < nd; d1++) if (md[d1] != 0.0) { ssum += 1.0; mu += md[d1]; }
+    if (cv.avail == 0u || (keep == 1 && !(cv.vmax > -EGDST_INF))) { o.bad = EGDST_PT_EVFINF; return o; }  // the reference's evf = -inf abort (egdst_solver.c:596)
+    double ssum, wmax, mu = 0.0, dv = 0.0;
+    if (!egdst_choice_weights(nd, cv, P.sigmaEps, ssum, wmax, [&](int d1, double e) {
+            mu += e * md[d1];
+            if (cv.above) dv += e * (cv.v[d1] - cv.vl[d1]);
+        })) {  // keep == 0 with every value at -inf
         o.mu = mu / ssum; o.ev = -EGDST_INF;
         return o;
     }
     o.mu = mu / ssum;
-    o.ev = wmax + sig * log(ssum) + dv / ssum;
+    o.ev = wmax + P.sigmaEps * log(ssum) + dv / ssum;
     return o;
 }
 

@@ -431,8 +431,12 @@ class EgdstModel:
         self.__dict__["M"], self.__dict__["D"] = sol.M, sol.D
         return self
 
-    def sim(self, init=None, shocks: str = "own_shocks", randstream=None):
-        """sims = egdst_simulator(model, rndtype), permuted to [nsim, nt, nsimout] (egdstmodel.m:1210-1276)."""
+    def sim(self, init=None, shocks: str = "own_shocks", randstream=None, draw_choices: bool = False):
+        """sims = egdst_simulator(model, rndtype), permuted to [nsim, nt, nsimout] (egdstmodel.m:1210-1276).
+
+        ``draw_choices`` (smoothing mode, ``sigma_eps > 0``): draw each period's decision from the choice probabilities
+        instead of taking the modal choice (egdst_solution_set_choice_draws); the uniform of period it is slot
+        3*(nt-1)+it of each agent's randstream block."""
         lib = self._capi()
         if self._solution is None:
             raise RuntimeError("The model needs to be compiled and solved first!")
@@ -449,6 +453,7 @@ class EgdstModel:
         if self.randstream is None:
             rng = np.random.default_rng()
             self.__dict__["randstream"] = rng.random(max(self.init.shape[0], 100) * self.nt * 100)
+        self._solution.set_choice_draws(draw_choices)
         sims = lib.simulate(self, self._solution, self.init, self.randstream, rndtype)  # [nsim, nt, nsimout]
         self.__dict__["sims"] = sims
         return self

@@ -138,6 +138,22 @@ int egdst_sim_moments(const egdst_desc *d, egdst_solution *s, int ivec0, int nve
 int egdst_sim_moments_device(const egdst_desc *d, egdst_solution *s, int ivec0, int nvec, const double *d_init, int nsim,
                              long long agent0, unsigned long long seed, double *d_moments);
 
+/* EXTENSION, smoothing mode only (desc.sigma_eps > 0): choice draws.  on != 0: every later simulation of s (all the
+ * simulate and moments entry points above) draws each period's decision d from the choice probabilities the solve
+ * weighs the decisions with, P_d(M) = softmax_d(v_d(M)/sigma_eps) over the available decisions (held at their values
+ * at the grid's bound above it; equal when every value is -inf): d is the first available decision whose cumulative
+ * probability reaches a uniform u.  The record is then that of d's choice cell (egdst_solution_choice_cell):
+ * consumption c_d(M), savings M - c, value v_d(M) (without the realised taste shock), decision d, utility and discount
+ * of (c, d).  No available decision: the record is NaN from that period on.  on = 0 (the default): the decision of
+ * the merged policy's thresholds, the modal choice.  The uniform of period it (0..nt-1):
+ *   randstream  slot 3*(nt-1)+it of the agent's 4*nt block (the transitions use slots 0..3*(nt-1)-1), shared by all
+ *               agents with rndtype 1 as the other slots are;
+ *   Philox      word 3 of the block of counter (agent, it), whose words 0-2 drive the transition into it.
+ * Returns 2 when on != 0 for a solution without choice cells (sigma_eps = 0, or imported), or for a model image with
+ * continuous states.  The setting belongs to the solution object: egdst_resolve keeps it, a new solve starts with
+ * it off. */
+int egdst_solution_set_choice_draws(egdst_solution *s, int on);
+
 /* ---- call -------------------------------------------------------------------------------- */
 /* sw: 1 utility, 2 marginal utility, 3 discount, 4 budget, 5 marginal budget, 6 value function;
  * args: [narg*k] column-major with k = 4,4,2,6,6,3 (egdst_call.c:45-58); res: [narg]. */
