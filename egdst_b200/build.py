@@ -24,8 +24,8 @@ LIBROOT = os.environ.get("EGDST_B200_LIB_DIR", os.path.join(HERE, "_lib"))
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--shared", "-fmad=false"] + os.environ.get("EGDST_NVCC_EXTRA", "").split()
 
-_SOURCES = ["egdst_capi.cu", "egdst_capi_sim.inc", "egdst_common.cuh", "egdst_envelope.cuh", "egdst_numerics.cuh",
-            "egdst_period.cuh", "egdst_simulator.cuh", "egdst_solver.cuh", "egdst_tables.cuh"]
+_SOURCES = ["egdst_capi.cu", "egdst_capi_sim.inc", "egdst_common.cuh", "egdst_envelope.cuh", "egdst_loglik.cuh",
+            "egdst_numerics.cuh", "egdst_period.cuh", "egdst_simulator.cuh", "egdst_solver.cuh", "egdst_tables.cuh"]
 
 
 def source_digest() -> str:

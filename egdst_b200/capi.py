@@ -183,6 +183,20 @@ class Solution:
         return int(self.lib.L.egdst_solution_resends(self.handle))
 
 
+def observations_from_sims(model, sims, consumption: bool = True) -> np.ndarray:
+    """The live records of a simulation ``sims`` [nsim, nt, nsimout] as observations for ``ModelLibrary.choice_loglik``:
+    [nobs, 5] (or [nobs, 4] without ``consumption``) of age t0 + it, state ist + 1, cash, decision id + 1 and
+    consumption, agent-major.  Dead and skipped records (NaN) are dropped."""
+    s = np.asarray(sims, dtype=np.float64)
+    cash, cons, dec, ist = s[:, :, 0], s[:, :, 1], s[:, :, 4], s[:, :, 5]
+    live = ~(np.isnan(cash) | np.isnan(dec) | np.isnan(ist))
+    ai, ti = np.nonzero(live)
+    cols = [model.t0 + ti.astype(np.float64), ist[ai, ti] + 1.0, cash[ai, ti], dec[ai, ti] + 1.0]
+    if consumption:
+        cols.append(cons[ai, ti])
+    return np.column_stack(cols) if ai.size else np.zeros((0, len(cols)))
+
+
 class ModelLibrary:
     """One loaded model image (libegdst_b200_<key>.so)."""
 
@@ -191,7 +205,8 @@ class ModelLibrary:
                "egdst_profile_enable", "egdst_profile_read", "egdst_solve", "egdst_solve_batch", "egdst_resolve", "egdst_solution_sizes",
                "egdst_solution_export", "egdst_solution_choice_cell", "egdst_solution_set_choice_draws", "egdst_solution_status", "egdst_solution_nvec", "egdst_solution_units", "egdst_solution_resends", "egdst_solution_phase_ms", "egdst_test_envelope2",
                "egdst_free_solution", "egdst_solution_import", "egdst_simulate", "egdst_simulate_philox",
-               "egdst_simulate_device", "egdst_sim_moments", "egdst_sim_moments_device", "egdst_call", "egdst_shutdown"]
+               "egdst_simulate_device", "egdst_sim_moments", "egdst_sim_moments_device", "egdst_choice_loglik",
+               "egdst_choice_loglik_device", "egdst_call", "egdst_shutdown"]
 
     def __init__(self, path: str):
         if not os.path.isfile(path):
@@ -231,6 +246,8 @@ class ModelLibrary:
         L.egdst_simulate_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, vp, C.c_int, C.c_longlong, C.c_ulonglong,
                                             vp, C.c_int, vp, vp]
         L.egdst_call.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, _dp, C.c_int, C.c_int, _dp]
+        L.egdst_choice_loglik.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, _dp, C.c_int, C.c_int, C.c_double, _dp, _dp]
+        L.egdst_choice_loglik_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, vp, C.c_int, C.c_int, C.c_double, vp, vp]
         L.egdst_sim_moments.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, _dp, C.c_int, C.c_longlong, C.c_ulonglong, _dp]
         L.egdst_sim_moments_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, vp, C.c_int, C.c_longlong, C.c_ulonglong, vp]
         L.egdst_test_envelope2.argtypes = [C.POINTER(EgdstDesc), C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, C.c_int, C.c_double,
@@ -382,6 +399,35 @@ class ModelLibrary:
         d = desc or Desc(model)
         nvec = sol.nvec - ivec0 if nvec is None else nvec
         rc = self.L.egdst_sim_moments_device(C.byref(d.c), sol.handle, ivec0, nvec, C.c_void_p(d_init), nsim, agent0, seed, C.c_void_p(d_moments))
+        if rc:
+            self._raise(rc)
+
+    def choice_loglik(self, model, sol: Solution, obs, sigma_c: float = 0.0, ivec0: int = 0, nvec: Optional[int] = None,
+                      rows: bool = False):
+        """Smoothing mode only: log-likelihood of the observations ``obs`` [nobs, 4 or 5] (age, 1-based state, cash,
+        1-based decision[, consumption]; see ``observations_from_sims``) under parameter vectors ivec0.. of ``sol``.
+        Returns the totals [nvec], and with ``rows=True`` also the per-row values [nvec, nobs].  See
+        egdst_choice_loglik in include/egdst_b200.h for the formula and the -inf / NaN rules."""
+        d = Desc(model)
+        o = np.atleast_2d(np.asarray(obs, dtype=np.float64))
+        nobs, k = o.shape
+        of = _arr(o.ravel(order="F"))
+        nvec = sol.nvec - ivec0 if nvec is None else nvec
+        tot = np.zeros(max(nvec, 1), dtype=np.float64)
+        rowll = np.empty(max(nvec, 1) * nobs, dtype=np.float64) if rows else None
+        rc = self.L.egdst_choice_loglik(C.byref(d.c), sol.handle, ivec0, nvec, _ptr(of), nobs, k, float(sigma_c), _ptr(tot), _ptr(rowll))
+        if rc:
+            self._raise(rc)
+        return (tot, rowll.reshape(nvec, nobs)) if rows else tot
+
+    def choice_loglik_device(self, model, sol: Solution, d_obs: int, nobs: int, k: int, d_loglik: int, sigma_c: float = 0.0,
+                             d_rowll: int = 0, ivec0: int = 0, nvec: Optional[int] = None, desc: "Desc" = None):
+        """Asynchronous launch on the library stream; d_obs [k][nobs], d_loglik [nvec] (accumulated into: the caller
+        zeroes it) and d_rowll [nvec][nobs] (optional) are device addresses (ints).  Rows are not checked."""
+        d = desc or Desc(model)
+        nvec = sol.nvec - ivec0 if nvec is None else nvec
+        rc = self.L.egdst_choice_loglik_device(C.byref(d.c), sol.handle, ivec0, nvec, C.c_void_p(d_obs or None), nobs, k,
+                                               float(sigma_c), C.c_void_p(d_loglik or None), C.c_void_p(d_rowll or None))
         if rc:
             self._raise(rc)
 

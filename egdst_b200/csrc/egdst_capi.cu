@@ -23,6 +23,7 @@
 #endif
 #include "egdst_period.cuh"
 #include "egdst_simulator.cuh"
+#include "egdst_loglik.cuh"
 
 #ifndef EGDST_MODEL_KEY
 #define EGDST_MODEL_KEY "unknown"
@@ -164,8 +165,9 @@ struct egdst_solution {
     // grow-only buffers (grow)
     double *d_pack = 0; size_t pack_cap = 0;                // export / import staging
     EgdstCellHdr *d_hdr = 0; size_t hdr_cap = 0;            // simulator cell headers
+    double *d_llpart = 0; size_t llpart_cap = 0;            // block partials of the choice log-likelihood
     // every device allocation, by the field that holds it
-    std::vector<void **> owned{(void **)&d_pack, (void **)&d_hdr};
+    std::vector<void **> owned{(void **)&d_pack, (void **)&d_hdr, (void **)&d_llpart};
     // state of the current owner (adopt)
     std::vector<int> h_mlen, h_thlen, h_status;
     bool sizes_valid = false;

@@ -1,0 +1,102 @@
+// egdst_loglik.cuh -- log-likelihood of observed discrete choices (and consumption) under a taste-shock solution
+// (opt-in extension of the smoothing mode; the reference has no counterpart).
+//
+// One thread per (observation, parameter vector); blockIdx.y walks the vectors as in egdst_k_simulate.  A row's
+// choice probability is what the draw simulator evaluates at the same (it, ist, cash): egdst_choice_values and
+// egdst_choice_weights, so the edge rules (unavailable decisions, held at the bound above the grid, equal weights when
+// every value is -inf) have one implementation.  The per-vector total is deterministic: a fixed-order warp and block
+// reduction writes one partial per block, and egdst_k_choice_loglik_sum adds the partials of a vector in a fixed
+// order.  The block partition depends on nobs only, so the total of the same rows has the same bits for any nvec,
+// ivec0 or launch.
+#pragma once
+
+#include "egdst_solver.cuh"
+
+#ifdef EGDST_HOSTEMU
+#define EGDST_LL_BLOCK 64
+#else
+#define EGDST_LL_BLOCK 256
+#endif
+// minimum resident blocks per SM of egdst_k_choice_loglik: 3 caps it at 80 registers (60 bytes of spill stores) where
+// it needs 116 without a bound; 24 instead of 16 resident warps hide more of the table gathers' latency, and the
+// kernel ran 1.19-1.29x faster so (tools/loglik_time.py, DESIGN 6b)
+#ifndef EGDST_LL_MINBLOCKS
+#define EGDST_LL_MINBLOCKS 3
+#endif
+
+struct EgdstLlArgs {
+    const double *obs;   // [k][nobs]: age, state (1-based), cash, decision (1-based)[, consumption]
+    int nobs, k, ivec0;
+    int prm_on;          // 1: the parameter values are param (a single model: this call's); 0: the solve's (P.bparams)
+    double sigma_c;      // consumption measurement error (0: no consumption term)
+    double param[EGDST_NPARAM_];
+    double *rowll;       // [nvec][nobs] or null
+    double *part;        // [nvec][gridDim.x] block partials
+};
+
+#if EGDST_SMOOTHING && EGDST_NCONT == 0
+// log P_d(M) (+ the consumption term) of row i under the parameter values in cx; NaN for a malformed row
+EGDST_DEV double egdst_choice_loglik_row(const EgdstDev &P, const egdst_ctx &cx, int ivec, const EgdstLlArgs &A, int i) {
+    const size_t n = (size_t)A.nobs;  // column offsets in size_t: k * nobs exceeds INT_MAX for panels of 430 M rows
+    const double age = A.obs[i], sti = A.obs[n + i], cash = A.obs[2 * n + i], dob = A.obs[3 * n + i];
+    if (!(age >= cx.t0 && age <= cx.T && age == floor(age)) || !(sti >= 1 && sti <= cx.nst && sti == floor(sti)) ||
+        !(dob >= 1 && dob <= cx.nd && dob == floor(dob)) || !(cash >= cx.a0 && cash < EGDST_INF))
+        return EGDST_NAN;
+    PeriodVars x;
+    x.it = (int)age - cx.t0; x.ist = (int)sti - 1; x.id = (int)dob - 1;
+    x.cash = cash; x.savings = 0; x.shock = 0;
+    egdst_fill_state(&cx, &x);
+    egdst_fill_decision(&cx, &x);
+    const int id = x.id;
+    EgdstChoiceVals cv;
+    egdst_choice_values(P, &cx, egdst_cell(P, ivec, x.it, x.ist), x, cv);
+    double ssum, wmax, ed = 0.0;
+    egdst_choice_weights(cx.nd, cv, P.sigmaEps, ssum, wmax, [&](int d, double e) { if (d == id) ed = e; });
+    // a decision without weight (not available, or exp underflows) has probability 0
+    double ll = ed > 0.0 ? log(ed) - log(ssum) : -EGDST_INF;
+    if (A.k == 5 && A.sigma_c > 0.0) {
+        const double cobs = A.obs[4 * n + i];
+        if (!isnan(cobs)) {
+            const double z = (cobs - cv.c[id]) / A.sigma_c;
+            ll += -0.5 * z * z - 0.91893853320467274178 - log(A.sigma_c);  // log phi(z) - log sigma_c
+        }
+    }
+    return ll;
+}
+
+__global__ void __launch_bounds__(EGDST_LL_BLOCK, EGDST_LL_MINBLOCKS) egdst_k_choice_loglik(EgdstDev P, EgdstLlArgs A) {
+    __shared__ double wsum[EGDST_LL_BLOCK / 32];
+    const int i = blockIdx.x * EGDST_LL_BLOCK + threadIdx.x;
+    const int v = blockIdx.y, ivec = A.ivec0 + v;
+    double ll = 0.0;
+    if (i < A.nobs) {
+        egdst_ctx cx; egdst_load_ctx(P, ivec, cx);
+        cx.status = 0;
+        if (A.prm_on) {
+#pragma unroll
+            for (int j = 0; j < EGDST_NPARAM; j++) cx.param[j] = A.param[j];
+        }
+        ll = egdst_choice_loglik_row(P, cx, ivec, A, i);
+        if (A.rowll) A.rowll[(size_t)v * A.nobs + i] = ll;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) ll += __shfl_down_sync(0xffffffffu, ll, o);
+    if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = ll;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double s = 0.0;
+        for (int w = 0; w < EGDST_LL_BLOCK / 32; w++) s += wsum[w];
+        A.part[(size_t)v * gridDim.x + blockIdx.x] = s;
+    }
+}
+
+// loglik[v] += the sum of the nblocks partials of vector v (one warp per vector, lanes stride the partials)
+__global__ void __launch_bounds__(32) egdst_k_choice_loglik_sum(const double *part, int nblocks, double *loglik) {
+    const int v = blockIdx.x, lane = threadIdx.x;
+    double s = 0.0;
+    for (int b = lane; b < nblocks; b += 32) s += part[(size_t)v * nblocks + b];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+    if (lane == 0) loglik[v] += s;
+}
+#endif  // EGDST_SMOOTHING && EGDST_NCONT == 0

@@ -1,5 +1,5 @@
-"""Multi-GPU sharding of the two workloads that shard (SURVEY 8(e)): forward simulation over agents and batched
-solves over parameter vectors.  One process per GPU; ``torch.distributed`` is plumbing only -- the single
+"""Multi-GPU sharding of the workloads that shard (SURVEY 8(e)): forward simulation over agents, batched solves over
+parameter vectors, and the choice log-likelihood over observations.  One process per GPU; ``torch.distributed`` is plumbing only -- the single
 collective on the data path is one all-reduce of the simulated-moment buffer (NCCL over NVLink on GPUs, gloo in
 the CPU tests of the host logic).  A single model's backward induction does not shard ("replicas only"): every
 rank solves it redundantly, bit-identically, which is cheaper than broadcasting the 16 MB arena every period.
@@ -103,3 +103,23 @@ def solve_batch_sharded(lib, model, params: np.ndarray, init: np.ndarray, seed: 
     flat = table.reshape(-1)
     all_reduce_moments(flat, group)
     return table, (lo, hi)
+
+
+def choice_loglik_sharded(lib, model, sol, obs: np.ndarray, sigma_c: float = 0.0, rank: Optional[int] = None,
+                          world: Optional[int] = None, loglik_fn: Optional[Callable] = None, group=None):
+    """Choice log-likelihood of the observations ``obs`` [nobs, k] under every parameter vector of ``sol``: each rank
+    evaluates its contiguous block of rows and one all-reduce of the [nvec] totals gives every rank the sum.
+    Returns (totals [nvec], (lo, hi)).  ``loglik_fn(obs_block) -> totals`` replaces the CUDA call in the CPU tests."""
+    dist = _dist()
+    if world is None:
+        world = dist.get_world_size(group) if dist else 1
+    if rank is None:
+        rank = dist.get_rank(group) if dist else 0
+    obs = np.atleast_2d(np.asarray(obs, dtype=np.float64))
+    lo, hi = shard_range(obs.shape[0], rank, world)
+    if loglik_fn is None:
+        def loglik_fn(block):
+            return lib.choice_loglik(model, sol, block, sigma_c=sigma_c)
+    tot = np.ascontiguousarray(loglik_fn(obs[lo:hi]), dtype=np.float64)
+    all_reduce_moments(tot, group)
+    return tot, (lo, hi)

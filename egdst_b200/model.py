@@ -458,6 +458,14 @@ class EgdstModel:
         self.__dict__["sims"] = sims
         return self
 
+    def loglik(self, obs, sigma_c: float = 0.0) -> float:
+        """Smoothing mode (``sigma_eps > 0``) only: log-likelihood of the observations ``obs`` [nobs, 4 or 5] under the
+        current solution (egdst_choice_loglik; ``capi.observations_from_sims`` builds ``obs`` from simulated records)."""
+        lib = self._capi()
+        if self._solution is None:
+            raise RuntimeError("The model needs to be compiled and solved first!")
+        return float(lib.choice_loglik(self, self._solution, obs, sigma_c=sigma_c)[0])
+
     def call(self, func: str, funcargs):
         """res = egdst_call(model, sw, args) (egdstmodel.m:1181-1207)."""
         lib = self._capi()

@@ -154,6 +154,33 @@ int egdst_sim_moments_device(const egdst_desc *d, egdst_solution *s, int ivec0, 
  * it off. */
 int egdst_solution_set_choice_draws(egdst_solution *s, int on);
 
+/* EXTENSION, smoothing images only: log-likelihood of observed choices (and consumption) under the parameter vectors
+ * ivec0..ivec0+nvec-1 of s, one launch.  obs: [nobs x k] column-major, k = 4 or 5, rows as in egdst_call:
+ *   0 age (t0..T; period it = age - t0), 1 state ist (1-based), 2 cash-in-hand M at the start of the period (the cash
+ *   column of a simulation record), 3 observed decision id (1-based), 4 (k = 5) observed consumption c_obs, NaN: not
+ *   observed.
+ * Per row and vector:  ll = log P_d(M) + [log phi((c_obs - c_d(M)) / sigma_c) - log sigma_c]
+ * with the bracket only when k = 5, sigma_c > 0 and c_obs is not NaN; phi is the standard normal density.  P_d(M)
+ * and c_d(M) are exactly what the choice draws evaluate (the probability rule of the solve, egdst_solution_set_choice_draws:
+ * held at the bound above the grid, equal weights when every value is -inf, the credit-constrained branch below the
+ * first grid point), and log P_d = log e_d - log sum_d' e_d' of its weights.  A row contributes -inf when its decision
+ * is not available in (it, ist) or its weight underflows (a non-modal choice as sigma_eps -> 0): such a total is -inf.
+ * Parameter values: a batched solution uses the vectors it was solved with, a single model those of d (as the
+ * simulate entry points do).
+ *   loglik  [nvec] per-vector totals (overwritten).  rowll: [nvec][nobs] per-row values, or NULL.
+ * The totals are deterministic: the rows are summed in a fixed order over a block partition that depends on nobs only,
+ * so the same obs give the same bits whatever nvec, ivec0 or launch.  The host entry point checks every row and
+ * returns 2, naming the first malformed row, for an age, state or decision that is not an integer in range, or cash
+ * that is not finite or lies below a0.  Returns 2 as well for a solution without choice cells (sigma_eps = 0, or
+ * imported), an image with continuous states or without smoothing, k not 4 or 5, sigma_c < 0, or a vector range out of
+ * bounds (at most 65535 vectors).  The _device variant takes device pointers, is asynchronous on the library stream,
+ * checks no rows (a malformed row gets rowll = NaN, and its vector's total is NaN) and adds each vector's total to
+ * d_loglik (the caller zeroes it), so a rank can all-reduce the buffer right after. */
+int egdst_choice_loglik(const egdst_desc *d, egdst_solution *s, int ivec0, int nvec, const double *obs, int nobs, int k,
+                        double sigma_c, double *loglik, double *rowll);
+int egdst_choice_loglik_device(const egdst_desc *d, egdst_solution *s, int ivec0, int nvec, const double *d_obs, int nobs,
+                               int k, double sigma_c, double *d_loglik, double *d_rowll);
+
 /* ---- call -------------------------------------------------------------------------------- */
 /* sw: 1 utility, 2 marginal utility, 3 discount, 4 budget, 5 marginal budget, 6 value function;
  * args: [narg*k] column-major with k = 4,4,2,6,6,3 (egdst_call.c:45-58); res: [narg]. */
