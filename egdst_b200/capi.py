@@ -183,10 +183,12 @@ class Solution:
         return int(self.lib.L.egdst_solution_resends(self.handle))
 
 
-def observations_from_sims(model, sims, consumption: bool = True) -> np.ndarray:
+def observations_from_sims(model, sims, consumption: bool = True, start: bool = False):
     """The live records of a simulation ``sims`` [nsim, nt, nsimout] as observations for ``ModelLibrary.choice_loglik``:
     [nobs, 5] (or [nobs, 4] without ``consumption``) of age t0 + it, state ist + 1, cash, decision id + 1 and
-    consumption, agent-major.  Dead and skipped records (NaN) are dropped."""
+    consumption, agent-major.  Dead and skipped records (NaN) are dropped.  With ``start=True`` returns (obs, start):
+    the int32 offsets [nsim + 1] of each agent's rows for ``ModelLibrary.mixture_loglik`` (individual i = agent i; an
+    agent without a live record is an empty individual)."""
     s = np.asarray(sims, dtype=np.float64)
     cash, cons, dec, ist = s[:, :, 0], s[:, :, 1], s[:, :, 4], s[:, :, 5]
     live = ~(np.isnan(cash) | np.isnan(dec) | np.isnan(ist))
@@ -194,7 +196,10 @@ def observations_from_sims(model, sims, consumption: bool = True) -> np.ndarray:
     cols = [model.t0 + ti.astype(np.float64), ist[ai, ti] + 1.0, cash[ai, ti], dec[ai, ti] + 1.0]
     if consumption:
         cols.append(cons[ai, ti])
-    return np.column_stack(cols) if ai.size else np.zeros((0, len(cols)))
+    obs = np.column_stack(cols) if ai.size else np.zeros((0, len(cols)))
+    if not start:
+        return obs
+    return obs, np.concatenate([[0], np.cumsum(live.sum(axis=1))]).astype(np.int32)
 
 
 class ModelLibrary:
@@ -206,7 +211,8 @@ class ModelLibrary:
                "egdst_solution_export", "egdst_solution_choice_cell", "egdst_solution_set_choice_draws", "egdst_solution_status", "egdst_solution_nvec", "egdst_solution_units", "egdst_solution_resends", "egdst_solution_phase_ms", "egdst_test_envelope2",
                "egdst_free_solution", "egdst_solution_import", "egdst_simulate", "egdst_simulate_philox",
                "egdst_simulate_device", "egdst_sim_moments", "egdst_sim_moments_device", "egdst_choice_loglik",
-               "egdst_choice_loglik_device", "egdst_call", "egdst_shutdown"]
+               "egdst_choice_loglik_device", "egdst_mixture_loglik", "egdst_mixture_loglik_device", "egdst_call",
+               "egdst_shutdown"]
 
     def __init__(self, path: str):
         if not os.path.isfile(path):
@@ -248,6 +254,10 @@ class ModelLibrary:
         L.egdst_call.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, _dp, C.c_int, C.c_int, _dp]
         L.egdst_choice_loglik.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, _dp, C.c_int, C.c_int, C.c_double, _dp, _dp]
         L.egdst_choice_loglik_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, vp, C.c_int, C.c_int, C.c_double, vp, vp]
+        L.egdst_mixture_loglik.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, _dp, C.c_int, C.c_int, C.c_double, _ip,
+                                           C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, _dp, _dp, _dp]
+        L.egdst_mixture_loglik_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, vp, C.c_int, C.c_int, C.c_double,
+                                                  vp, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp, vp, vp]
         L.egdst_sim_moments.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, _dp, C.c_int, C.c_longlong, C.c_ulonglong, _dp]
         L.egdst_sim_moments_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, vp, C.c_int, C.c_longlong, C.c_ulonglong, vp]
         L.egdst_test_envelope2.argtypes = [C.POINTER(EgdstDesc), C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, C.c_int, C.c_double,
@@ -428,6 +438,62 @@ class ModelLibrary:
         nvec = sol.nvec - ivec0 if nvec is None else nvec
         rc = self.L.egdst_choice_loglik_device(C.byref(d.c), sol.handle, ivec0, nvec, C.c_void_p(d_obs or None), nobs, k,
                                                float(sigma_c), C.c_void_p(d_loglik or None), C.c_void_p(d_rowll or None))
+        if rc:
+            self._raise(rc)
+
+    def mixture_loglik(self, model, sol: Solution, obs, start, tvec, weights, sigma_c: float = 0.0, ivec0: int = 0,
+                       nvec: Optional[int] = None, individuals: bool = False, posterior: bool = False, desc: "Desc" = None):
+        """Smoothing mode only: finite-mixture log-likelihood over unobserved types.  ``obs`` [nobs, 4 or 5] as for
+        ``choice_loglik``, grouped by individual with offsets ``start`` [nind + 1] (``observations_from_sims(...,
+        start=True)``); ``tvec`` [nmix, ntypes] the vector of each type relative to ``ivec0``, ``weights`` [nmix,
+        ntypes] the type weights (normalised by the library).  A 1-D ``tvec`` / ``weights`` is one mixture.  Returns
+        the totals [nmix]; with ``individuals=True`` or ``posterior=True`` a tuple (totals, then indll [nvec, nind] and
+        mixll [nmix, nind] if ``individuals``, then post [nmix, ntypes, nind] if ``posterior``).  See
+        egdst_mixture_loglik in include/egdst_b200.h for the formula, the edge rules and the determinism contract."""
+        d = desc or Desc(model)
+        o = np.atleast_2d(np.asarray(obs, dtype=np.float64))
+        nobs, k = o.shape
+        of = _arr(o.ravel(order="F"))
+        st = np.ascontiguousarray(np.asarray(start), dtype=np.int32)
+        tv = np.ascontiguousarray(np.atleast_2d(np.asarray(tvec)), dtype=np.int32)
+        w = _arr(np.atleast_2d(np.asarray(weights, dtype=np.float64)))
+        if st.ndim != 1 or st.size < 1:
+            raise ValueError("start must be a 1-D array of nind + 1 offsets")
+        if tv.ndim != 2 or tv.shape != w.shape:
+            raise ValueError("tvec and weights must both be [nmix, ntypes]")
+        nind, (nmix, ntypes) = st.size - 1, tv.shape
+        nvec = sol.nvec - ivec0 if nvec is None else nvec
+        tot = np.zeros(max(nmix, 1), dtype=np.float64)
+        indll = np.empty(max(nvec, 1) * nind, dtype=np.float64) if individuals else None
+        mixll = np.empty(max(nmix, 1) * nind, dtype=np.float64) if individuals else None
+        post = np.empty(max(nmix * ntypes, 1) * nind, dtype=np.float64) if posterior else None
+        rc = self.L.egdst_mixture_loglik(C.byref(d.c), sol.handle, ivec0, nvec, _ptr(of), nobs, k, float(sigma_c),
+                                         st.ctypes.data_as(_ip), nind, ntypes, nmix, tv.ctypes.data_as(_ip), _ptr(w),
+                                         _ptr(tot), _ptr(indll), _ptr(mixll), _ptr(post))
+        if rc:
+            self._raise(rc)
+        out = (tot,)
+        if individuals:
+            out += (indll.reshape(nvec, nind), mixll.reshape(nmix, nind))
+        if posterior:
+            out += (post.reshape(nmix, ntypes, nind),)
+        return out if len(out) > 1 else tot
+
+    def mixture_loglik_device(self, model, sol: Solution, d_obs: int, nobs: int, k: int, d_start: int, nind: int,
+                              d_tvec: int, d_w: int, ntypes: int, nmix: int, d_loglik: int, sigma_c: float = 0.0,
+                              d_indll: int = 0, d_mixll: int = 0, d_post: int = 0, ivec0: int = 0,
+                              nvec: Optional[int] = None, desc: "Desc" = None):
+        """Asynchronous launch on the library stream; d_obs [k][nobs], d_start [nind + 1] (int32), d_tvec [nmix][ntypes]
+        (int32), d_w [nmix][ntypes], d_loglik [nmix] (accumulated into: the caller zeroes it) and the optional d_indll
+        [nvec][nind], d_mixll [nmix][nind] and d_post [nmix][ntypes][nind] are device addresses (ints).  Rows, offsets,
+        type vectors and weights are not checked."""
+        d = desc or Desc(model)
+        nvec = sol.nvec - ivec0 if nvec is None else nvec
+        vp = C.c_void_p
+        rc = self.L.egdst_mixture_loglik_device(C.byref(d.c), sol.handle, ivec0, nvec, vp(d_obs or None), nobs, k,
+                                                float(sigma_c), vp(d_start or None), nind, ntypes, nmix, vp(d_tvec or None),
+                                                vp(d_w or None), vp(d_loglik or None), vp(d_indll or None),
+                                                vp(d_mixll or None), vp(d_post or None))
         if rc:
             self._raise(rc)
 

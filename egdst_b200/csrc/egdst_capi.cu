@@ -166,8 +166,10 @@ struct egdst_solution {
     double *d_pack = 0; size_t pack_cap = 0;                // export / import staging
     EgdstCellHdr *d_hdr = 0; size_t hdr_cap = 0;            // simulator cell headers
     double *d_llpart = 0; size_t llpart_cap = 0;            // block partials of the choice log-likelihood
+    double *d_llrow = 0; size_t llrow_cap = 0;              // row values [nvec][nobs] of the mixture log-likelihood
+    double *d_llind = 0; size_t llind_cap = 0;              // per-individual values [nvec][nind] of the same
     // every device allocation, by the field that holds it
-    std::vector<void **> owned{(void **)&d_pack, (void **)&d_hdr, (void **)&d_llpart};
+    std::vector<void **> owned{(void **)&d_pack, (void **)&d_hdr, (void **)&d_llpart, (void **)&d_llrow, (void **)&d_llind};
     // state of the current owner (adopt)
     std::vector<int> h_mlen, h_thlen, h_status;
     bool sizes_valid = false;

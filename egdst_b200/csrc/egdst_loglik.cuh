@@ -8,6 +8,14 @@
 // reduction writes one partial per block, and egdst_k_choice_loglik_sum adds the partials of a vector in a fixed
 // order.  The block partition depends on nobs only, so the total of the same rows has the same bits for any nvec,
 // ivec0 or launch.
+//
+// Finite mixtures over unobserved types (egdst_mixture_loglik) take three passes: egdst_k_choice_loglik writes the
+// row values [nvec][nobs] to a scratch buffer (keeping its (row x vector) parallelism), egdst_k_indiv_loglik adds each
+// individual's rows in row order (one thread per (individual, vector)), and egdst_k_mixture_loglik combines the types
+// of each mixture per individual (one thread per (individual, mixture), blockIdx.y over the mixtures) and writes one
+// fixed-order partial per block, which egdst_k_choice_loglik_sum adds up.  The block partition depends on nind only.
+// So an individual's value under a vector does not depend on nvec, ivec0 or the launch, and a mixture's values and
+// total have the same bits whether it is evaluated alone or with other mixtures, in any ivec0 window holding its vectors.
 #pragma once
 
 #include "egdst_solver.cuh"
@@ -32,6 +40,16 @@ struct EgdstLlArgs {
     double param[EGDST_NPARAM_];
     double *rowll;       // [nvec][nobs] or null
     double *part;        // [nvec][gridDim.x] block partials
+};
+
+struct EgdstMixArgs {
+    const double *indll; // [nvec][nind] per-individual values
+    const int *tvec;     // [nmix][ntypes] vector of each type, relative to ivec0
+    const double *w;     // [nmix][ntypes] type weights (normalised here)
+    int nind, nvec, ntypes;
+    double *mixll;       // [nmix][nind] or null
+    double *post;        // [nmix][ntypes][nind] or null
+    double *part;        // [nmix][gridDim.x] block partials
 };
 
 #if EGDST_SMOOTHING && EGDST_NCONT == 0
@@ -98,5 +116,68 @@ __global__ void __launch_bounds__(32) egdst_k_choice_loglik_sum(const double *pa
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
     if (lane == 0) loglik[v] += s;
+}
+
+// indll[v][i] = the rows start[i]..start[i+1]-1 of rowll[v], added in row order (0 for an empty individual; NaN for
+// offsets that decrease or leave 0..nobs, which only the _device entry point lets through)
+__global__ void __launch_bounds__(EGDST_LL_BLOCK) egdst_k_indiv_loglik(const double *rowll, int nobs, const int *start,
+                                                                      int nind, double *indll) {
+    const int i = blockIdx.x * EGDST_LL_BLOCK + threadIdx.x, v = blockIdx.y;
+    if (i >= nind) return;
+    const int lo = start[i], hi = start[i + 1];
+    double s = 0.0;
+    if (lo < 0 || hi < lo || hi > nobs) {
+        s = EGDST_NAN;
+    } else {
+        const double *r = rowll + (size_t)v * nobs;
+        for (int j = lo; j < hi; j++) s += r[j];
+    }
+    indll[(size_t)v * nind + i] = s;
+}
+
+// mixture x = blockIdx.y, individual i: over the types k with w_k > 0 (ascending), a_k = log(w_k / sum w) +
+// indll[tvec_k][i], m = max a_k, mixll = m + log sum exp(a_k - m) (-inf when m = -inf), post_k = exp(a_k - m) / sum
+// (0 for zero weights, NaN when mixll is -inf or NaN).  A type vector outside 0..nvec-1 (the _device entry point does
+// not check them) gives NaN.
+__global__ void __launch_bounds__(EGDST_LL_BLOCK) egdst_k_mixture_loglik(EgdstMixArgs A) {
+    __shared__ double wsum[EGDST_LL_BLOCK / 32];
+    const int i = blockIdx.x * EGDST_LL_BLOCK + threadIdx.x, x = blockIdx.y, nk = A.ntypes;
+    const int *tv = A.tvec + (size_t)x * nk;
+    const double *w = A.w + (size_t)x * nk;
+    double ll = 0.0;
+    if (i < A.nind) {
+        double wt = 0.0;
+        for (int k = 0; k < nk; k++) wt += w[k];
+        auto a = [&](int k) {
+            const int t = tv[k];
+            return t >= 0 && t < A.nvec ? log(w[k] / wt) + A.indll[(size_t)t * A.nind + i] : EGDST_NAN;
+        };
+        double m = -EGDST_INF;  // NaN-propagating maximum
+        for (int k = 0; k < nk; k++) {
+            if (!(w[k] > 0.0)) continue;
+            const double ak = a(k);
+            if (ak > m || isnan(ak)) m = ak;
+        }
+        double s = 0.0;
+        for (int k = 0; k < nk; k++)
+            if (w[k] > 0.0) s += exp(a(k) - m);
+        const bool none = m == -EGDST_INF;
+        ll = none ? -EGDST_INF : m + log(s);
+        if (A.mixll) A.mixll[(size_t)x * A.nind + i] = ll;
+        if (A.post) {
+            double *p = A.post + (size_t)x * nk * A.nind + i;
+            for (int k = 0; k < nk; k++)
+                p[(size_t)k * A.nind] = !(w[k] > 0.0) ? 0.0 : none ? EGDST_NAN : exp(a(k) - m) / s;
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) ll += __shfl_down_sync(0xffffffffu, ll, o);
+    if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = ll;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double s = 0.0;
+        for (int k = 0; k < EGDST_LL_BLOCK / 32; k++) s += wsum[k];
+        A.part[(size_t)x * gridDim.x + blockIdx.x] = s;
+    }
 }
 #endif  // EGDST_SMOOTHING && EGDST_NCONT == 0

@@ -1,5 +1,6 @@
 """Multi-GPU sharding of the workloads that shard (SURVEY 8(e)): forward simulation over agents, batched solves over
-parameter vectors, and the choice log-likelihood over observations.  One process per GPU; ``torch.distributed`` is plumbing only -- the single
+parameter vectors, the choice log-likelihood over observations and the mixture log-likelihood over individuals.
+One process per GPU; ``torch.distributed`` is plumbing only -- the single
 collective on the data path is one all-reduce of the simulated-moment buffer (NCCL over NVLink on GPUs, gloo in
 the CPU tests of the host logic).  A single model's backward induction does not shard ("replicas only"): every
 rank solves it redundantly, bit-identically, which is cheaper than broadcasting the 16 MB arena every period.
@@ -123,3 +124,32 @@ def choice_loglik_sharded(lib, model, sol, obs: np.ndarray, sigma_c: float = 0.0
     tot = np.ascontiguousarray(loglik_fn(obs[lo:hi]), dtype=np.float64)
     all_reduce_moments(tot, group)
     return tot, (lo, hi)
+
+
+def mixture_loglik_sharded(lib, model, sol, obs: np.ndarray, start: np.ndarray, tvec, weights, sigma_c: float = 0.0,
+                           individuals: bool = False, posterior: bool = False, rank: Optional[int] = None,
+                           world: Optional[int] = None, fn: Optional[Callable] = None, group=None):
+    """Mixture log-likelihood (``ModelLibrary.mixture_loglik``) of the observations ``obs`` grouped by individual with
+    offsets ``start`` [nind + 1]: each rank evaluates its contiguous block of individuals [lo, hi), i.e. the rows
+    start[lo]..start[hi]-1 with the offsets rebased to 0, and one all-reduce of the [nmix] totals gives every rank the
+    sum.  Returns (totals [nmix], per-individual outputs of the rank's block (the tuple after the totals that
+    ``mixture_loglik`` returns with ``individuals`` / ``posterior``; empty without them), (lo, hi)).
+    ``fn(obs_block, start_block)`` (returning what ``mixture_loglik`` returns) replaces the CUDA call in the CPU tests."""
+    dist = _dist()
+    if world is None:
+        world = dist.get_world_size(group) if dist else 1
+    if rank is None:
+        rank = dist.get_rank(group) if dist else 0
+    obs = np.atleast_2d(np.asarray(obs, dtype=np.float64))
+    start = np.asarray(start, dtype=np.int64)
+    lo, hi = shard_range(start.size - 1, rank, world)
+    r0, r1 = int(start[lo]), int(start[hi])
+    if fn is None:
+        def fn(block, sblock):
+            return lib.mixture_loglik(model, sol, block, sblock, tvec, weights, sigma_c=sigma_c, individuals=individuals,
+                                      posterior=posterior)
+    res = fn(obs[r0:r1], (start[lo:hi + 1] - r0).astype(np.int32))
+    tot, parts = (res[0], tuple(res[1:])) if isinstance(res, tuple) else (res, ())
+    tot = np.ascontiguousarray(tot, dtype=np.float64)
+    all_reduce_moments(tot, group)
+    return tot, parts, (lo, hi)

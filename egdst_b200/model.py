@@ -466,6 +466,27 @@ class EgdstModel:
             raise RuntimeError("The model needs to be compiled and solved first!")
         return float(lib.choice_loglik(self, self._solution, obs, sigma_c=sigma_c)[0])
 
+    def mixture_loglik(self, obs, start, type_params, weights, sigma_c: float = 0.0, posterior: bool = False):
+        """Smoothing mode (``sigma_eps > 0``) only: log-likelihood of a finite mixture over unobserved types.  Solves the
+        parameter vectors ``type_params`` [ntypes, nparam] as one batch and evaluates the mixture with type weights
+        ``weights`` [ntypes] (normalised by the library) over the observations ``obs`` grouped by individual with
+        offsets ``start`` (``capi.observations_from_sims(..., start=True)``).  Returns the total, or (total, post
+        [ntypes, nind]) with ``posterior=True`` (egdst_mixture_loglik)."""
+        from . import capi
+        lib = self._capi()
+        tp = np.atleast_2d(np.asarray(type_params, dtype=np.float64))
+        sol = lib.solve_batch(self, tp)
+        if sol.warning:
+            import warnings
+            warnings.warn(sol.warning, capi.EgdstWarning)
+        # a one-vector solution takes its parameter values from the descriptor (as egdst_simulate does)
+        desc = capi.Desc(self)
+        desc.params[:] = tp[0]
+        ntypes = tp.shape[0]
+        res = lib.mixture_loglik(self, sol, obs, start, np.arange(ntypes), np.asarray(weights, dtype=np.float64).reshape(1, ntypes),
+                                 sigma_c=sigma_c, posterior=posterior, desc=desc)
+        return (float(res[0][0]), res[1][0]) if posterior else float(res[0])
+
     def call(self, func: str, funcargs):
         """res = egdst_call(model, sw, args) (egdstmodel.m:1181-1207)."""
         lib = self._capi()

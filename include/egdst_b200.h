@@ -181,6 +181,39 @@ int egdst_choice_loglik(const egdst_desc *d, egdst_solution *s, int ivec0, int n
 int egdst_choice_loglik_device(const egdst_desc *d, egdst_solution *s, int ivec0, int nvec, const double *d_obs, int nobs,
                                int k, double sigma_c, double *d_loglik, double *d_rowll);
 
+/* EXTENSION, smoothing images only: finite-mixture log-likelihood over unobserved types (Keane-Wolpin types), for
+ * nmix mixtures of ntypes types each, one launch.  obs and its rows are those of egdst_choice_loglik, grouped by
+ * individual: individual i owns rows start[i]..start[i+1]-1 (start [nind+1]: start[0] = 0, non-decreasing,
+ * start[nind] = nobs; empty individuals are allowed).  tvec [nmix][ntypes]: the vector of each type, relative to ivec0
+ * (0..nvec-1; a vector may serve several types and mixtures).  w [nmix][ntypes]: type weights, finite and >= 0 with a
+ * positive sum per mixture, normalised here (w~_k = w_k / sum_k w_k), so unnormalised or softmax weights can be passed.
+ *   indll [nvec][nind]:  L_i(v) = the sum of individual i's row values under vector v (0 for an empty individual).
+ *   mixll [nmix][nind]:  over the types k with w_k > 0 only, a_k = log w~_k + L_i(tvec_k), m = max_k a_k and
+ *                        mixll = m + log sum_k exp(a_k - m), summed in ascending k; -inf when m = -inf.
+ *   post [nmix][ntypes][nind]: the posterior type probabilities exp(a_k - m) / sum; 0 for zero-weight types, NaN for
+ *                        the other types where mixll is -inf (or NaN).
+ *   loglik [nmix]:       the sum of mixll over individuals (overwritten by the host entry point).
+ * Zero-weight types are skipped entirely: a -inf or NaN under them does not matter.  ntypes = 1 with any positive
+ * weight gives mixll == indll bit for bit.  indll, mixll and post are optional (NULL).
+ * Determinism: the rows of an individual are added in row order and mixtures are summed over a block partition that
+ * depends on nind only.  So an individual's indll under a vector does not depend on nvec, ivec0 or the launch, and a
+ * mixture's mixll, post and total have the same bits whether it is evaluated alone or with other mixtures, and in any
+ * ivec0 window holding its vectors.
+ * Returns 2 under the conditions of egdst_choice_loglik (the host entry point checks every row) and for nind < 0,
+ * ntypes < 1, nmix < 1 or nmix > 65535.  The host entry point also returns 2, naming the first offending index, for
+ * offsets that do not start at 0, decrease or do not end at nobs, a tvec entry outside 0..nvec-1, a weight that is
+ * negative or not finite, and a mixture whose weights sum to 0.  The _device variant takes device pointers (d_start
+ * and d_tvec int32), is asynchronous on the library stream, checks no rows, offsets, type vectors or weights (a
+ * malformed row makes its individual's indll NaN, and so the mixll and totals of every mixture that gives it positive
+ * weight; a malformed offset or type vector gives NaN likewise) and adds each mixture's total to d_loglik (the caller
+ * zeroes it).  It keeps the row values [nvec][nobs] (and indll when d_indll is NULL) in grow-only buffers of s. */
+int egdst_mixture_loglik(const egdst_desc *d, egdst_solution *s, int ivec0, int nvec, const double *obs, int nobs, int k,
+                         double sigma_c, const int *start, int nind, int ntypes, int nmix, const int *tvec, const double *w,
+                         double *loglik, double *indll, double *mixll, double *post);
+int egdst_mixture_loglik_device(const egdst_desc *d, egdst_solution *s, int ivec0, int nvec, const double *d_obs, int nobs,
+                                int k, double sigma_c, const int *d_start, int nind, int ntypes, int nmix, const int *d_tvec,
+                                const double *d_w, double *d_loglik, double *d_indll, double *d_mixll, double *d_post);
+
 /* ---- call -------------------------------------------------------------------------------- */
 /* sw: 1 utility, 2 marginal utility, 3 discount, 4 budget, 5 marginal budget, 6 value function;
  * args: [narg*k] column-major with k = 4,4,2,6,6,3 (egdst_call.c:45-58); res: [narg]. */
