@@ -202,6 +202,20 @@ def observations_from_sims(model, sims, consumption: bool = True, start: bool = 
     return obs, np.concatenate([[0], np.cumsum(live.sum(axis=1))]).astype(np.int32)
 
 
+def _mixture_args(obs, start, tvec, weights):
+    """The arrays of a mixture call: (obs column-major, nobs, k, start int32, tvec int32 [nmix, ntypes], weights)."""
+    o = np.atleast_2d(np.asarray(obs, dtype=np.float64))
+    nobs, k = o.shape
+    st = np.ascontiguousarray(np.asarray(start), dtype=np.int32)
+    tv = np.ascontiguousarray(np.atleast_2d(np.asarray(tvec)), dtype=np.int32)
+    w = _arr(np.atleast_2d(np.asarray(weights, dtype=np.float64)))
+    if st.ndim != 1 or st.size < 1:
+        raise ValueError("start must be a 1-D array of nind + 1 offsets")
+    if tv.ndim != 2 or tv.shape != w.shape:
+        raise ValueError("tvec and weights must both be [nmix, ntypes]")
+    return _arr(o.ravel(order="F")), nobs, k, st, tv, w
+
+
 class ModelLibrary:
     """One loaded model image (libegdst_b200_<key>.so)."""
 
@@ -211,8 +225,8 @@ class ModelLibrary:
                "egdst_solution_export", "egdst_solution_choice_cell", "egdst_solution_set_choice_draws", "egdst_solution_status", "egdst_solution_nvec", "egdst_solution_units", "egdst_solution_resends", "egdst_solution_phase_ms", "egdst_test_envelope2",
                "egdst_free_solution", "egdst_solution_import", "egdst_simulate", "egdst_simulate_philox",
                "egdst_simulate_device", "egdst_sim_moments", "egdst_sim_moments_device", "egdst_choice_loglik",
-               "egdst_choice_loglik_device", "egdst_mixture_loglik", "egdst_mixture_loglik_device", "egdst_call",
-               "egdst_shutdown"]
+               "egdst_choice_loglik_device", "egdst_mixture_loglik", "egdst_mixture_loglik_device",
+               "egdst_mixture_scores", "egdst_mixture_scores_device", "egdst_call", "egdst_shutdown"]
 
     def __init__(self, path: str):
         if not os.path.isfile(path):
@@ -258,6 +272,10 @@ class ModelLibrary:
                                            C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, _dp, _dp, _dp]
         L.egdst_mixture_loglik_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, vp, C.c_int, C.c_int, C.c_double,
                                                   vp, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp, vp, vp]
+        L.egdst_mixture_scores.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, _dp, C.c_int, C.c_int, C.c_double, _ip,
+                                           C.c_int, C.c_int, C.c_int, _ip, _dp, C.c_int, _ip, _ip, _dp, _dp, _dp, _dp, _dp]
+        L.egdst_mixture_scores_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, vp, C.c_int, C.c_int, C.c_double,
+                                                  vp, C.c_int, C.c_int, C.c_int, vp, vp, C.c_int, vp, vp, vp, vp, vp, vp, vp]
         L.egdst_sim_moments.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, _dp, C.c_int, C.c_longlong, C.c_ulonglong, _dp]
         L.egdst_sim_moments_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, vp, C.c_int, C.c_longlong, C.c_ulonglong, vp]
         L.egdst_test_envelope2.argtypes = [C.POINTER(EgdstDesc), C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, C.c_int, C.c_double,
@@ -451,16 +469,7 @@ class ModelLibrary:
         mixll [nmix, nind] if ``individuals``, then post [nmix, ntypes, nind] if ``posterior``).  See
         egdst_mixture_loglik in include/egdst_b200.h for the formula, the edge rules and the determinism contract."""
         d = desc or Desc(model)
-        o = np.atleast_2d(np.asarray(obs, dtype=np.float64))
-        nobs, k = o.shape
-        of = _arr(o.ravel(order="F"))
-        st = np.ascontiguousarray(np.asarray(start), dtype=np.int32)
-        tv = np.ascontiguousarray(np.atleast_2d(np.asarray(tvec)), dtype=np.int32)
-        w = _arr(np.atleast_2d(np.asarray(weights, dtype=np.float64)))
-        if st.ndim != 1 or st.size < 1:
-            raise ValueError("start must be a 1-D array of nind + 1 offsets")
-        if tv.ndim != 2 or tv.shape != w.shape:
-            raise ValueError("tvec and weights must both be [nmix, ntypes]")
+        of, nobs, k, st, tv, w = _mixture_args(obs, start, tvec, weights)
         nind, (nmix, ntypes) = st.size - 1, tv.shape
         nvec = sol.nvec - ivec0 if nvec is None else nvec
         tot = np.zeros(max(nmix, 1), dtype=np.float64)
@@ -494,6 +503,55 @@ class ModelLibrary:
                                                 float(sigma_c), vp(d_start or None), nind, ntypes, nmix, vp(d_tvec or None),
                                                 vp(d_w or None), vp(d_loglik or None), vp(d_indll or None),
                                                 vp(d_mixll or None), vp(d_post or None))
+        if rc:
+            self._raise(rc)
+
+    def mixture_scores(self, model, sol: Solution, obs, start, tvec, weights, mplus, mminus, hinv, sigma_c: float = 0.0,
+                       ivec0: int = 0, nvec: Optional[int] = None, scores: bool = False, desc: "Desc" = None):
+        """Smoothing mode only: central-difference scores of the mixtures ``tvec`` / ``weights`` (as for
+        ``mixture_loglik``).  Component p is the difference of mixtures ``mplus[p]`` and ``mminus[p]`` times ``hinv[p]``
+        (1 / the difference of the perturbed values solved); a one-type mixture of weight 1 is the plain likelihood.
+        Returns (totals [nmix], grad [npar], opg [npar, npar]), and scores [npar, nind] too with ``scores=True``.  See
+        egdst_mixture_scores in include/egdst_b200.h for the NaN rule and the determinism contract."""
+        d = desc or Desc(model)
+        of, nobs, k, st, tv, w = _mixture_args(obs, start, tvec, weights)
+        nind, (nmix, ntypes) = st.size - 1, tv.shape
+        mp = np.ascontiguousarray(np.atleast_1d(np.asarray(mplus)), dtype=np.int32)
+        mm = np.ascontiguousarray(np.atleast_1d(np.asarray(mminus)), dtype=np.int32)
+        h = _arr(np.atleast_1d(np.asarray(hinv, dtype=np.float64)))
+        if not (mp.ndim == 1 and mp.shape == mm.shape == h.shape):
+            raise ValueError("mplus, mminus and hinv must be 1-D of one length npar")
+        npar = mp.size
+        nvec = sol.nvec - ivec0 if nvec is None else nvec
+        tot = np.zeros(max(nmix, 1), dtype=np.float64)
+        grad = np.zeros(max(npar, 1), dtype=np.float64)
+        opg = np.zeros(max(npar * npar, 1), dtype=np.float64)
+        sc = np.empty(max(npar, 1) * nind, dtype=np.float64) if scores else None
+        rc = self.L.egdst_mixture_scores(C.byref(d.c), sol.handle, ivec0, nvec, _ptr(of), nobs, k, float(sigma_c),
+                                         st.ctypes.data_as(_ip), nind, ntypes, nmix, tv.ctypes.data_as(_ip), _ptr(w), npar,
+                                         mp.ctypes.data_as(_ip), mm.ctypes.data_as(_ip), _ptr(h), _ptr(tot), _ptr(grad),
+                                         _ptr(opg), _ptr(sc))
+        if rc:
+            self._raise(rc)
+        out = (tot, grad, opg.reshape(npar, npar))
+        return out + (sc.reshape(npar, nind),) if scores else out
+
+    def mixture_scores_device(self, model, sol: Solution, d_obs: int, nobs: int, k: int, d_start: int, nind: int,
+                              d_tvec: int, d_w: int, ntypes: int, nmix: int, npar: int, d_mplus: int, d_mminus: int,
+                              d_hinv: int, d_loglik: int, d_grad: int, d_opg: int, sigma_c: float = 0.0, d_scores: int = 0,
+                              ivec0: int = 0, nvec: Optional[int] = None, desc: "Desc" = None):
+        """Asynchronous launch on the library stream; the arguments of ``mixture_loglik_device`` plus d_mplus, d_mminus
+        [npar] (int32) and d_hinv [npar]; d_loglik [nmix], d_grad [npar] and d_opg [npar][npar] are accumulated into
+        (the caller zeroes them), d_scores [npar][nind] is optional.  Nothing is checked per row, offset, type, weight
+        or component: an out-of-range mixture index gives NaN scores."""
+        d = desc or Desc(model)
+        nvec = sol.nvec - ivec0 if nvec is None else nvec
+        vp = C.c_void_p
+        rc = self.L.egdst_mixture_scores_device(C.byref(d.c), sol.handle, ivec0, nvec, vp(d_obs or None), nobs, k,
+                                                float(sigma_c), vp(d_start or None), nind, ntypes, nmix, vp(d_tvec or None),
+                                                vp(d_w or None), npar, vp(d_mplus or None), vp(d_mminus or None),
+                                                vp(d_hinv or None), vp(d_loglik or None), vp(d_grad or None),
+                                                vp(d_opg or None), vp(d_scores or None))
         if rc:
             self._raise(rc)
 

@@ -168,8 +168,10 @@ struct egdst_solution {
     double *d_llpart = 0; size_t llpart_cap = 0;            // block partials of the choice log-likelihood
     double *d_llrow = 0; size_t llrow_cap = 0;              // row values [nvec][nobs] of the mixture log-likelihood
     double *d_llind = 0; size_t llind_cap = 0;              // per-individual values [nvec][nind] of the same
+    double *d_llmix = 0; size_t llmix_cap = 0;              // per-individual mixture values [nmix][nind] of the scores
     // every device allocation, by the field that holds it
-    std::vector<void **> owned{(void **)&d_pack, (void **)&d_hdr, (void **)&d_llpart, (void **)&d_llrow, (void **)&d_llind};
+    std::vector<void **> owned{(void **)&d_pack, (void **)&d_hdr, (void **)&d_llpart, (void **)&d_llrow, (void **)&d_llind,
+                               (void **)&d_llmix};
     // state of the current owner (adopt)
     std::vector<int> h_mlen, h_thlen, h_status;
     bool sizes_valid = false;

@@ -16,6 +16,14 @@
 // fixed-order partial per block, which egdst_k_choice_loglik_sum adds up.  The block partition depends on nind only.
 // So an individual's value under a vector does not depend on nvec, ivec0 or the launch, and a mixture's values and
 // total have the same bits whether it is evaluated alone or with other mixtures, in any ivec0 window holding its vectors.
+//
+// Central-difference scores (egdst_mixture_scores) add one pass after those three: egdst_k_mixture_scores takes a fixed
+// chunk of EGDST_SC_CHUNK individuals per block (a partition that depends on nind only), computes the chunk's
+// s_ip = (mixll[mplus_p][i] - mixll[mminus_p][i]) * hinv_p into shared memory, and then one thread per entry of the
+// list grad[0..P-1], opg[p][q] (p <= q) adds the chunk's terms in individual order and writes one partial per
+// (entry, block); an off-diagonal partial goes to both opg[p][q] and opg[q][p].  egdst_k_choice_loglik_sum adds each
+// entry's partials in a fixed order.  So grad[p], opg[p][q] and the scores depend only on the rows and on the mixtures
+// and factors of components p and q: not on npar, the other components or their order, nvec, ivec0 or the launch.
 #pragma once
 
 #include "egdst_solver.cuh"
@@ -31,6 +39,16 @@
 #ifndef EGDST_LL_MINBLOCKS
 #define EGDST_LL_MINBLOCKS 3
 #endif
+// egdst_k_mixture_scores: individuals per block (fewer on the emulator, so that its tests cross block boundaries),
+// threads per block, and the most score components per launch (shared memory holds [EGDST_SC_MAXPAR][chunk])
+#ifdef EGDST_HOSTEMU
+#define EGDST_SC_CHUNK 16
+#define EGDST_SC_BLOCK 32
+#else
+#define EGDST_SC_CHUNK 64
+#define EGDST_SC_BLOCK 128
+#endif
+#define EGDST_SC_MAXPAR 32
 
 struct EgdstLlArgs {
     const double *obs;   // [k][nobs]: age, state (1-based), cash, decision (1-based)[, consumption]
@@ -50,6 +68,16 @@ struct EgdstMixArgs {
     double *mixll;       // [nmix][nind] or null
     double *post;        // [nmix][ntypes][nind] or null
     double *part;        // [nmix][gridDim.x] block partials
+};
+
+struct EgdstScoreArgs {
+    const double *mixll; // [nmix][nind] per-individual mixture values
+    const int *mplus;    // [npar] mixture of the upper member of each difference
+    const int *mminus;   // [npar] mixture of the lower member
+    const double *hinv;  // [npar] 1 / (theta_plus - theta_minus)
+    int nind, nmix, npar;
+    double *scores;      // [npar][nind] or null
+    double *part;        // [npar + npar * npar][gridDim.x] block partials: grad, then opg row-major
 };
 
 #if EGDST_SMOOTHING && EGDST_NCONT == 0
@@ -178,6 +206,45 @@ __global__ void __launch_bounds__(EGDST_LL_BLOCK) egdst_k_mixture_loglik(EgdstMi
         double s = 0.0;
         for (int k = 0; k < EGDST_LL_BLOCK / 32; k++) s += wsum[k];
         A.part[(size_t)x * gridDim.x + blockIdx.x] = s;
+    }
+}
+
+// individuals blockIdx.x * EGDST_SC_CHUNK.. : s_ip = (mixll[mplus_p][i] - mixll[mminus_p][i]) * hinv_p (NaN for a
+// mixture index outside 0..nmix-1, which only the _device entry point lets through), then one partial per block of
+// each entry: grad[p] = sum s_ip and opg[p][q] = sum s_ip s_iq, added in individual order
+__global__ void __launch_bounds__(EGDST_SC_BLOCK) egdst_k_mixture_scores(EgdstScoreArgs A) {
+    constexpr int LD = EGDST_SC_CHUNK + 1;  // padded row: the entries' threads read different rows at one column
+    __shared__ double sc[EGDST_SC_MAXPAR * LD];
+    const int i0 = blockIdx.x * EGDST_SC_CHUNK, np = A.npar;
+    const int n = A.nind - i0 < EGDST_SC_CHUNK ? A.nind - i0 : EGDST_SC_CHUNK;
+    for (int e = threadIdx.x; e < np * EGDST_SC_CHUNK; e += EGDST_SC_BLOCK) {
+        const int p = e / EGDST_SC_CHUNK, j = e % EGDST_SC_CHUNK, i = i0 + j;
+        if (j >= n) continue;
+        const int a = A.mplus[p], b = A.mminus[p];
+        const double s = a >= 0 && a < A.nmix && b >= 0 && b < A.nmix
+                             ? (A.mixll[(size_t)a * A.nind + i] - A.mixll[(size_t)b * A.nind + i]) * A.hinv[p]
+                             : EGDST_NAN;
+        sc[p * LD + j] = s;
+        if (A.scores) A.scores[(size_t)p * A.nind + i] = s;
+    }
+    __syncthreads();
+    const size_t nb = gridDim.x;
+    for (int e = threadIdx.x; e < np + np * (np + 1) / 2; e += EGDST_SC_BLOCK) {
+        if (e < np) {
+            const double *x = sc + e * LD;
+            double s = 0.0;
+            for (int j = 0; j < n; j++) s += x[j];
+            A.part[e * nb + blockIdx.x] = s;
+        } else {
+            int p = 0, r = e - np;  // the upper triangle row by row: (0,0), (0,1), .., (0,P-1), (1,1), ..
+            while (r >= np - p) r -= np - p++;
+            const int q = p + r;
+            const double *x = sc + p * LD, *y = sc + q * LD;
+            double s = 0.0;
+            for (int j = 0; j < n; j++) s += x[j] * y[j];
+            A.part[(np + p * np + q) * nb + blockIdx.x] = s;
+            A.part[(np + q * np + p) * nb + blockIdx.x] = s;
+        }
     }
 }
 #endif  // EGDST_SMOOTHING && EGDST_NCONT == 0

@@ -1,5 +1,6 @@
 """Multi-GPU sharding of the workloads that shard (SURVEY 8(e)): forward simulation over agents, batched solves over
-parameter vectors, the choice log-likelihood over observations and the mixture log-likelihood over individuals.
+parameter vectors, the choice log-likelihood over observations, and the mixture log-likelihood and its scores over
+individuals.
 One process per GPU; ``torch.distributed`` is plumbing only -- the single
 collective on the data path is one all-reduce of the simulated-moment buffer (NCCL over NVLink on GPUs, gloo in
 the CPU tests of the host logic).  A single model's backward induction does not shard ("replicas only"): every
@@ -153,3 +154,30 @@ def mixture_loglik_sharded(lib, model, sol, obs: np.ndarray, start: np.ndarray, 
     tot = np.ascontiguousarray(tot, dtype=np.float64)
     all_reduce_moments(tot, group)
     return tot, parts, (lo, hi)
+
+
+def mixture_scores_sharded(lib, model, sol, obs: np.ndarray, start: np.ndarray, tvec, weights, mplus, mminus, hinv,
+                           sigma_c: float = 0.0, rank: Optional[int] = None, world: Optional[int] = None,
+                           fn: Optional[Callable] = None, group=None):
+    """Mixture scores (``ModelLibrary.mixture_scores``) over individuals sharded as in ``mixture_loglik_sharded``: each
+    rank evaluates its contiguous block of individuals with the offsets rebased to 0, and its totals [nmix], grad
+    [npar] and opg [npar * npar] are concatenated and all-reduced once (the OPG is a sum over individuals).  Returns
+    (totals [nmix], grad [npar], opg [npar, npar], (lo, hi)).  ``fn(obs_block, start_block)`` (returning (totals,
+    grad, opg)) replaces the CUDA call in the CPU tests."""
+    dist = _dist()
+    if world is None:
+        world = dist.get_world_size(group) if dist else 1
+    if rank is None:
+        rank = dist.get_rank(group) if dist else 0
+    obs = np.atleast_2d(np.asarray(obs, dtype=np.float64))
+    start = np.asarray(start, dtype=np.int64)
+    lo, hi = shard_range(start.size - 1, rank, world)
+    r0, r1 = int(start[lo]), int(start[hi])
+    if fn is None:
+        def fn(block, sblock):
+            return lib.mixture_scores(model, sol, block, sblock, tvec, weights, mplus, mminus, hinv, sigma_c=sigma_c)
+    tot, grad, opg = fn(obs[r0:r1], (start[lo:hi + 1] - r0).astype(np.int32))
+    nmix, npar = np.size(tot), np.size(grad)
+    buf = np.ascontiguousarray(np.concatenate([np.ravel(tot), np.ravel(grad), np.ravel(opg)]), dtype=np.float64)
+    all_reduce_moments(buf, group)
+    return buf[:nmix], buf[nmix:nmix + npar], buf[nmix + npar:].reshape(npar, npar), (lo, hi)

@@ -214,6 +214,40 @@ int egdst_mixture_loglik_device(const egdst_desc *d, egdst_solution *s, int ivec
                                 int k, double sigma_c, const int *d_start, int nind, int ntypes, int nmix, const int *d_tvec,
                                 const double *d_w, double *d_loglik, double *d_indll, double *d_mixll, double *d_post);
 
+/* EXTENSION, smoothing images only: central-difference scores of mixture log-likelihoods, with their sum (the
+ * gradient) and the outer-product-of-gradients (OPG) matrix, one launch after the passes of egdst_mixture_loglik.  obs,
+ * start, tvec and w are those of egdst_mixture_loglik.  A plain one-type likelihood is the mixture with ntypes = 1 and
+ * weight 1 (mixll == indll bit for bit).  Component p (npar of them, 1..32) is the pair of mixtures mplus[p], mminus[p]
+ * (0..nmix-1) and the factor hinv[p] = 1 / (theta_plus - theta_minus), computed by the caller from the perturbed values
+ * actually solved (a forward difference is the pair (perturbed, centre)).  Parameters that enter the solve are
+ * perturbed as vectors of the batch, type weights as mixtures over the same vectors.  Per individual i:
+ *   s_ip = (mixll[mplus[p]][i] - mixll[mminus[p]][i]) * hinv[p]
+ *   grad [npar]:         sum_i s_ip.
+ *   opg [npar][npar]:    sum_i s_ip s_iq, both triangles from one sum (opg[q][p] has the bits of opg[p][q]).
+ *   loglik [nmix]:       the mixture totals of egdst_mixture_loglik.
+ *   scores [npar][nind]: s_ip, or NULL.
+ * An individual whose mixll is -inf under both members of a pair gets a NaN score, and that NaN propagates into grad
+ * and opg (-inf under one member only gives an infinite score); neither is masked.
+ * Determinism: the individuals are summed in index order within blocks of a partition that depends on nind only, and
+ * the block partials in a fixed order.  So grad[p], opg[p][q] and the scores of p depend only on the rows and on the
+ * mixtures and hinv of components p and q: not on npar, on which other components are requested or in what order, on
+ * nvec or ivec0, or on the launch.
+ * Returns 2 under the conditions of egdst_mixture_loglik (the host entry point checks every row, offset, type vector
+ * and weight) and for npar < 1 or npar > 32.  The host entry point also returns 2, naming the first offending
+ * component, for an mplus or mminus entry outside 0..nmix-1 and a hinv that is 0 or not finite; it overwrites loglik,
+ * grad and opg.  The _device variant takes device pointers (d_start, d_tvec, d_mplus and d_mminus int32), is
+ * asynchronous on the library stream, checks no data (an out-of-range mixture index gives NaN scores, never an
+ * out-of-bounds read) and adds into d_loglik, d_grad and d_opg (the caller zeroes them).  It keeps the row, individual
+ * and mixture values in grow-only buffers of s. */
+int egdst_mixture_scores(const egdst_desc *d, egdst_solution *s, int ivec0, int nvec, const double *obs, int nobs, int k,
+                         double sigma_c, const int *start, int nind, int ntypes, int nmix, const int *tvec, const double *w,
+                         int npar, const int *mplus, const int *mminus, const double *hinv, double *loglik, double *grad,
+                         double *opg, double *scores);
+int egdst_mixture_scores_device(const egdst_desc *d, egdst_solution *s, int ivec0, int nvec, const double *d_obs, int nobs,
+                                int k, double sigma_c, const int *d_start, int nind, int ntypes, int nmix, const int *d_tvec,
+                                const double *d_w, int npar, const int *d_mplus, const int *d_mminus, const double *d_hinv,
+                                double *d_loglik, double *d_grad, double *d_opg, double *d_scores);
+
 /* ---- call -------------------------------------------------------------------------------- */
 /* sw: 1 utility, 2 marginal utility, 3 discount, 4 budget, 5 marginal budget, 6 value function;
  * args: [narg*k] column-major with k = 4,4,2,6,6,3 (egdst_call.c:45-58); res: [narg]. */
