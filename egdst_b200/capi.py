@@ -185,8 +185,9 @@ class Solution:
 
 def observations_from_sims(model, sims, consumption: bool = True, start: bool = False):
     """The live records of a simulation ``sims`` [nsim, nt, nsimout] as observations for ``ModelLibrary.choice_loglik``:
-    [nobs, 5] (or [nobs, 4] without ``consumption``) of age t0 + it, state ist + 1, cash, decision id + 1 and
-    consumption, agent-major.  Dead and skipped records (NaN) are dropped.  With ``start=True`` returns (obs, start):
+    [nobs, 5 + K] (or [nobs, 4 + K] without ``consumption``) of age t0 + it, state ist + 1, cash, decision id + 1, the
+    exact values x_1..x_K of the model's K continuous states (record columns 11 + j, in state order) and consumption,
+    agent-major.  Dead and skipped records (NaN) are dropped.  With ``start=True`` returns (obs, start):
     the int32 offsets [nsim + 1] of each agent's rows for ``ModelLibrary.mixture_loglik`` (individual i = agent i; an
     agent without a live record is an empty individual)."""
     s = np.asarray(sims, dtype=np.float64)
@@ -194,6 +195,7 @@ def observations_from_sims(model, sims, consumption: bool = True, start: bool = 
     live = ~(np.isnan(cash) | np.isnan(dec) | np.isnan(ist))
     ai, ti = np.nonzero(live)
     cols = [model.t0 + ti.astype(np.float64), ist[ai, ti] + 1.0, cash[ai, ti], dec[ai, ti] + 1.0]
+    cols += [s[ai, ti, 11 + j] for j, v in enumerate(model.s) if v["continuous"]]
     if consumption:
         cols.append(cons[ai, ti])
     obs = np.column_stack(cols) if ai.size else np.zeros((0, len(cols)))
@@ -432,8 +434,8 @@ class ModelLibrary:
 
     def choice_loglik(self, model, sol: Solution, obs, sigma_c: float = 0.0, ivec0: int = 0, nvec: Optional[int] = None,
                       rows: bool = False):
-        """Smoothing mode only: log-likelihood of the observations ``obs`` [nobs, 4 or 5] (age, 1-based state, cash,
-        1-based decision[, consumption]; see ``observations_from_sims``) under parameter vectors ivec0.. of ``sol``.
+        """Smoothing mode only: log-likelihood of the observations ``obs`` [nobs, 4 + K or 5 + K] (age, 1-based state,
+        cash, 1-based decision, the values of the K continuous states[, consumption]; see ``observations_from_sims``) under parameter vectors ivec0.. of ``sol``.
         Returns the totals [nvec], and with ``rows=True`` also the per-row values [nvec, nobs].  See
         egdst_choice_loglik in include/egdst_b200.h for the formula and the -inf / NaN rules."""
         d = Desc(model)
@@ -461,7 +463,7 @@ class ModelLibrary:
 
     def mixture_loglik(self, model, sol: Solution, obs, start, tvec, weights, sigma_c: float = 0.0, ivec0: int = 0,
                        nvec: Optional[int] = None, individuals: bool = False, posterior: bool = False, desc: "Desc" = None):
-        """Smoothing mode only: finite-mixture log-likelihood over unobserved types.  ``obs`` [nobs, 4 or 5] as for
+        """Smoothing mode only: finite-mixture log-likelihood over unobserved types.  ``obs`` [nobs, 4 + K or 5 + K] as for
         ``choice_loglik``, grouped by individual with offsets ``start`` [nind + 1] (``observations_from_sims(...,
         start=True)``); ``tvec`` [nmix, ntypes] the vector of each type relative to ``ivec0``, ``weights`` [nmix,
         ntypes] the type weights (normalised by the library).  A 1-D ``tvec`` / ``weights`` is one mixture.  Returns

@@ -459,6 +459,14 @@ static int launch_solve(egdst_solution *s, cudaStream_t st) {
     P.self = s->d_self;
     P.phase_ns = g_prof_on ? s->d_phase : 0;  // measurement aid: in-kernel phase timers while profiling is enabled
     if (EGDST_SMOOTHING) CK(cudaMemcpyAsync(s->d_self, &P, sizeof(EgdstDev), cudaMemcpyHostToDevice, st));  // read by egdst_smooth_node
+#ifndef EGDST_HOSTEMU
+    // the dynamic shared memory limit is a property of the kernel, not of the solution object: another object's plan
+    // (a model with fewer quadrature nodes or states) may have lowered it since this one was planned or taken from
+    // the cache, and a launch above the limit is refused
+    const void *kern = pl.scope == SCOPE_WARP ? (const void *)egdst_k_solve_warps
+                       : pl.scope == SCOPE_CTA ? (const void *)egdst_k_solve_cta : (const void *)egdst_k_solve_grid;
+    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+#endif
     switch (pl.scope) {
     case SCOPE_WARP: KLAUNCH(KC_SOLVE, egdst_k_solve_warps, dim3(pl.ctas), dim3(32, pl.warps), pl.smem, st, P, pl.syncOff, pl.groupBytes); break;
     case SCOPE_CTA: KLAUNCH(KC_SOLVE, egdst_k_solve_cta, dim3(pl.ctas), dim3(pl.block), pl.smem, st, P, pl.syncOff); break;

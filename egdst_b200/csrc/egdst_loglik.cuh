@@ -51,7 +51,7 @@
 #define EGDST_SC_MAXPAR 32
 
 struct EgdstLlArgs {
-    const double *obs;   // [k][nobs]: age, state (1-based), cash, decision (1-based)[, consumption]
+    const double *obs;   // [k][nobs]: age, state (1-based), cash, decision (1-based), x_1..x_NCONT[, consumption]
     int nobs, k, ivec0;
     int prm_on;          // 1: the parameter values are param (a single model: this call's); 0: the solve's (P.bparams)
     double sigma_c;      // consumption measurement error (0: no consumption term)
@@ -80,8 +80,10 @@ struct EgdstScoreArgs {
     double *part;        // [npar + npar * npar][gridDim.x] block partials: grad, then opg row-major
 };
 
-#if EGDST_SMOOTHING && EGDST_NCONT == 0
-// log P_d(M) (+ the consumption term) of row i under the parameter values in cx; NaN for a malformed row
+#if EGDST_SMOOTHING
+// log P_d(M) (+ the consumption term) of row i under the parameter values in cx; NaN for a malformed row.  With
+// continuous states, P_d is that of the mixed choice values at the row's exact state x_1..x_NCONT (columns 4..) and the
+// consumption term is centred on the consumption a choice draw records, min(c_d, M - a0) (egdst_choice_values_cont)
 EGDST_DEV double egdst_choice_loglik_row(const EgdstDev &P, const egdst_ctx &cx, int ivec, const EgdstLlArgs &A, int i) {
     const size_t n = (size_t)A.nobs;  // column offsets in size_t: k * nobs exceeds INT_MAX for panels of 430 M rows
     const double age = A.obs[i], sti = A.obs[n + i], cash = A.obs[2 * n + i], dob = A.obs[3 * n + i];
@@ -95,15 +97,31 @@ EGDST_DEV double egdst_choice_loglik_row(const EgdstDev &P, const egdst_ctx &cx,
     egdst_fill_decision(&cx, &x);
     const int id = x.id;
     EgdstChoiceVals cv;
+#if EGDST_NCONT > 0
+#pragma unroll
+    for (int k = 0; k < EGDST_NCONT; k++) {
+        const double xk = A.obs[(4 + k) * n + i];
+        if (!(fabs(xk) < EGDST_INF)) return EGDST_NAN;
+        x.st[egdst_contvar[k]] = xk;
+    }
+    int istrec;
+    if (!egdst_choice_values_cont(P, &cx, ivec, x, cv, istrec)) return EGDST_NAN;
+#else
     egdst_choice_values(P, &cx, egdst_cell(P, ivec, x.it, x.ist), x, cv);
+#endif
     double ssum, wmax, ed = 0.0;
     egdst_choice_weights(cx.nd, cv, P.sigmaEps, ssum, wmax, [&](int d, double e) { if (d == id) ed = e; });
     // a decision without weight (not available, or exp underflows) has probability 0
     double ll = ed > 0.0 ? log(ed) - log(ssum) : -EGDST_INF;
-    if (A.k == 5 && A.sigma_c > 0.0) {
-        const double cobs = A.obs[4 * n + i];
+    if (A.k == 5 + EGDST_NCONT && A.sigma_c > 0.0) {
+        const double cobs = A.obs[(4 + EGDST_NCONT) * n + i];
         if (!isnan(cobs)) {
-            const double z = (cobs - cv.c[id]) / A.sigma_c;
+#if EGDST_NCONT > 0
+            const double cd = MIN(cv.c[id], cash - cx.a0);  // the consumption a choice draw records
+#else
+            const double cd = cv.c[id];
+#endif
+            const double z = (cobs - cd) / A.sigma_c;
             ll += -0.5 * z * z - 0.91893853320467274178 - log(A.sigma_c);  // log phi(z) - log sigma_c
         }
     }
@@ -118,6 +136,9 @@ __global__ void __launch_bounds__(EGDST_LL_BLOCK, EGDST_LL_MINBLOCKS) egdst_k_ch
     if (i < A.nobs) {
         egdst_ctx cx; egdst_load_ctx(P, ivec, cx);
         cx.status = 0;
+#if EGDST_NCONT > 0
+        cx.byval = 1;  // model functions read the row's exact continuous state from x.st
+#endif
         if (A.prm_on) {
 #pragma unroll
             for (int j = 0; j < EGDST_NPARAM; j++) cx.param[j] = A.param[j];
@@ -247,4 +268,4 @@ __global__ void __launch_bounds__(EGDST_SC_BLOCK) egdst_k_mixture_scores(EgdstSc
         }
     }
 }
-#endif  // EGDST_SMOOTHING && EGDST_NCONT == 0
+#endif  // EGDST_SMOOTHING

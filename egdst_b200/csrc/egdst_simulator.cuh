@@ -241,7 +241,7 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
     constexpr int WPB = (PB == 2 ? EGDST_SIM_WIDE : EGDST_SIM_BLOCK) / 32;
     constexpr bool SIMS = (OUT & 1) != 0, MOM = (OUT & 2) != 0, DRAW = (OUT & 4) != 0;
     constexpr bool PIPE = PB == 2 && EGDST_NCONT == 0;  // pipelined period order
-    static_assert(!DRAW || (PB == 1 && !HDR && EGDST_SMOOTHING && EGDST_NCONT == 0), "choice draws: plain period order, choice cells in global memory");
+    static_assert(!DRAW || (PB == 1 && !HDR && EGDST_SMOOTHING), "choice draws: plain period order, choice cells in global memory");
     // position of column j in the row of the agent staged by lane l: rotated rows spread a column over the banks
 #define EGDST_TILE_POS(l, j) ((l) * TS + (SWZ ? (((j) + (((l) >> 2) & 3) >= W) ? (j) + (((l) >> 2) & 3) - W : (j) + (((l) >> 2) & 3)) : (j)))
     // blockIdx.y walks the parameter vectors of a batched sweep: same agents and shocks under every vector,
@@ -361,6 +361,37 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
                     eqs_sim(&cx, &cur, (const PeriodVars *)0, eqs);
                 }
 #if EGDST_NCONT > 0
+#if EGDST_SMOOTHING
+                if (DRAW) {
+                    if (state == 0) {
+                        // choice draw at the exact continuous state: P_d of the mixed choice values of the kept corner
+                        // cells (egdst_choice_values_cont), d drawn as in the all-discrete branch below; the record is d's
+                        // mixed consumption (clamped as in the modal branch), its mixed value, and the corner at which
+                        // the cumulated normalised weight passes one half
+                        EgdstChoiceVals cv;
+                        int istrec;
+                        int dr = -1;
+                        double pe[EGDST_SMOOTH_MAXND];
+                        if (egdst_choice_values_cont(P, &cx, ivec, cur, cv, istrec)) {
+                            double ssum, wmax;
+                            for (int d = 0; d < cx.nd; d++) pe[d] = 0.0;
+                            egdst_choice_weights(cx.nd, cv, P.sigmaEps, ssum, wmax, [&](int d, double e) { pe[d] = e; });
+                            const double u = PHILOX ? egdst_u01(cr3) : rs[(size_t)3 * (nt - 1) + it];
+                            dr = egdst_draw_decision(cx.nd, cv, pe, ssum, u);
+                        }
+                        if (dr < 0) { state = 1; }  // no decision available at every kept corner
+                        else {
+                            c = MIN(cv.c[dr], cur.cash - cx.a0);
+                            cur.savings = cur.cash - c;
+                            vf = cv.v[dr];
+                            cur.ist = istrec;
+                            cur.id = dr;
+                            egdst_fill_decision(&cx, &cur);
+                            uu = utility(&cx, &cur, c); bb = discount(&cx, &cur);
+                        }
+                    }
+                } else
+#endif
                 if (state == 0) {
                     // Continuous states (egdst_simulator.c:309-365): consumption and value are the multilinear mix of the
                     // policies of the 2^NCONT surrounding grid cells (weights <= 0 are skipped, as there); the recorded
@@ -433,14 +464,7 @@ egdst_k_simulate(EgdstDev P, EgdstSimArgs S, const EGDST_GRID_CONSTANT EgdstSimH
                         for (int d = 0; d < cx.nd; d++) pe[d] = 0.0;
                         egdst_choice_weights(cx.nd, cv, P.sigmaEps, ssum, wmax, [&](int d, double e) { pe[d] = e; });
                         const double u = PHILOX ? egdst_u01(cr3) : rs[(size_t)3 * (nt - 1) + it];
-                        int dr = -1;
-                        double cum = 0.0;
-                        for (int d = 0; d < cx.nd; d++) {
-                            if (!(cv.avail >> d & 1u)) continue;
-                            cum += pe[d] / ssum;
-                            dr = d;  // the last available decision if rounding keeps the sum below u
-                            if (cum >= u) break;
-                        }
+                        const int dr = egdst_draw_decision(cx.nd, cv, pe, ssum, u);
                         if (dr < 0) { state = 1; }  // no decision available in (it, ist)
                         else {
                             const int dcell = egdst_dcell(P, cell, dr);

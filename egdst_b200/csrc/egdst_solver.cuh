@@ -175,6 +175,9 @@ EGDST_DEV void egdst_choice_values(const EgdstDev &P, const egdst_ctx *cx, int c
         if (cash > t.Mlast) c1 = MAX(c1, t.Clast);
         cv.c[d1] = c1;
         x.id = d1;
+#if EGDST_NCONT > 0
+        egdst_fill_decision(cx, &x);  // read by the model functions when they take the state by value (cx->byval)
+#endif
         double v1;
         if (cash < t.M1 && t.evf > -EGDST_INF) {
             v1 = utility(cx, &x, cash - cx->a0) + discount(cx, &x) * t.evf;
@@ -223,6 +226,88 @@ EGDST_DEV bool egdst_choice_weights(int nd, const EgdstChoiceVals &cv, double si
     if (ssum > 0.0) return true;
     for (int d1 = 0; d1 < nd; d1++) if (cv.avail >> d1 & 1u) { ssum += 1.0; f(d1, 1.0); }
     return false;
+}
+
+#if EGDST_NCONT > 0
+// The choice values at the exact continuous state x.st (cx->byval = 1) of period x.it, discrete part of x.ist (its grid
+// part is ignored), cash x.cash.  The 2^NCONT grid cells around x are those of the simulator's modal continuous branch;
+// corners with weight <= 0 are skipped and the kept weights are renormalised to sum 1 (outside the grid: held at its
+// edge).  With the normalised weights w, c[d], v[d] and vl[d] are the w-mixes of egdst_choice_values at the kept
+// corners, avail the AND and above the OR over them, so egdst_choice_weights applies unchanged.  istrec: the corner at
+// which the cumulated weight passes 1/2.  False: no corner kept (x not finite).
+EGDST_DEV bool egdst_choice_values_cont(const EgdstDev &P, const egdst_ctx *cx, int ivec, PeriodVars x, EgdstChoiceVals &cv, int &istrec) {
+    int j1[EGDST_NCONT], stride[EGDST_NCONT];
+    double wlo[EGDST_NCONT], whi[EGDST_NCONT];
+    int base = x.ist;
+#pragma unroll
+    for (int k = 0; k < EGDST_NCONT; k++) {
+        const int j0 = egdst_contvar[k], n = (int)cx->stm[j0];
+        const double *g = egdst_contgrid(k);
+        const double xk = x.st[j0];
+        stride[k] = (int)cx->stm[cx->nnst + j0];
+        base -= ((x.ist / stride[k]) % n) * stride[k];
+        j1[k] = egdst_gridcell(xk, g, n);
+        wlo[k] = (g[j1[k] + 1] - xk) / (g[j1[k] + 1] - g[j1[k]]);
+        whi[k] = (xk - g[j1[k]]) / (g[j1[k] + 1] - g[j1[k]]);
+    }
+    auto corner = [&](int ii, int &ist) {
+        double wt = 1;
+        ist = base;
+#pragma unroll
+        for (int k = 0; k < EGDST_NCONT; k++) {
+            const int up = (ii >> k) & 1;
+            wt *= up ? whi[k] : wlo[k];
+            ist += stride[k] * (j1[k] + up);
+        }
+        return wt;
+    };
+    double wsum = 0.0;
+    for (int ii = 0; ii < (1 << EGDST_NCONT); ii++) {
+        int ist;
+        const double wt = corner(ii, ist);
+        if (wt > 0) wsum += wt;
+    }
+    cv.avail = ~0u; cv.above = false;
+    for (int d = 0; d < cx->nd; d++) { cv.c[d] = 0.0; cv.v[d] = 0.0; cv.vl[d] = 0.0; }
+    double rr = .5;
+    int istlast = -1;
+    istrec = -1;
+    for (int ii = 0; ii < (1 << EGDST_NCONT); ii++) {
+        int ist;
+        const double wt = corner(ii, ist);
+        if (!(wt > 0)) continue;
+        const double w = wt / wsum;
+        EgdstChoiceVals cc;
+        x.ist = ist;
+        egdst_choice_values(P, cx, egdst_cell(P, ivec, x.it, ist), x, cc);
+        cv.avail &= cc.avail;
+        cv.above = cv.above || cc.above;
+        for (int d = 0; d < cx->nd; d++) { cv.c[d] += w * cc.c[d]; cv.v[d] += w * cc.v[d]; cv.vl[d] += w * cc.vl[d]; }
+        rr -= w;
+        istlast = ist;
+        if (rr < 0 && istrec < 0) istrec = ist;
+    }
+    if (istlast < 0) return false;
+    if (istrec < 0) istrec = istlast;
+    cv.vmax = -EGDST_INF;
+    for (int d = 0; d < cx->nd; d++) if (cv.v[d] > cv.vmax) cv.vmax = cv.v[d];
+    return true;
+}
+#endif
+
+// The decision drawn with uniform u from the weights pe[d] / ssum (egdst_choice_weights) of cv: the first available
+// decision whose cumulative probability reaches u, or the last available one if rounding keeps the sum below u; -1 when
+// no decision is available.
+EGDST_DEV int egdst_draw_decision(int nd, const EgdstChoiceVals &cv, const double *pe, double ssum, double u) {
+    int dr = -1;
+    double cum = 0.0;
+    for (int d = 0; d < nd; d++) {
+        if (!(cv.avail >> d & 1u)) continue;
+        cum += pe[d] / ssum;
+        dr = d;
+        if (cum >= u) break;
+    }
+    return dr;
 }
 
 // Out of line, with scalar arguments and the kernel-argument block read from its copy in global memory (P.self): the

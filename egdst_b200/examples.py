@@ -334,8 +334,24 @@ def retirement_two_period(sigma_eps=0.5, ngridm=2000) -> EgdstModel:
     return m
 
 
+def humancapital_smooth(sigma_eps=0.2, **kw) -> EgdstModel:
+    """humancapital (one continuous state) with extreme-value taste shocks of scale ``sigma_eps`` on the labour-supply
+    choice: choice draws and the choice likelihood at the exact human capital z."""
+    m = humancapital(**kw)
+    m.sigma_eps = sigma_eps
+    return m
+
+
+def humancapital2_smooth(sigma_eps=0.2, **kw) -> EgdstModel:
+    """humancapital2 (two continuous states: four corner cells) with taste shocks of scale ``sigma_eps``."""
+    m = humancapital(health=True, **kw)
+    m.sigma_eps = sigma_eps
+    return m
+
+
 # images of the smoothing mode (compiled with EGDST_SMOOTHING, codegen.emit_devspec)
-SMOOTH = {"retirement2_smooth": retirement2_smooth, "retirement_two_period": retirement_two_period}
+SMOOTH = {"retirement2_smooth": retirement2_smooth, "retirement_two_period": retirement_two_period,
+          "humancapital_smooth": humancapital_smooth, "humancapital2_smooth": humancapital2_smooth}
 
 EXTRA = {"deaton_normal": deaton_normal, "deaton_meanstest": deaton_meanstest, "humancapital": humancapital, "humancapital2": humancapital2,
          "retirement_mortal": retirement_mortal, "retirement_jobloss": retirement_jobloss}

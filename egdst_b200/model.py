@@ -459,7 +459,7 @@ class EgdstModel:
         return self
 
     def loglik(self, obs, sigma_c: float = 0.0) -> float:
-        """Smoothing mode (``sigma_eps > 0``) only: log-likelihood of the observations ``obs`` [nobs, 4 or 5] under the
+        """Smoothing mode (``sigma_eps > 0``) only: log-likelihood of the observations ``obs`` [nobs, 4 + K or 5 + K] under the
         current solution (egdst_choice_loglik; ``capi.observations_from_sims`` builds ``obs`` from simulated records)."""
         lib = self._capi()
         if self._solution is None:

@@ -149,19 +149,28 @@ int egdst_sim_moments_device(const egdst_desc *d, egdst_solution *s, int ivec0, 
  *   randstream  slot 3*(nt-1)+it of the agent's 4*nt block (the transitions use slots 0..3*(nt-1)-1), shared by all
  *               agents with rndtype 1 as the other slots are;
  *   Philox      word 3 of the block of counter (agent, it), whose words 0-2 drive the transition into it.
- * Returns 2 when on != 0 for a solution without choice cells (sigma_eps = 0, or imported), or for a model image with
- * continuous states.  The setting belongs to the solution object: egdst_resolve keeps it, a new solve starts with
+ * With K continuous states (an image with EGDST_NCONT = K > 0) the probabilities are those of the mixed choice values
+ * at the agent's exact state x: the 2^K grid cells around x (the corners of the modal simulation), corners with weight
+ * <= 0 skipped and the kept weights w renormalised to sum 1 (so x outside the grid is held at its edge), and per
+ * decision c_d = sum w c_d^corner, v_d = sum w v_d^corner (-inf if -inf at any kept corner), available when available
+ * at every kept corner.  The record holds consumption min(c_d, M - a0), savings M - c, value v_d, decision d, the
+ * corner at which the cumulated weight passes 1/2 as state, and utility and discount of (c, d) at the exact state.
+ * Returns 2 when on != 0 for a solution without choice cells (sigma_eps = 0, or imported).  The setting belongs to the solution object: egdst_resolve keeps it, a new solve starts with
  * it off. */
 int egdst_solution_set_choice_draws(egdst_solution *s, int on);
 
 /* EXTENSION, smoothing images only: log-likelihood of observed choices (and consumption) under the parameter vectors
- * ivec0..ivec0+nvec-1 of s, one launch.  obs: [nobs x k] column-major, k = 4 or 5, rows as in egdst_call:
+ * ivec0..ivec0+nvec-1 of s, one launch.  obs: [nobs x k] column-major, k = 4 + K or 5 + K for an image with K
+ * continuous states (K = 0: 4 or 5), rows as in egdst_call:
  *   0 age (t0..T; period it = age - t0), 1 state ist (1-based), 2 cash-in-hand M at the start of the period (the cash
- *   column of a simulation record), 3 observed decision id (1-based), 4 (k = 5) observed consumption c_obs, NaN: not
- *   observed.
+ *   column of a simulation record), 3 observed decision id (1-based), 4..3+K the exact values x_1..x_K of the continuous
+ *   states (record columns 11 + j of the continuous state variables j, in state order; the grid part of the state
+ *   column is then ignored, and values outside the grid are held at its edge), 4+K (k = 5 + K) observed consumption
+ *   c_obs, NaN: not observed.
  * Per row and vector:  ll = log P_d(M) + [log phi((c_obs - c_d(M)) / sigma_c) - log sigma_c]
- * with the bracket only when k = 5, sigma_c > 0 and c_obs is not NaN; phi is the standard normal density.  P_d(M)
- * and c_d(M) are exactly what the choice draws evaluate (the probability rule of the solve, egdst_solution_set_choice_draws:
+ * with the bracket only when k = 5 + K, sigma_c > 0 and c_obs is not NaN; phi is the standard normal density.  P_d(M)
+ * and c_d(M) are exactly what the choice draws evaluate and record (with continuous states: the mixed values at x,
+ * and c_d = min(c_d, M - a0)) (the probability rule of the solve, egdst_solution_set_choice_draws:
  * held at the bound above the grid, equal weights when every value is -inf, the credit-constrained branch below the
  * first grid point), and log P_d = log e_d - log sum_d' e_d' of its weights.  A row contributes -inf when its decision
  * is not available in (it, ist) or its weight underflows (a non-modal choice as sigma_eps -> 0): such a total is -inf.
@@ -170,9 +179,10 @@ int egdst_solution_set_choice_draws(egdst_solution *s, int on);
  *   loglik  [nvec] per-vector totals (overwritten).  rowll: [nvec][nobs] per-row values, or NULL.
  * The totals are deterministic: the rows are summed in a fixed order over a block partition that depends on nobs only,
  * so the same obs give the same bits whatever nvec, ivec0 or launch.  The host entry point checks every row and
- * returns 2, naming the first malformed row, for an age, state or decision that is not an integer in range, or cash
- * that is not finite or lies below a0.  Returns 2 as well for a solution without choice cells (sigma_eps = 0, or
- * imported), an image with continuous states or without smoothing, k not 4 or 5, sigma_c < 0, or a vector range out of
+ * returns 2, naming the first malformed row, for an age, state or decision that is not an integer in range, cash
+ * that is not finite or lies below a0, or a continuous state value that is not finite.  Returns 2 as well for a
+ * solution without choice cells (sigma_eps = 0, or imported), an image without smoothing, k not 4 + K or 5 + K,
+ * sigma_c < 0, or a vector range out of
  * bounds (at most 65535 vectors).  The _device variant takes device pointers, is asynchronous on the library stream,
  * checks no rows (a malformed row gets rowll = NaN, and its vector's total is NaN) and adds each vector's total to
  * d_loglik (the caller zeroes it), so a rank can all-reduce the buffer right after. */

@@ -1,5 +1,5 @@
-"""Time the choice log-likelihood (egdst_choice_loglik_device) of retirement2_smooth at its defaults: a panel from a
-Philox draw simulation, evaluated for nvec = 1 and 64 parameter vectors, once in agent-major row order and once sorted
+"""Time the choice log-likelihood (egdst_choice_loglik_device) of a smoothing image (retirement2_smooth by default) at
+its defaults: a panel from a Philox draw simulation, evaluated for nvec = 1 and 64 parameter vectors, once in agent-major row order and once sorted
 by (age, state), with warm-up (CUDA events).  Then the mixture log-likelihood (egdst_mixture_loglik_device) on the
 agent-major panel, one individual per agent, at the same 64 vectors: 32 mixtures of K = 2 types and 64 one-type
 mixtures with the per-individual values written out, timed in alternation with the plain choice log-likelihood.
@@ -7,7 +7,10 @@ Then the central-difference scores (egdst_mixture_scores_device) of (duw, wage, 
 stencil, in alternation with the mixture log-likelihood of the same 7 vectors, and one BHHH iteration of
 EgdstModel.fit end to end (host clock).
 
-    python tools/loglik_time.py [agents (default 200000)] [reps (default 20)]
+    python tools/loglik_time.py [--model NAME] [agents (default 200000)] [reps (default 20)]
+
+--model: an image of examples.SMOOTH (default retirement2_smooth; humancapital_smooth and humancapital2_smooth time
+the continuous-state rows, which mix the choice values of 2^K corner cells).
 """
 import os
 import subprocess
@@ -20,9 +23,15 @@ import torch  # noqa: E402
 
 from egdst_b200 import capi, examples  # noqa: E402
 
-nsim = int(sys.argv[1]) if len(sys.argv) > 1 else 200_000
-reps = int(sys.argv[2]) if len(sys.argv) > 2 else 20
-m = examples.retirement2_smooth()
+args = sys.argv[1:]
+name = "retirement2_smooth"
+if "--model" in args:
+    i = args.index("--model")
+    name = args[i + 1]
+    del args[i:i + 2]
+nsim = int(args[0]) if len(args) > 0 else 200_000
+reps = int(args[1]) if len(args) > 1 else 20
+m = examples.SMOOTH[name]()
 m.compile()
 lib = m._capi()
 dev = torch.device("cuda", 0)
@@ -42,8 +51,8 @@ sims, _ = lib.simulate_philox(m, sol, init, seed=12345, ivec=32)
 sol.set_choice_draws(False)
 obs, start = capi.observations_from_sims(m, sims, start=True)
 nobs, k = obs.shape
-print("retirement2_smooth: sigma_eps %g, nt %d, nd %d, %d agents, %d observations (k = %d), %d launches per timing" % (
-    m.sigma_eps, m.nt, m.nd, nsim, nobs, k, reps))
+print("%s: sigma_eps %g, nt %d, nd %d, %d agents, %d observations (k = %d), %d launches per timing" % (
+    name, m.sigma_eps, m.nt, m.nd, nsim, nobs, k, reps))
 orders = {"agent-major": obs, "sorted by (age, state)": obs[np.lexsort((obs[:, 1], obs[:, 0]))]}
 desc = capi.Desc(m)
 d_tot = torch.zeros(64, dtype=torch.float64, device=dev)

@@ -1,7 +1,10 @@
-"""Time the simulation of retirement2_smooth with modal choices against choice draws (egdst_solution_set_choice_draws):
-sims+moments and moments only, the same solution, agents and Philox seed, the two modes alternating (CUDA events).
+"""Time the simulation of a smoothing image (retirement2_smooth by default) with modal choices against choice draws
+(egdst_solution_set_choice_draws): sims+moments and moments only, the same solution, agents and Philox seed, the two modes alternating (CUDA events).
 
-    python tools/sim_choice_time.py [nsim (default 4000000)] [rounds (default 3)]
+    python tools/sim_choice_time.py [--model NAME] [nsim (default 4000000)] [rounds (default 3)]
+
+--model: an image of examples.SMOOTH (default retirement2_smooth; humancapital_smooth and humancapital2_smooth time
+the continuous-state branch, whose draws mix the choice values of 2^K corner cells).
 """
 import os
 import subprocess
@@ -13,10 +16,16 @@ import torch  # noqa: E402
 
 from egdst_b200 import capi, examples  # noqa: E402
 
-nsim = int(sys.argv[1]) if len(sys.argv) > 1 else 4_000_000
-rounds = int(sys.argv[2]) if len(sys.argv) > 2 else 3
+args = sys.argv[1:]
+name = "retirement2_smooth"
+if "--model" in args:
+    i = args.index("--model")
+    name = args[i + 1]
+    del args[i:i + 2]
+nsim = int(args[0]) if len(args) > 0 else 4_000_000
+rounds = int(args[1]) if len(args) > 1 else 3
 reps = 5
-m = examples.retirement2_smooth()
+m = examples.SMOOTH[name]()
 m.compile()
 lib = m._capi()
 sol = lib.solve(m, strict=True)
@@ -27,7 +36,7 @@ except OSError:
     q = "%s, power limit not readable" % torch.cuda.get_device_name(dev)
 print("card: %s" % q)
 nt, nso = m.nt, m.nsimout()
-print("retirement2_smooth: sigma_eps %g, nt %d, nd %d, nsimout %d, %d agents, %d launches per timing" % (m.sigma_eps, nt, m.nd, nso, nsim, reps))
+print("%s: sigma_eps %g, nt %d, nd %d, nsimout %d, %d agents, %d launches per timing" % (name, m.sigma_eps, nt, m.nd, nso, nsim, reps))
 d_init = torch.empty(2 * nsim, dtype=torch.float64, device=dev)
 d_init[:nsim] = 1.0
 d_init[nsim:] = m.a0 + 0.5 * (m.mmax - m.a0) * torch.rand(nsim, dtype=torch.float64, device=dev, generator=torch.Generator(device=dev).manual_seed(1))
