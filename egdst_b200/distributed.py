@@ -30,6 +30,26 @@ def _dist():
     return dist if dist.is_available() and dist.is_initialized() else None
 
 
+def _rank_world(rank: Optional[int], world: Optional[int], group=None) -> Tuple[int, int]:
+    """``(rank, world)`` as given, else those of the process group (rank 0 of 1 without one)."""
+    dist = _dist()
+    if world is None:
+        world = dist.get_world_size(group) if dist else 1
+    if rank is None:
+        rank = dist.get_rank(group) if dist else 0
+    return rank, world
+
+
+def _individual_shard(obs, start, rank: int, world: int):
+    """Rank ``rank``'s contiguous block of individuals [lo, hi) of the offsets ``start`` [nind + 1]: its rows
+    start[lo]..start[hi]-1 of ``obs`` [nobs, k] and its offsets rebased to 0.  Returns (rows, offsets, (lo, hi))."""
+    obs = np.atleast_2d(np.asarray(obs, dtype=np.float64))
+    start = np.asarray(start, dtype=np.int64)
+    lo, hi = shard_range(start.size - 1, rank, world)
+    r0, r1 = int(start[lo]), int(start[hi])
+    return obs[r0:r1], (start[lo:hi + 1] - r0).astype(np.int32), (lo, hi)
+
+
 def all_reduce_moments(moments, group=None):
     """Sum the moment buffer [3, nsimout, nt] (sum x, sum x^2, alive count) over all ranks, in place.
     ``moments`` is a torch tensor (CUDA with nccl, CPU with gloo) or a numpy array (gloo only)."""
@@ -59,11 +79,7 @@ def simulate_sharded(lib, model, sol, init: np.ndarray, seed: int, rank: Optiona
     """Simulate this rank's block of the global agent list ``init`` [nsim, 2] and all-reduce the moments.
     Returns (sims of the local block or None, global moments [3, nsimout, nt], (lo, hi)).
     ``simulate_fn(init_block, agent0) -> (sims, moments)`` replaces the CUDA call in the CPU tests."""
-    dist = _dist()
-    if world is None:
-        world = dist.get_world_size(group) if dist else 1
-    if rank is None:
-        rank = dist.get_rank(group) if dist else 0
+    rank, world = _rank_world(rank, world, group)
     init = np.atleast_2d(np.asarray(init, dtype=np.float64))
     lo, hi = shard_range(init.shape[0], rank, world)
     block = init[lo:hi]
@@ -85,11 +101,7 @@ def solve_batch_sharded(lib, model, params: np.ndarray, init: np.ndarray, seed: 
     each rank solves its vectors in one batched pass, simulates ``init`` under every vector and contributes the
     per-vector moments [nvec, 3, nsimout, nt]; one all-reduce (sum, other ranks' rows are zero) assembles the table
     on every rank.  ``solve_sim_fn(params_block, first_index) -> moments_block`` replaces the CUDA path in CPU tests."""
-    dist = _dist()
-    if world is None:
-        world = dist.get_world_size(group) if dist else 1
-    if rank is None:
-        rank = dist.get_rank(group) if dist else 0
+    rank, world = _rank_world(rank, world, group)
     params = np.atleast_2d(np.asarray(params, dtype=np.float64))
     nvec = params.shape[0]
     lo, hi = shard_range(nvec, rank, world)
@@ -112,11 +124,7 @@ def choice_loglik_sharded(lib, model, sol, obs: np.ndarray, sigma_c: float = 0.0
     """Choice log-likelihood of the observations ``obs`` [nobs, k] under every parameter vector of ``sol``: each rank
     evaluates its contiguous block of rows and one all-reduce of the [nvec] totals gives every rank the sum.
     Returns (totals [nvec], (lo, hi)).  ``loglik_fn(obs_block) -> totals`` replaces the CUDA call in the CPU tests."""
-    dist = _dist()
-    if world is None:
-        world = dist.get_world_size(group) if dist else 1
-    if rank is None:
-        rank = dist.get_rank(group) if dist else 0
+    rank, world = _rank_world(rank, world, group)
     obs = np.atleast_2d(np.asarray(obs, dtype=np.float64))
     lo, hi = shard_range(obs.shape[0], rank, world)
     if loglik_fn is None:
@@ -136,20 +144,13 @@ def mixture_loglik_sharded(lib, model, sol, obs: np.ndarray, start: np.ndarray, 
     sum.  Returns (totals [nmix], per-individual outputs of the rank's block (the tuple after the totals that
     ``mixture_loglik`` returns with ``individuals`` / ``posterior``; empty without them), (lo, hi)).
     ``fn(obs_block, start_block)`` (returning what ``mixture_loglik`` returns) replaces the CUDA call in the CPU tests."""
-    dist = _dist()
-    if world is None:
-        world = dist.get_world_size(group) if dist else 1
-    if rank is None:
-        rank = dist.get_rank(group) if dist else 0
-    obs = np.atleast_2d(np.asarray(obs, dtype=np.float64))
-    start = np.asarray(start, dtype=np.int64)
-    lo, hi = shard_range(start.size - 1, rank, world)
-    r0, r1 = int(start[lo]), int(start[hi])
+    rank, world = _rank_world(rank, world, group)
+    rows, offsets, (lo, hi) = _individual_shard(obs, start, rank, world)
     if fn is None:
         def fn(block, sblock):
             return lib.mixture_loglik(model, sol, block, sblock, tvec, weights, sigma_c=sigma_c, individuals=individuals,
                                       posterior=posterior)
-    res = fn(obs[r0:r1], (start[lo:hi + 1] - r0).astype(np.int32))
+    res = fn(rows, offsets)
     tot, parts = (res[0], tuple(res[1:])) if isinstance(res, tuple) else (res, ())
     tot = np.ascontiguousarray(tot, dtype=np.float64)
     all_reduce_moments(tot, group)
@@ -164,19 +165,12 @@ def mixture_scores_sharded(lib, model, sol, obs: np.ndarray, start: np.ndarray, 
     [npar] and opg [npar * npar] are concatenated and all-reduced once (the OPG is a sum over individuals).  Returns
     (totals [nmix], grad [npar], opg [npar, npar], (lo, hi)).  ``fn(obs_block, start_block)`` (returning (totals,
     grad, opg)) replaces the CUDA call in the CPU tests."""
-    dist = _dist()
-    if world is None:
-        world = dist.get_world_size(group) if dist else 1
-    if rank is None:
-        rank = dist.get_rank(group) if dist else 0
-    obs = np.atleast_2d(np.asarray(obs, dtype=np.float64))
-    start = np.asarray(start, dtype=np.int64)
-    lo, hi = shard_range(start.size - 1, rank, world)
-    r0, r1 = int(start[lo]), int(start[hi])
+    rank, world = _rank_world(rank, world, group)
+    rows, offsets, (lo, hi) = _individual_shard(obs, start, rank, world)
     if fn is None:
         def fn(block, sblock):
             return lib.mixture_scores(model, sol, block, sblock, tvec, weights, mplus, mminus, hinv, sigma_c=sigma_c)
-    tot, grad, opg = fn(obs[r0:r1], (start[lo:hi + 1] - r0).astype(np.int32))
+    tot, grad, opg = fn(rows, offsets)
     nmix, npar = np.size(tot), np.size(grad)
     buf = np.ascontiguousarray(np.concatenate([np.ravel(tot), np.ravel(grad), np.ravel(opg)]), dtype=np.float64)
     all_reduce_moments(buf, group)
