@@ -225,6 +225,7 @@ class ModelLibrary:
                "egdst_set_stream", "egdst_launch_count", "egdst_profile_classes", "egdst_profile_class_name",
                "egdst_profile_enable", "egdst_profile_read", "egdst_solve", "egdst_solve_batch", "egdst_resolve", "egdst_solution_sizes",
                "egdst_solution_export", "egdst_solution_choice_cell", "egdst_solution_set_choice_draws", "egdst_solution_status", "egdst_solution_nvec", "egdst_solution_units", "egdst_solution_resends", "egdst_solution_phase_ms", "egdst_test_envelope2",
+               "egdst_test_sim_variant",
                "egdst_free_solution", "egdst_solution_import", "egdst_simulate", "egdst_simulate_philox",
                "egdst_simulate_device", "egdst_sim_moments", "egdst_sim_moments_device", "egdst_choice_loglik",
                "egdst_choice_loglik_device", "egdst_mixture_loglik", "egdst_mixture_loglik_device",
@@ -280,6 +281,7 @@ class ModelLibrary:
                                                   vp, C.c_int, C.c_int, C.c_int, vp, vp, C.c_int, vp, vp, vp, vp, vp, vp, vp]
         L.egdst_sim_moments.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, _dp, C.c_int, C.c_longlong, C.c_ulonglong, _dp]
         L.egdst_sim_moments_device.argtypes = [C.POINTER(EgdstDesc), vp, C.c_int, C.c_int, vp, C.c_int, C.c_longlong, C.c_ulonglong, vp]
+        L.egdst_test_sim_variant.argtypes = [C.POINTER(C.c_longlong)]
         L.egdst_test_envelope2.argtypes = [C.POINTER(EgdstDesc), C.c_int, C.c_int, C.c_int, _dp, _dp, _dp, C.c_int, C.c_double,
                                            _dp, _dp, _dp, _ip]
         if L.egdst_abi_version() != ABI_VERSION:
@@ -570,6 +572,13 @@ class ModelLibrary:
             import warnings
             warnings.warn(self.last_error(), EgdstWarning)
         return res
+
+    def sim_variant(self):
+        """(PHILOX, OUT, HDR, PB, mom_smem) of the egdst_k_simulate launch this thread made last, and the number of
+        simulation launches the thread has made (diagnostic, egdst_test_sim_variant)."""
+        v = (C.c_longlong * 6)()
+        self.L.egdst_test_sim_variant(v)
+        return (bool(v[0]), int(v[1]), bool(v[2]), int(v[3]), bool(v[4])), int(v[5])
 
     def test_envelope2(self, model, it: int, idd: int, X, Cc, V, evfa0: float):
         """Secondary envelope of one decision's EGM points (generation order) by the solve kernel's phases."""

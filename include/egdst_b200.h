@@ -103,6 +103,12 @@ int egdst_solution_phase_ms(egdst_solution *s, double *ms);
  * doubles each; *nout receives the number of points kept.  The tests compare it with the reference's envelope2. */
 int egdst_test_envelope2(const egdst_desc *d, int it, int ist, int id, const double *X, const double *C, const double *V, int n,
                          double evfa0, double *outX, double *outC, double *outV, int *nout);
+/* diagnostic: the egdst_k_simulate instantiation that the calling thread's last simulation launch took and
+ * where its moments were summed: out[0..5] = PHILOX (1: Philox uniforms, 0: randstream), OUT (bit 0 sims, bit 1
+ * moments, bit 2 choice draws), HDR (per-cell headers in the kernel arguments), PB (periods per write), mom_smem (1:
+ * moment accumulators in shared memory, 0: global atomics) and the number of simulation launches the thread has made
+ * (a host-buffer call launches once per chunk).  Returns 6.  The tests hold each launch variant to what it claims. */
+int egdst_test_sim_variant(long long *out);
 void egdst_free_solution(egdst_solution *s);
 /* Frees what the library keeps between calls: the one released solution object it caches for re-use by the next
  * solve of the same shape, and the calling thread's simulation workspace.  (The reference leaks on error paths and
